@@ -18,10 +18,16 @@ predict, and the SAME C4 tables through fit()'s fused single-GPU kernel, csrc/tr
 predict).  `--workload c2_fm`,
 `c3_mlp`, `c5_predict`, `c1_linear`, `c4_fused`, `c4_linear` select one of them as the headline instead.
 
-  value      whole-job samples/s, every input already resident in HBM, CUDA events, max over ranks.  The K-step
-             block is repeated `config.repeats` times inside the timed region so that it lasts >= ~100 ms; the
-             timed region contains EVERYTHING a step needs: (N > 1: the id all-gather,) Philox negatives, the
-             sort plan (coalesce's sort) and the persistent kernel.
+  value      whole-job samples/s, every input already resident in HBM, CUDA events, max over ranks.  The timed
+             region is exactly K steps, one epoch (one persistent launch unless K x global batch exceeds
+             SAMPLE_CAP), and contains EVERYTHING a step needs: (N > 1: the id all-gather,) Philox negatives, the
+             sort plan (coalesce's sort) and the persistent kernel.  The epoch's fixed cost (plan build, launch:
+             about 0.5 ms on one B200 at 1000 W) is spread over K steps, so the rate of a long epoch wants K in
+             the thousands.  (The fused single-GPU workloads repeat their K-step block `config.repeats` times so
+             that the region lasts >= --min-ms.)
+  --dump-outputs DIR  writes what the K timed steps computed as DIR/<name>.npy: the per-step losses and the user /
+             item rows their last step updated (a seeded sample of at most 8192 per table).  The inputs are
+             seeded, so two builds run with the same arguments can be compared array for array.
   e2e        the same blocks with the ids starting in pinned HOST memory (H2D inside the timed region) and the
              per-step losses read back to the host (D2H inside).
   roofline   the persistent kernel alone: algorithmic HBM bytes (SURVEY.md §8d: ids + each unique touched row's
@@ -84,7 +90,8 @@ def parse_args():
     ap.add_argument("--dim", type=int, default=0, help="override the workload's n_factors")
     ap.add_argument("--zipf", type=float, default=0.0, help="draw training ids from Zipf(A), A > 1, instead of uniformly")
     ap.add_argument("--cpu-seconds", type=float, default=20.0, help="budget of the CPU baseline sample")
-    ap.add_argument("--min-ms", type=float, default=100.0, help="the K-step block is repeated until the timed region lasts this long")
+    ap.add_argument("--min-ms", type=float, default=100.0,
+                    help="fused single-GPU workloads: the K-step block is repeated until the timed region lasts this long")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-others", action="store_true", help="skip the other_workloads sub-results")
     ap.add_argument("--shard-it", type=int, default=0, help="tuning: 16-byte chunks per lane of the sharded kernel (1 or 2)")
@@ -92,7 +99,14 @@ def parse_args():
     ap.add_argument("--shard-overlap", type=int, default=None, help="tuning: force the early first pass of phase A on (1) / off (0)")
     ap.add_argument("--emulate-world", type=int, default=0,
                     help="c4_linear on ONE GPU: host a group of this many ranks in one launch (structure check, no NVLink)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="c4 / c4_linear: after the timed steps, write what they computed to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload not in ("c4", "c4_linear") or args.impl != "b200"):
+        ap.error("--dump-outputs covers the row-sharded workload (c4, c4_linear), whose timed steps are exactly --steps")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -680,6 +694,47 @@ def shard_parity_check(dev, world, rank):
     return out
 
 
+DUMP_ROWS = 8192        # rows per table that --dump-outputs writes
+DUMP_BYTES = 64 << 20
+
+
+def shard_outputs(tr, loss, users, items):
+    """What a caller of the timed epoch receives: its per-step losses, and the user / item rows (embedding and bias)
+    that its last step updated -- all of them up to DUMP_ROWS per table, else a fixed, seeded sample; only the rows this
+    process holds.  Row ids are stored as float64 (exact below 2^53)."""
+    import numpy as np
+    import torch
+    out = {"loss": loss.float().cpu().numpy()}
+    G = tr.world
+    for name, ids in (("user", users), ("item", items)):
+        rows = np.unique(ids.cpu().numpy())
+        rows = rows[np.isin(rows % G, tr.local_ranks)]
+        if len(rows) > DUMP_ROWS:
+            rows = np.sort(np.random.default_rng(1234).choice(rows, DUMP_ROWS, replace=False))
+        weight = np.empty((len(rows), tr.dim), np.float32)
+        bias = np.empty(len(rows), np.float32)
+        for q in tr.local_ranks:
+            mine = rows % G == q
+            local = torch.from_numpy(rows[mine] // G).to(tr.device)
+            emb, lin = tr.tables[q][name]
+            weight[mine] = emb.index_select(0, local).cpu().numpy()
+            bias[mine] = lin.index_select(0, local).view(-1).cpu().numpy()
+        out[f"{name}_ids"] = rows.astype(np.float64)
+        out[f"{name}_weight"] = weight
+        out[f"{name}_bias"] = bias
+    return out
+
+
+def write_outputs(path, arrays):
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_BYTES} byte budget")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def sharded_bench(args, wl, name):
     import numpy as np
     import torch
@@ -703,6 +758,7 @@ def sharded_bench(args, wl, name):
     Bg = B * G
     D = wl["dim"]
     parity = shard_parity_check(dev, world, rank) if world > 1 else None
+    torch.manual_seed(1234 + rank)         # the tables' N(0, 1/dim) initialisation: the same inputs on every run
     tr = ShardedLinearTrainer(wl["n_users"], wl["n_items"], D, global_batch=Bg, optimizer=wl["opt"], lr=wl["lr"],
                               device=dev, emulate_world=emu or (1 if world == 1 else None))
     # every rank's loader output: (K + W) steps of its own B samples, stored [step, {user, positive}, B] so that a
@@ -749,72 +805,67 @@ def sharded_bench(args, wl, name):
     tr.check_status()
     first_loss = float(loss_w[0].item())
 
-    def timed(fn, n):
+    def timed(fn):
         e0, e1 = ev(), ev()
         sync_all()
         e0.record()
-        for _ in range(n):
-            loss = fn()
+        out = fn()
         e1.record()
         sync_all()
-        return e0.elapsed_time(e1), loss
+        return e0.elapsed_time(e1), out
 
-    # how many replays of the K-step block make a timed region of >= min_ms: probe one block, then put the replays
-    # into ONE epoch (r_in x K steps: one id all-gather, one plan build, one persistent launch per rank)
-    block(ids_d, W, K)
-    probe_ms, _ = timed(lambda: block(ids_d, W, K)[0], 1)
-    R = pick_repeats(probe_ms, args.min_ms, world, dev)
-    r_in, n_launch = split_repeats(R, K * Bg)
-    R = r_in * n_launch
-    rep_d = {q: t[W:].repeat(r_in, 1, 1) for q, t in ids_d.items()}
-    rep_h = {q: t[W:].repeat(r_in, 1, 1).pin_memory() for q, t in ids_h.items()}
-    loss_host = torch.empty(r_in * K, dtype=torch.float32).pin_memory()
-    resident_block = lambda: block(rep_d, 0, r_in * K, timing=True)[0]   # events around the plan and the kernel
+    # the K timed steps (loader steps [W, W + K)) are ONE epoch: one id all-gather, one plan build, one persistent
+    # launch per rank -- cut into several launches only where K x global batch exceeds the sample cap
+    n_launch = -(-K * Bg // SAMPLE_CAP)
+    per_launch = -(-K // n_launch)
+    loss_host = torch.empty(K, dtype=torch.float32).pin_memory()
+
+    def resident_epoch():
+        """The K steps from ids already in HBM; per launch: its losses, the events around its plan build and kernel,
+        and its (user, positive, negative) ids."""
+        launches = []
+        for s in range(0, K, per_launch):
+            loss, step_ids = block(ids_d, W + s, min(per_launch, K - s), timing=True)
+            launches.append((loss, tr.events, step_ids))
+        return launches
+
     if emu:
-        e2e_block = lambda: block(rep_h, 0, r_in * K, loss_host=loss_host)[0]
+        def e2e_epoch():
+            return torch.cat([block(ids_h, W + s, min(per_launch, K - s), loss_host=loss_host[s:s + per_launch])[0]
+                              for s in range(0, K, per_launch)])
     else:   # the trainer's own host-fed epoch: chunks copied on a side stream while the previous chunk trains
         def draw(gp, first):
             neg, _ = _lib.philox_negatives(1234, seen[0] + first, gp, wl["n_items"])
             return neg
 
-        def e2e_block():
-            loss = tr.train_epoch_host(rep_h[rank], draw, loss_host)
-            seen[0] += r_in * K * Bg
+        def e2e_epoch():
+            loss = tr.train_epoch_host(ids_h[rank][W:], draw, loss_host)
+            seen[0] += K * Bg
             return loss
-    resident_block()
-    e2e_block()
+    # both timed epochs are run once untimed first, on the same steps: the plan, workspace and allocator blocks of a
+    # K-step epoch exist before the timed region (no cudaMalloc inside it)
+    resident_epoch()
+    e2e_epoch()
+    sync_all()
+    tr.check_status()
     launches0 = tr.launches
-    # the timed region runs REGIONS times back to back (each: barrier + sync, n_launch epochs, sync + barrier); the
-    # line reports the MEDIAN region (max over ranks per region first) and lists all of them in config.region_ms --
-    # one region is a single ~100 ms launch, and a stray host / allocator hiccup on any rank would otherwise be the number
-    REGIONS = 3
-    ms_all, e2e_all, kern_all, plan_all = [], [], [], []
     with ClockSampler(local) as clocks:
-        for _ in range(REGIONS):
-            ms_i, loss = timed(resident_block, n_launch)
-            ms_all.append(ms_i)
-            p0, p1, k0, k1 = tr.events           # the region's last launch of r_in x K steps, scaled to the K-step block
-            kern_all.append(k0.elapsed_time(k1) / r_in)
-            plan_all.append(p0.elapsed_time(p1) / r_in)
-    launches = (tr.launches - launches0) // (n_launch * REGIONS) + 1
+        ms, timed_launches = timed(resident_epoch)
+    loss = torch.cat([l for l, _, _ in timed_launches])
+    events = [e for _, e, _ in timed_launches]
+    gu, gp, neg = (torch.cat(c) for c in zip(*(i for _, _, i in timed_launches)))
+    launches = (tr.launches - launches0) // n_launch + 1   # per launch; + the Philox kernel
     tr.check_status()
     mean_loss = float(loss.mean().item())
-    for _ in range(REGIONS):
-        e2e_all.append(timed(e2e_block, n_launch)[0])
-    # the ids of one K-step block (for the algorithmic bytes); the kernel's time is the one measured INSIDE the timed
-    # regions above (CUDA events around the persistent launch of the median region)
-    sync_all()
-    _, (gu, gp, neg) = block(ids_d, W, K)
-    sync_all()
+    outputs = shard_outputs(tr, loss, gu[-Bg:], torch.cat([gp[-Bg:], neg[-Bg:]])) if args.dump_outputs else None
+    e2e_ms, _ = timed(e2e_epoch)
     tr.check_status()
-    times = torch.tensor(ms_all + e2e_all + kern_all + plan_all, dtype=torch.float64, device=dev)
+    kernel_ms = sum(k0.elapsed_time(k1) for _, _, k0, k1 in events)     # per K steps
+    plan_ms = sum(p0.elapsed_time(p1) for p0, p1, _, _ in events)
+    times = torch.tensor([ms, e2e_ms, kernel_ms, plan_ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(times, op=dist.ReduceOp.MAX)
-    times = [float(x) for x in times.cpu()]
-    ms_all, e2e_all, kern_all, plan_all = (times[i * REGIONS:(i + 1) * REGIONS] for i in range(4))
-    mid = sorted(range(REGIONS), key=lambda i: ms_all[i])[REGIONS // 2]
-    ms, e2e_ms = ms_all[mid], sorted(e2e_all)[REGIONS // 2]
-    kernel_ms, plan_ms = kern_all[mid], plan_all[mid]          # per K steps
+    ms, e2e_ms, kernel_ms, plan_ms = (float(x) for x in times.cpu())
 
     S_ = {"sgd": 0, "adagrad": 1, "sparse_adam": 2}[wl["opt"]]
     alg = algorithmic_bytes(wl, gu, gp, neg, K, Bg, S_)        # of the GLOBAL batch; every rank owns 1/G of the rows
@@ -828,14 +879,11 @@ def sharded_bench(args, wl, name):
     nvl_ach = nvl_dir / (kernel_ms * 1e-3) / 1e9
     t_hbm, t_nvl = alg / G / (peak * 1e9), nvl_dir / (NVLINK_GBS * 1e9)
     out = {
-        "metric": "train samples/sec (fwd+bwd+sparse update)", "value": R * K * Bg / (ms * 1e-3), "unit": "samples/s",
-        "n_gpus": world, "steps": K, "warmup": W, "ms_per_step": ms / (R * K), "higher_is_better": True,
+        "metric": "train samples/sec (fwd+bwd+sparse update)", "value": K * Bg / (ms * 1e-3), "unit": "samples/s",
+        "n_gpus": world, "steps": K, "warmup": W, "ms_per_step": ms / K, "higher_is_better": True,
         "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": wl["desc"], "name": name, "batch_per_gpu": B, "global_batch": Bg, "optimizer": wl["opt"],
-                   "repeats": R, "steps_per_launch": r_in * K, "launches": n_launch,
-                   "timed_regions": REGIONS, "region_ms": [round(x, 3) for x in ms_all],
-                   "e2e_region_ms": [round(x, 3) for x in e2e_all],
-                   "region_note": "value / e2e are the MEDIAN of the timed regions listed here (each max over ranks)",
+                   "steps_per_launch": per_launch, "launches": n_launch,
                    "parallelism": (f"user / item tables ROW-SHARDED over {G} ranks (row % {G}); samples run on their "
                                    "user row's owner; item rows read from and gradient rows stored into the owner's "
                                    "HBM over NVLink by one persistent kernel per rank (CUDA-IPC mapped shards, flag "
@@ -844,13 +892,14 @@ def sharded_bench(args, wl, name):
                    "l2": f"inputs larger than L2: {(wl['n_users'] + wl['n_items']) * (D + 1) * 4 * (1 + S_) / G / 1e9:.1f} "
                          "GB of tables + optimizer state per rank, rows hit at random",
                    "timed_region": "id all-gather (NCCL) + Philox negatives + routing / sort plan + persistent sharded "
-                                   "kernel + loss all-reduce; the K-step block replayed `repeats` times, `steps_per_launch` "
-                                   "steps per all-gather + plan build + kernel launch",
+                                   "kernel + loss all-reduce; exactly K steps, `steps_per_launch` steps per all-gather + plan "
+                                   "build + kernel launch (max over ranks); each timed epoch also ran once untimed on "
+                                   "the same steps",
                    "clock_ramp": "0.3 s of device copies before the warm-up steps",
                    "first_step_loss": first_loss, "mean_loss_last_block": mean_loss,
-                   "loss_note": "the K-step block is replayed `repeats` times (fresh negatives each time): the model "
-                                "memorises its few samples, the hinge goes to 0; the work per step does not change"},
-        "e2e": {"value": R * K * Bg / (e2e_ms * 1e-3), "unit": "samples/s", "h2d_bytes_per_step": 16 * B,
+                   "loss_note": "mean over the K timed steps, the third pass over their samples (fresh negatives "
+                                "each time)"},
+        "e2e": {"value": K * Bg / (e2e_ms * 1e-3), "unit": "samples/s", "h2d_bytes_per_step": 16 * B,
                 "d2h_bytes_per_step": 4,
                 "note": "ShardedLinearTrainer.train_epoch_host: each rank's user+positive ids from pinned host memory in "
                         "chunks of >= 64 steps, chunk i+1 copied on a side stream while chunk i trains; negatives are "
@@ -861,11 +910,11 @@ def sharded_bench(args, wl, name):
                      "traffic_source": "static: profiles/shard_r2.md (ncu --set full of a 1-rank launch on 4M x 1M tables; "
                                        "per step, times K; not measured by this run)",
                      "kernel": "trs::shard_train_kernel (one persistent launch per rank)",
-                     "kernel_time_source": "CUDA events around the persistent launch INSIDE the median timed region "
-                                           "(steps_per_launch steps), max over ranks",
+                     "kernel_time_source": "CUDA events around the persistent launches INSIDE the timed region, "
+                                           "summed over its launches, max over ranks",
                      "kernel_ms_per_step": kernel_ms / K, "plan_ms_per_step": plan_ms / K,
                      "algorithmic_bytes_per_step": alg / K / G,
-                     "whole_step_frac": alg / G / (ms / R * 1e-3) / 1e9 / peak,
+                     "whole_step_frac": alg / G / (ms * 1e-3) / 1e9 / peak,
                      "nvlink": {"bytes_per_step_per_direction": nvl_dir / K, "achieved": nvl_ach, "peak": NVLINK_GBS,
                                 "unit": "GB/s per direction per GPU", "frac": nvl_ach / NVLINK_GBS,
                                 "peak_source": "measured peer copy on this pool (B200_PROFILING.md); 900 nominal"},
@@ -879,7 +928,7 @@ def sharded_bench(args, wl, name):
     tr.close()
     del tr
     torch.cuda.empty_cache()
-    return out, rank
+    return out, outputs
 
 
 # ------------------------------------------------------------------------------------------------
@@ -995,10 +1044,11 @@ def main():
         if rank == 0:
             print(json.dumps(reference_line(args, wl, name, "cpu" if args.impl == "reference" else "cuda")))
         return
+    outputs = None
     if wl.get("predict"):
         out = predict_bench(args, wl, name)
     elif wl.get("sharded"):
-        out, _ = sharded_bench(args, wl, name)
+        out, outputs = sharded_bench(args, wl, name)
     else:
         out, _ = gpu_bench(args, wl, name)
     # ---- the other BASELINE configs, in the same line ----
@@ -1031,6 +1081,8 @@ def main():
         return
     if others:
         out["other_workloads"] = others
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
     if args.gpus == 1 and not args.no_cpu_baseline:
         r = cpu_predict(wl, args.cpu_seconds) if wl.get("predict") else \
             port_reference(wl, steps=8, warmup=1, budget_s=args.cpu_seconds)
