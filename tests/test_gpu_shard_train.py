@@ -47,43 +47,94 @@ def _to(dev, a):
     return torch.from_numpy(np.ascontiguousarray(a)).to(dev)
 
 
-@pytest.mark.parametrize("world", [1, 2, 3, 4, 8])
-@pytest.mark.parametrize("dim", [16, 64, 128, 256])
-@pytest.mark.parametrize("opt", ["sgd", "adagrad", "sparse_adam"])
-def test_sharded_steps_match_the_oracle_on_the_global_batch(dev, world, dim, opt):
-    if opt != "sparse_adam" and (dim in (16, 256) or world in (3, 8)):
-        pytest.skip("optimizer variants are covered on the other shapes")
+@pytest.fixture
+def shard_hooks():
+    """The sharded kernel's tuning hooks are process-wide settings: whoever changes one gets the defaults back
+    afterwards (chunks per lane 1, overlap automatic, remote L2 hint on), also when the test fails."""
+    from torchrecsys_b200 import _lib
+    L = _lib.lib()
+    yield L
+    L.trs_debug_shard_chunks_per_lane(1)
+    L.trs_debug_shard_overlap(-1)
+    L.trs_debug_shard_remote_hint(1)
+
+
+def _train_vs_oracle(dev, world, opt, lr, B, params, user, pos, neg):
+    """Train the epoch (user, pos, neg) on ``world`` ranks and compare losses, tables and optimizer state with the
+    oracle's single-process steps on the global batch; rows nobody looked up must be bit-identical to ``params``.
+    Returns the trainer, the losses and the numbers of untouched user / item rows."""
+    U, dim = params["user.weight"].shape
+    I = params["item.weight"].shape[0]
+    init = {k: v.copy() for k, v in params.items()}
+    tr = _trainer(dev, world, U, I, dim, B, opt, lr, params)
+    loss = tr.train_epoch(_to(dev, user), _to(dev, pos), _to(dev, neg), B).cpu().numpy()
+
+    spec = O.OptSpec(opt, lr=lr)
+    ref = {k: v.copy() for k, v in params.items()}
+    state = O.init_opt_state(ref, spec)
+    want = []
+    for s in range(-(-len(user) // B)):
+        batch = {"user": user[s * B:(s + 1) * B], "pos": pos[s * B:(s + 1) * B], "neg": neg[s * B:(s + 1) * B]}
+        want.append(O.train_step("linear", ref, state, batch, spec, s + 1))
+    np.testing.assert_allclose(loss[0], want[0], rtol=2e-5, atol=2e-6)
+    np.testing.assert_allclose(loss, np.array(want), rtol=2e-5 if opt == "sgd" else 5e-4, atol=2e-6)
+    tol = dict(rtol=2e-3, atol=2e-3 * lr * 20) if opt == "sparse_adam" else dict(rtol=1e-4, atol=2e-5)
+    got = {k: v.cpu().numpy() for k, v in tr.state_dict().items()}
+    for k in ref:
+        np.testing.assert_allclose(got[k], ref[k], err_msg=k, **tol)
+    gst = tr.optimizer_state_dict()
+    for k in ref:
+        for sname, want_s in state[k].items():
+            if k == "user_bias.weight":
+                continue  # its gradient is exactly 0 (SURVEY D12): state stays 0 here; the oracle decays nothing either
+            np.testing.assert_allclose(gst[k][sname].cpu().numpy(), want_s, err_msg=f"{k}.{sname}", **tol)
+    # rows nobody looked up are bit-identical to the initial tables: embedding and bias, user and item
+    untouched = {"user": np.setdiff1d(np.arange(U), user), "item": np.setdiff1d(np.arange(I), np.concatenate([pos, neg]))}
+    for name, rows in untouched.items():
+        for k in (f"{name}.weight", f"{name}_bias.weight"):
+            assert np.array_equal(got[k][rows], init[k][rows]), k
+    return tr, loss, len(untouched["user"]), len(untouched["item"])
+
+
+def _steps_match_the_oracle(dev, world, dim, opt):
     U, I, steps = 3001, 701, 4
     B = 1500 if opt == "sgd" else 1024   # power-of-two batch: g = 1/B sums exactly (see test_gpu_train_shapes)
     lr = 0.05
     rng = np.random.default_rng(dim * 11 + world)
     params = _full_params(rng, U, I, dim)
     n = B * steps - (37 if opt == "sgd" else 0)   # SGD: short last batch
-    user, pos, neg = _skewed(rng, U, n), _skewed(rng, I, n), _skewed(rng, I, n)
-    tr = _trainer(dev, world, U, I, dim, B, opt, lr, params)
-    loss = tr.train_epoch(_to(dev, user), _to(dev, pos), _to(dev, neg), B).cpu().numpy()
+    items = np.setdiff1d(np.arange(I), rng.choice(I, 40, replace=False))   # 40 item rows nobody looks up
+    user = _skewed(rng, U, n)
+    pos, neg = items[_skewed(rng, len(items), n)], items[_skewed(rng, len(items), n)]
+    _, _, n_user_rows, n_item_rows = _train_vs_oracle(dev, world, opt, lr, B, params, user, pos, neg)
+    assert n_user_rows and n_item_rows >= 40
 
-    spec = O.OptSpec(opt, lr=lr)
-    state = O.init_opt_state(params, spec)
-    want = []
-    for s in range(steps):
-        batch = {"user": user[s * B:(s + 1) * B], "pos": pos[s * B:(s + 1) * B], "neg": neg[s * B:(s + 1) * B]}
-        want.append(O.train_step("linear", params, state, batch, spec, s + 1))
-    np.testing.assert_allclose(loss[0], want[0], rtol=2e-5, atol=2e-6)
-    np.testing.assert_allclose(loss, np.array(want), rtol=2e-5 if opt == "sgd" else 5e-4, atol=2e-6)
-    tol = dict(rtol=2e-3, atol=2e-3 * lr * 20) if opt == "sparse_adam" else dict(rtol=1e-4, atol=2e-5)
-    got = {k: v.cpu().numpy() for k, v in tr.state_dict().items()}
-    for k in params:
-        np.testing.assert_allclose(got[k], params[k], err_msg=k, **tol)
-    gst = tr.optimizer_state_dict()
-    for k in params:
-        for sname, want_s in state[k].items():
-            if k == "user_bias.weight":
-                continue  # its gradient is exactly 0 (SURVEY D12): state stays 0 here; the oracle decays nothing either
-            np.testing.assert_allclose(gst[k][sname].cpu().numpy(), want_s, err_msg=f"{k}.{sname}", **tol)
-    # rows nobody looked up are bit-identical to the initial tables
-    untouched = np.setdiff1d(np.arange(U), user)
-    assert untouched.size and np.array_equal(got["user.weight"][untouched], params["user.weight"][untouched])
+
+# dims 16, 64, 128 and 256 give the row shapes (G lanes, IT chunks per lane) = (4,1), (16,1), (32,1), (32,2), each
+# filled by dim / 4 chunks.  These add the other default shapes, (8,1) at 20 and (32,4) at 260-512, and partial rows,
+# where dim / 4 is not a multiple of G: 4, 12 (4,1), 20 (8,1), 36 (16,1), 100 (32,1), 132 (32,2), 260 and 384 (32,4)
+_NEW_DIMS = (4, 12, 20, 36, 100, 132, 260, 384, 512)
+
+
+@pytest.mark.parametrize("world", [1, 2, 3, 4, 8])
+@pytest.mark.parametrize("dim", sorted((16, 64, 128, 256) + _NEW_DIMS))
+@pytest.mark.parametrize("opt", ["sgd", "adagrad", "sparse_adam"])
+def test_sharded_steps_match_the_oracle_on_the_global_batch(dev, world, dim, opt):
+    if opt != "sparse_adam" and (world != 3 if dim in _NEW_DIMS else (dim in (16, 256) or world in (3, 8))):
+        pytest.skip("optimizer variants are covered on the other shapes")
+    _steps_match_the_oracle(dev, world, dim, opt)
+
+
+@pytest.mark.parametrize("world", [1, 3])
+@pytest.mark.parametrize("dim", [32, 48, 64, 100, 128])
+@pytest.mark.parametrize("opt", ["sgd", "sparse_adam"])
+def test_two_chunks_per_lane_match_the_oracle(dev, shard_hooks, world, dim, opt):
+    """trs_debug_shard_chunks_per_lane(2): (G, IT) = (4,2), (8,2) with a partial row, (8,2), (16,2) partial, (16,2) --
+    shapes only this setting reaches, and the ones without the item-row prefetch region.  Against the oracle, not bit
+    for bit against one chunk per lane: a lane sums its IT chunks before the lanes are added, so the dot products'
+    association differs."""
+    shard_hooks.trs_debug_shard_chunks_per_lane(2)
+    _steps_match_the_oracle(dev, world, dim, opt)
 
 
 def test_group_sizes_agree_bit_for_bit_and_split_launches_equal_one(dev):
@@ -124,35 +175,58 @@ def _plan_words(plan, n, B):
     return out
 
 
-@pytest.mark.parametrize("world,n_items", [(1, 3000), (4, 3000), (2, 3_000_000), (8, 3_000_000)])
-def test_plan_flags_never_miss_a_row_the_previous_step_updates(dev, world, n_items):
-    """Phase A runs a sample BEFORE the previous step's owners are done unless the plan flags one of its three rows as
-    updated by that step (bits 28 / 30 / 31 of its samp entry).  A flag may be set needlessly (the filter is hashed for
-    large tables), it must never be missing; bit 27 marks the users with one lookup in the step."""
+def _check_shard_plan(dev, user, pos, neg, B, n_users, n_items, world):
+    """Every rank's plan (csrc/shard.cu: trs_shard_plan_build) against a numpy restatement, entry by entry:
+      samp_cnt / samp   the samples whose user the rank owns (user % W == rank), their positions in ascending order;
+      ukey / uval       (local row user // W, index in the rank's list), stably sorted by row, rows the step looks up
+                        once dropped (phase A finishes those: every lookup of a user is on its owner); own_cnt[2s]
+      ikey / ival       (local row id // W, lookup j) of the owned item lookups j < 2 B_s (j < B_s: positive of sample j,
+                        else negative of sample j - B_s), stably sorted by row; own_cnt[2s + 1]
+    Only the first own_cnt entries of a step's segment are compared: the rest is scratch.
+    Flags of the samp entries: phase A runs a sample BEFORE the previous step's owners are done unless the plan flags one
+    of its three rows as updated by that step (bits 28 / 30 / 31).  A flag may be set needlessly (the filter is hashed
+    for large tables), it must never be missing; bit 27 marks the users with one lookup in the step, bit 29 is unused."""
     from torchrecsys_b200 import _lib
-    U, B, steps = 4000, 1024, 5
-    rng = np.random.default_rng(world + n_items)
-    n = B * steps - 100                                   # a ragged last step
-    user, pos, neg = _skewed(rng, U, n), _skewed(rng, n_items, n), rng.integers(0, n_items, n)
+    n = len(user)
+    steps = -(-n // B)
     ids = [_to(dev, a) for a in (user, pos, neg)]          # make_epoch takes addresses: the tensors must stay alive
     epoch = _lib.make_epoch(*ids, None, None, B)
     needless = total = 0
     for rank in range(world):
         sh = _lib.Shard()
-        sh.rank, sh.world, sh.dim, sh.n_users, sh.n_items = rank, world, 64, U, n_items
+        sh.rank, sh.world, sh.dim, sh.n_users, sh.n_items = rank, world, 64, n_users, n_items
         P = _plan_words(_lib.shard_plan_build(sh, epoch, dev), n, B)
         torch.cuda.synchronize()
         for s in range(steps):
             lo, hi = s * B, min(n, (s + 1) * B)
-            mine = np.flatnonzero(user[lo:hi] % world == rank)
+            u_s, p_s, n_s = user[lo:hi], pos[lo:hi], neg[lo:hi]
+            mine = np.flatnonzero(u_s % world == rank)
             cnt = int(P["samp_cnt"][s])
+            assert cnt == len(mine), (rank, s)
             ent = P["samp"][lo:lo + cnt]
-            b = (ent & 0x07FFFFFF).astype(np.int64)
-            np.testing.assert_array_equal(b, mine)        # the rank's samples, in batch order
-            u, p_, n_ = user[lo + b], pos[lo + b], neg[lo + b]
-            uniq, c = np.unique(user[lo:hi], return_counts=True)
+            np.testing.assert_array_equal(ent & 0x07FFFFFF, mine)        # the rank's samples, in batch order
+            u, p_, n_ = u_s[mine], p_s[mine], n_s[mine]
+            uniq, c = np.unique(u_s, return_counts=True)
             single = np.isin(u, uniq[c == 1])
             np.testing.assert_array_equal((ent >> 27) & 1, single.astype(np.uint32))
+            assert not ((ent >> 29) & 1).any()
+
+            key = u // world
+            order = np.argsort(key, kind="stable")
+            kept = order[~single[order]]
+            nu = int(P["own_cnt"][2 * s])
+            assert nu == len(kept), (rank, s)
+            np.testing.assert_array_equal(P["ukey"][lo:lo + nu], key[kept])
+            np.testing.assert_array_equal(P["uval"][lo:lo + nu], kept)    # bit 31 (done in phase A) clear
+
+            both = np.concatenate([p_s, n_s])
+            j = np.flatnonzero(both % world == rank)
+            order = np.argsort(both[j] // world, kind="stable")
+            ni = int(P["own_cnt"][2 * s + 1])
+            assert ni == len(j), (rank, s)
+            np.testing.assert_array_equal(P["ikey"][2 * lo:2 * lo + ni], both[j[order]] // world)
+            np.testing.assert_array_equal(P["ival"][2 * lo:2 * lo + ni], j[order])
+
             f_user, f_pos, f_neg = (((ent >> k) & 1).astype(bool) for k in (28, 30, 31))
             if s == 0:                                     # nothing is known about the step before the plan
                 assert f_user.all() and f_pos.all() and f_neg.all()
@@ -166,6 +240,41 @@ def test_plan_flags_never_miss_a_row_the_previous_step_updates(dev, world, n_ite
                 needless += int((flag & ~need).sum())
                 total += len(flag)
     assert needless <= 0.04 * total
+
+
+@pytest.mark.parametrize("world,n_items", [(1, 3000), (4, 3000), (2, 3_000_000), (8, 3_000_000)])
+def test_plan_flags_never_miss_a_row_the_previous_step_updates(dev, world, n_items):
+    """The whole plan (_check_shard_plan) with an exact item filter (3000 items) and a hashed one (3M)."""
+    U, B, steps = 4000, 1024, 5
+    rng = np.random.default_rng(world + n_items)
+    n = B * steps - 100                                   # a ragged last step
+    user, pos, neg = _skewed(rng, U, n), _skewed(rng, n_items, n), rng.integers(0, n_items, n)
+    _check_shard_plan(dev, user, pos, neg, B, U, n_items, world)
+
+
+def _ids(rng, kind, n_rows, n):
+    """Uniform ids, or _skewed's mix with half of it mirrored to the top of the table (hot rows at both ends)."""
+    if kind == "uniform":
+        return rng.integers(0, n_rows, n, dtype=np.int64)
+    x = _skewed(rng, n_rows, n)
+    return np.where(rng.random(n) < 0.5, x, n_rows - 1 - x)
+
+
+@pytest.mark.parametrize("ids", ["uniform", "skewed"])
+@pytest.mark.parametrize("n_users,n_items,world,B", [   # radix passes of the user / item sort on every rank
+    (1000, 200, 4, 1000),                               # 1 / 1
+    (3001, 701, 8, 1000),                               # 2 / 1
+    (50_000_000, 5_000_000, 1, 16384),                  # 4 / 3: the benchmark's workload (C4) on one GPU
+    (50_000_000, 5_000_000, 8, 131072),                 # 3 / 3: C4 on eight GPUs (16384 samples per rank and step)
+    (2 ** 32 - 1, 2 ** 32 - 1, 3, 16384),               # 4 / 4: ids >= 2^31, a group size that is not a power of two
+])
+def test_shard_plan_matches_its_numpy_restatement(dev, n_users, n_items, world, B, ids):
+    """The plan at the benchmark's table sizes and batches: odd pass counts start the sort in the scratch buffer, a
+    step spans many route tiles (2048 lookups each) and many 1024-pair chunks of the in-place user compaction."""
+    rng = np.random.default_rng(n_users % 1000 + world + (ids == "skewed"))
+    n = 3 * B - B // 3 - 1                                # a ragged last step
+    user, pos, neg = (_ids(rng, ids, m, n) for m in (n_users, n_items, n_items))
+    _check_shard_plan(dev, user, pos, neg, B, n_users, n_items, world)
 
 
 def test_host_fed_epoch_in_chunks_equals_one_resident_epoch(dev):

@@ -1473,7 +1473,9 @@ extern "C" int trs_shard_train_steps(const trs_shard* shards, int n_local, const
     return TRS_OK;
 }
 
-// tuning hook (not part of trs.h; results do not depend on it): chunks per lane the sharded kernel prefers (1 or 2)
+// tuning hook (not part of trs.h): chunks per lane the sharded kernel prefers (1 or 2).  Results agree to rounding, not
+// bit for bit: row_dot_partial sums a lane's IT chunks before group_sum<G> adds the lanes, so the dot products'
+// association follows the row shape
 extern "C" void trs_debug_shard_chunks_per_lane(int it) { g_shard_prefer_it = it == 1 ? 1 : 2; }
 // debug hook: device buffer of n_local * n_steps * CTAs-per-rank * 8 uint64 that the next launches fill with phase
 // time stamps (tools/shard_phases.py); NULL switches it off
