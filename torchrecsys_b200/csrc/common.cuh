@@ -124,6 +124,18 @@ __device__ __forceinline__ void store_row(float* __restrict__ base, int nch, int
         if (c < nch) r.c[i].st(base + (size_t)c * V);
     }
 }
+template <int V, int IT>
+__device__ __forceinline__ void row_zero(Row<V, IT>& r) {
+#pragma unroll
+    for (int i = 0; i < IT; ++i) r.c[i] = Vec<V>::zero();
+}
+template <int V, int IT>
+__device__ __forceinline__ void row_acc(Row<V, IT>& a, const Row<V, IT>& b) {  // a += b, unfused
+#pragma unroll
+    for (int i = 0; i < IT; ++i)
+#pragma unroll
+        for (int k = 0; k < V; ++k) a.c[i][k] = __fadd_rn(a.c[i][k], b.c[i][k]);
+}
 
 // sum over the G lanes of a group (G a power of two, groups aligned inside the warp)
 template <int G>
@@ -134,6 +146,28 @@ __device__ __forceinline__ float group_sum(float x) {
 }
 
 __device__ __forceinline__ float warp_sum(float x) { return group_sum<32>(x); }
+
+// order-preserving map float -> uint32: a < b  <=>  float_key(a) < float_key(b)
+__device__ __forceinline__ uint32_t float_key(float x) {
+    const uint32_t u = __float_as_uint(x);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+
+// Philox4x32-10: the ten rounds on counter c under key (k0, k1); c holds the four output words afterwards
+__device__ __forceinline__ void philox4x32_10(uint32_t c[4], uint32_t k0, uint32_t k1) {
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const uint32_t hi0 = __umulhi(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
+        const uint32_t n0 = hi1 ^ c[1] ^ k0, n2 = hi0 ^ c[3] ^ k1;
+        c[0] = n0;
+        c[1] = lo1;
+        c[2] = n2;
+        c[3] = lo0;
+        k0 += 0x9E3779B9u;
+        k1 += 0xBB67AE85u;
+    }
+}
 
 // ---- launch-shape dispatch -----------------------------------------------------------------
 // (V, G, IT) chosen from dim: see DESIGN.md "row layout".

@@ -109,11 +109,6 @@ static void launch_scores_backward(const trs_model* m, const int64_t* user, cons
 // ------------------------------------------------------------------------------------------------------------
 // sort-based ROC-AUC
 // ------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t float_key(float x) {  // order-preserving: a < b  <=>  key(a) < key(b)
-    const uint32_t u = __float_as_uint(x);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-
 __global__ void __launch_bounds__(256)
 auc_keys_kernel(const float* __restrict__ pos, int64_t n_pos, const float* __restrict__ neg, int64_t n_neg,
                 uint32_t* __restrict__ key, uint32_t* __restrict__ val) {
@@ -172,16 +167,7 @@ __global__ void auc_final_kernel(const unsigned long long* __restrict__ sum2, in
 // ------------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t philox_word(uint64_t seed, uint64_t idx) {
     uint32_t c[4] = {(uint32_t)idx, (uint32_t)(idx >> 32), 0x5EED5EEDu, 0u};
-    uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        const uint32_t hi0 = __umulhi(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
-        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
-        const uint32_t n0 = hi1 ^ c[1] ^ k0, n2 = hi0 ^ c[3] ^ k1;
-        c[0] = n0; c[1] = lo1; c[2] = n2; c[3] = lo0;
-        k0 += 0x9E3779B9u;
-        k1 += 0xBB67AE85u;
-    }
+    philox4x32_10(c, (uint32_t)seed, (uint32_t)(seed >> 32));
     return c[0];
 }
 __global__ void __launch_bounds__(256)

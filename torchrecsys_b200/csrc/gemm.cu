@@ -89,11 +89,11 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
         tc::tma_prefetch_desc(&tmap_a);
         tc::tma_prefetch_desc(&tmap_b);
         for (int s = 0; s < STAGES; ++s) {
-            tc::mbar_init(&full[s], 1);
-            tc::mbar_init(&empty[s], 1);
+            mbar_init(&full[s], 1);
+            mbar_init(&empty[s], 1);
         }
-        tc::mbar_init(acc_full, 1);
-        tc::fence_barrier_init();
+        mbar_init(acc_full, 1);
+        fence_barrier_init();
     }
     if (warp == 1) tc::tmem_alloc(tmem_slot, BN);
     tc::tc_fence_before();
@@ -106,8 +106,8 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
             for (int kb = 0; kb < nkb; ++kb) {
                 const int s = kb % STAGES;
                 const uint32_t ph = (uint32_t)(kb / STAGES) & 1u;
-                tc::mbar_wait(&empty[s], ph ^ 1u);
-                tc::mbar_arrive_expect_tx(&full[s], S::A_BYTES + S::B_BYTES);
+                mbar_wait(&empty[s], ph ^ 1u);
+                mbar_arrive_expect_tx(&full[s], S::A_BYTES + S::B_BYTES);
                 const int k = (kb0 + kb) * GEMM_BK;
                 if (A_MN) {
 #pragma unroll
@@ -131,7 +131,7 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
         for (int kb = 0; kb < nkb; ++kb) {
             const int s = kb % STAGES;
             const uint32_t ph = (uint32_t)(kb / STAGES) & 1u;
-            tc::mbar_wait(&full[s], ph);
+            mbar_wait(&full[s], ph);
             tc::tc_fence_after();
             if (tc::elect_one()) {
 #pragma unroll
@@ -156,7 +156,7 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
         const bool row_valid = row_in && (row % g.rows_per_half) < g.rows_valid;
         const bool stats = g.col_sum != nullptr;
         if (nkb > 0) {
-            tc::mbar_wait(acc_full, 0);
+            mbar_wait(acc_full, 0);
             tc::tc_fence_after();
         }
 #pragma unroll 1

@@ -152,21 +152,6 @@ static void launch_eval(const trs_model* m, const trs_epoch* ep, float* loss, fl
 // ---------------------------------------------------------------------------------------
 // a9: Philox4x32-10 negatives
 // ---------------------------------------------------------------------------------------
-__device__ __forceinline__ void philox4x32_10(uint32_t c[4], uint32_t k0, uint32_t k1) {
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        uint32_t hi0 = __umulhi(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
-        uint32_t hi1 = __umulhi(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
-        uint32_t n0 = hi1 ^ c[1] ^ k0, n2 = hi0 ^ c[3] ^ k1;
-        c[0] = n0;
-        c[1] = lo1;
-        c[2] = n2;
-        c[3] = lo0;
-        k0 += 0x9E3779B9u;
-        k1 += 0xBB67AE85u;
-    }
-}
-
 __global__ void __launch_bounds__(256)
 philox_neg_kernel(uint64_t seed, uint64_t first, const int64_t* __restrict__ pos, int64_t n,
                   int64_t n_items, const int64_t* __restrict__ item_meta, int n_meta,

@@ -39,6 +39,7 @@
 #include <string.h>
 
 #include "plan.cuh"
+#include "ptx.cuh"
 #include "scorer.cuh"
 #include "train.cuh"
 
@@ -357,6 +358,34 @@ static int dirty_log2_bits(const trs_epoch* ep, int64_t n_items, bool* exact) {
     return *exact ? le : lb;
 }
 
+// scratch of the plan build: the radix sort's other (key, value) buffers, sized for the item space (two lookups per
+// sample), the per-tile counts of the route kernels, the sort's digit histograms and the dirty bitmaps of every step,
+// one for the item rows and one for the user rows
+struct ShardPlanTmp {
+    size_t tkey, tval, tile_cnt, hist, bitmap, ubitmap, total;
+};
+static ShardPlanTmp shard_plan_tmp(const trs_epoch* ep) {
+    ShardPlanTmp L;
+    size_t off = 0;
+    auto take = [&](size_t bytes) {
+        size_t o = off;
+        off += (bytes + 255) / 256 * 256;
+        return o;
+    };
+    const size_t n = (size_t)ep->n_samples, steps = (size_t)n_steps_of(ep);
+    const size_t tiles = (size_t)((2ll * ep->batch + RT_TILE - 1) / RT_TILE);
+    bool exact;
+    const int lb = dirty_log2_bits(ep, (int64_t)1 << 40, &exact);  // the hashed size: an exact bitmap is never larger
+    L.tkey = take(2 * n * sizeof(uint32_t));
+    L.tval = take(2 * n * sizeof(uint32_t));
+    L.tile_cnt = take(steps * tiles * sizeof(uint32_t));
+    L.hist = take(hist_bytes(ep));
+    L.bitmap = take((steps << lb) / 8);
+    L.ubitmap = take((steps << lb) / 8);
+    L.total = off;
+    return L;
+}
+
 // ------------------------------------------------------------------------------------------------------------
 // the kernel
 // ------------------------------------------------------------------------------------------------------------
@@ -391,72 +420,6 @@ struct ShardCtx {  // everything one (virtual) rank needs; copied to shared memo
     unsigned long long* trace;  // debug (trs_debug_shard_trace): [n_steps][cta_per_rank][8] globaltimer stamps, or NULL
 };
 
-// sync words of one rank (zeroed ONCE when allocated): word 64 = arrivals at cross-rank barriers, added to by every
-// CTA of every rank, never reset; word 16 = arrivals of the rank's own CTAs at rank-local barriers (memset before
-// every launch: no peer touches it)
-
-__device__ __forceinline__ void st_relaxed_sys(unsigned* p, unsigned v) {
-    asm volatile("st.relaxed.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-__device__ __forceinline__ void st_relaxed_gpu(unsigned* p, unsigned v) {
-    asm volatile("st.relaxed.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-__device__ __forceinline__ unsigned ld_relaxed_sys(const unsigned* p) {
-    unsigned v;
-    asm volatile("ld.relaxed.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ unsigned ld_relaxed_gpu(const unsigned* p) {
-    unsigned v;
-    asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ unsigned long long shard_now_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)::"memory");
-    return t;
-}
-__device__ __forceinline__ void sh_cp_async16(void* smem, const void* gmem) {
-    const unsigned sa = (unsigned)__cvta_generic_to_shared(smem);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa), "l"(gmem) : "memory");
-}
-__device__ __forceinline__ void sh_cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-// at most n copy groups still pending (n is a compile-time constant after unrolling)
-__device__ __forceinline__ void sh_cp_async_wait(int n) {
-    switch (n) {
-        case 0: asm volatile("cp.async.wait_group 0;" ::: "memory"); break;
-        case 1: asm volatile("cp.async.wait_group 1;" ::: "memory"); break;
-        case 2: asm volatile("cp.async.wait_group 2;" ::: "memory"); break;
-        case 3: asm volatile("cp.async.wait_group 3;" ::: "memory"); break;
-        case 4: asm volatile("cp.async.wait_group 4;" ::: "memory"); break;
-        case 5: asm volatile("cp.async.wait_group 5;" ::: "memory"); break;
-        case 6: asm volatile("cp.async.wait_group 6;" ::: "memory"); break;
-        default: asm volatile("cp.async.wait_group 7;" ::: "memory"); break;
-    }
-}
-
-// L2 policies: a staged gradient row is written in phase A and read once in phase B of the same step -- it should
-// stay in L2 in between (evict_last) and leave right after (evict_first), while the table rows stream through.
-__device__ __forceinline__ uint64_t l2_policy_evict_last() {
-    uint64_t p;
-    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-    return p;
-}
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-    uint64_t p;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
-    return p;
-}
-__device__ __forceinline__ void st_v4_hint(float* p, const float4& v, uint64_t pol) {
-    asm volatile("st.global.L2::cache_hint.v4.f32 [%0], {%1, %2, %3, %4}, %5;" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z),
-                 "f"(v.w), "l"(pol)
-                 : "memory");
-}
-__device__ __forceinline__ void sh_cp_async16_hint(void* smem, const void* gmem, uint64_t pol) {
-    const unsigned sa = (unsigned)__cvta_generic_to_shared(smem);
-    asm volatile("cp.async.cg.shared.global.L2::cache_hint [%0], [%1], 16, %2;" ::"r"(sa), "l"(gmem), "l"(pol) : "memory");
-}
-
 template <int IT>
 constexpr int shard_threads() { return IT <= 2 ? 512 : 256; }
 template <int IT>
@@ -476,34 +439,15 @@ constexpr size_t shard_smem_bytes() { return (size_t)shard_threads<IT>() * shard
 //     sequentially-consistent __threadfence_system() of a last-CTA-posts-flags scheme.
 // Arrivals are never reset across launches: the target only depends on how many barriers the group has passed,
 // e * CTAs-per-rank * world.
-__device__ __forceinline__ void red_relaxed_sys(unsigned* p) {
-    asm volatile("red.relaxed.sys.global.add.u32 [%0], 1;" ::"l"(p) : "memory");
-}
-__device__ __forceinline__ void red_relaxed_gpu(unsigned* p) {
-    asm volatile("red.relaxed.gpu.global.add.u32 [%0], 1;" ::"l"(p) : "memory");
-}
-__device__ __forceinline__ unsigned ld_acquire_sys(const unsigned* p) {
-    unsigned v;
-    asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ unsigned ld_acquire_gpu(const unsigned* p) {
-    unsigned v;
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void fence_acq_rel_sys() { asm volatile("fence.acq_rel.sys;" ::: "memory"); }
-__device__ __forceinline__ void fence_acq_rel_gpu() { asm volatile("fence.acq_rel.gpu;" ::: "memory"); }
-
 __device__ __forceinline__ void spin_until(const ShardCtx& C, const unsigned* cnt, unsigned target, bool sys,
                                            unsigned long long timeout_ns) {
     volatile int* status = C.status;
-    const unsigned long long t0 = shard_now_ns();
+    const unsigned long long t0 = global_ns();
     unsigned spins = 0;
     while ((int)((sys ? ld_relaxed_sys(cnt) : ld_relaxed_gpu(cnt)) - target) < 0) {
         if ((++spins & 1023u) == 0) {
             if (*status != 0) break;
-            if (shard_now_ns() - t0 > timeout_ns) {
+            if (global_ns() - t0 > timeout_ns) {
                 atomicExch(C.status, 1);
                 break;
             }
@@ -535,55 +479,6 @@ __device__ __forceinline__ void cross_wait(const ShardCtx& C, unsigned e, unsign
         if (sys) (void)ld_acquire_sys(mine); else (void)ld_acquire_gpu(mine);
     }
     __syncthreads();
-}
-
-template <int KIND, int IT>
-__device__ __forceinline__ void sh_update_store(const trs_table& t, size_t roff, int nch, int gl, int G_,
-                                                const OptScalars& o, float scale, Row<4, IT>& p, Row<4, IT>& s0,
-                                                Row<4, IT>& s1, const Row<4, IT>& g) {
-    OptScalars ok = o;
-    ok.kind = KIND;  // compile-time optimizer: opt_update's branches fold
-#pragma unroll
-    for (int a = 0; a < IT; ++a)
-#pragma unroll
-        for (int b = 0; b < 4; ++b) opt_update(ok, scale, g.c[a][b], p.c[a][b], s0.c[a][b], s1.c[a][b]);
-#pragma unroll
-    for (int a = 0; a < IT; ++a) {
-        const int c = gl + a * G_;
-        if (c < nch) {
-            p.c[a].st(t.emb + roff + (size_t)c * 4);
-            if (KIND != TRS_OPT_SGD) s0.c[a].st(t.emb_s0 + roff + (size_t)c * 4);
-            if (KIND == TRS_OPT_SPARSE_ADAM) s1.c[a].st(t.emb_s1 + roff + (size_t)c * 4);
-        }
-    }
-}
-
-// ---- bulk async copies (TMA engine, no tensor map) completing on an mbarrier: the cross-step prefetch ---------
-__device__ __forceinline__ uint32_t sh_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void sh_mbar_init(uint64_t* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(sh_smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void sh_mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.expect_tx.relaxed.cta.shared::cta.b64 [%0], %1;" ::"r"(sh_smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void sh_mbar_arrive(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(sh_smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ bool sh_mbar_try_wait(uint64_t* bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(sh_smem_u32(bar)), "r"(parity)
-        : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ void sh_bulk_g2s(void* smem_dst, const void* gsrc, uint32_t bytes, uint64_t* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(sh_smem_u32(smem_dst)), "l"(gsrc), "r"(bytes), "r"(sh_smem_u32(bar))
-                 : "memory");
 }
 
 // samples per row group whose item rows are fetched a step ahead (IT == 1 only: shared memory)
@@ -619,9 +514,9 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
     static_assert(!PFS || (PFS > SBA && PFS <= 2 * SBA), "round layout");
     __shared__ ShardCtx C;
     __shared__ float s_loss[NT / 32];
-    extern __shared__ __align__(128) unsigned char sh_smem[];
-    float4* rows = reinterpret_cast<float4*>(sh_smem);  // [slot][IT][NT]
-    unsigned char* pf_rows = sh_smem + shard_smem_bytes<IT>();             // [GPB][PFS][2][ROWB]
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    float4* rows = reinterpret_cast<float4*>(smem_raw);  // [slot][IT][NT]
+    unsigned char* pf_rows = smem_raw + shard_smem_bytes<IT>();             // [GPB][PFS][2][ROWB]
     unsigned char* pf_bias = pf_rows + (size_t)GPB * PFS * 2 * ROWB;       // [GPB][PFS][2][16]
     uint64_t* pf_bars = reinterpret_cast<uint64_t*>(pf_bias + (size_t)GPB * PFS * 2 * 16);  // [GPB]
 
@@ -635,8 +530,8 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
     uint64_t* const my_bar = pf_bars + g_in_cta;
     unsigned char* const my_pf_rows = pf_rows + (size_t)g_in_cta * PFS * 2 * ROWB;
     unsigned char* const my_pf_bias = pf_bias + (size_t)g_in_cta * PFS * 2 * 16;
-    if (PFS && gl == 0) sh_mbar_init(my_bar, 1);
-    if (PFS) asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    if (PFS && gl == 0) mbar_init(my_bar, 1);
+    if (PFS) fence_barrier_init();
     __syncthreads();
     const uint32_t W = (uint32_t)C.world;
     const bool wpow2 = (W & (W - 1u)) == 0u;
@@ -667,23 +562,25 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
 #pragma unroll
         for (int a = 0; a < IT; ++a) {
             const int ch = gl + a * G;
-            if (ch < nch) sh_cp_async16(slot(j, a), base + (size_t)ch * 4);
+            if (ch < nch) cp_async16(slot(j, a), base + (size_t)ch * 4);
         }
     };
     auto copy_region = [&](int j, const float* base) {
 #pragma unroll
         for (int a = 0; a < IT; ++a) {
             const int ch = gl + a * G;
-            if (ch < nch) sh_cp_async16(my_pf_rows + (size_t)j * ROWB + ch * 16, base + (size_t)ch * 4);
+            if (ch < nch) cp_async16(my_pf_rows + (size_t)j * ROWB + ch * 16, base + (size_t)ch * 4);
         }
     };
     auto ld_row = [&](const float* base) { return load_row_cg<4, G, IT>(base, nch, gl); };
+    // L2 policies: a staged gradient row is written in phase A and read once in phase B of the same step -- it should
+    // stay in L2 in between (evict_last) and leave right after (evict_first), while the table rows stream through.
     const uint64_t pol_keep = l2_policy_evict_last(), pol_drop = l2_policy_evict_first();
     auto copy_row_drop = [&](int j, const float* base) {  // a row nobody reads again: out of L2 first
 #pragma unroll
         for (int a = 0; a < IT; ++a) {
             const int ch = gl + a * G;
-            if (ch < nch) sh_cp_async16_hint(slot(j, a), base + (size_t)ch * 4, pol_drop);
+            if (ch < nch) cp_async16_hint(slot(j, a), base + (size_t)ch * 4, pol_drop);
         }
     };
     const trs_table& tU = C.user[me];
@@ -781,7 +678,7 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
         float* const my_stage_i = C.stage_i[me] + po;
         const float* const my_stage_b = C.stage_b[me] + po;
         unsigned long long* tr = C.trace ? C.trace + ((size_t)si * cpr + c) * 8 : nullptr;
-        if (tr && threadIdx.x == 0) tr[0] = shard_now_ns();
+        if (tr && threadIdx.x == 0) tr[0] = global_ns();
 
         // ------------------------------ phase A ------------------------------------------
         {   // this step's phase-B lists (sorted keys and slots, streamed from HBM exactly once) -> L2 now: a round's
@@ -792,7 +689,7 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
                                  : t < 2 * lu ? (const char*)(C.uval + lo)
                                  : t < 2 * lu + li ? (const char*)(C.ikey + 2 * lo) : (const char*)(C.ival + 2 * lo);
                 const int line = t < lu ? t : t < 2 * lu ? t - lu : t < 2 * lu + li ? t - 2 * lu : t - 2 * lu - li;
-                asm volatile("prefetch.global.L2 [%0];" ::"l"(base + (size_t)line * 128));
+                prefetch_l2(base + (size_t)line * 128);
             }
         }
         // hinge terms: one per regular-round sample, added up in sample order afterwards (the order in which the two
@@ -801,8 +698,7 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
 #pragma unroll
         for (int i = 0; i < 2 * SBA; ++i) hreg[i] = 0.f;
         if (PFS && pf_live) {  // rows fetched while the previous step's owners were updating: landed?
-            while (!sh_mbar_try_wait(my_bar, pf_parity)) {
-            }
+            mbar_wait(my_bar, pf_parity);
             pf_parity ^= 1u;
         }
         // One sample: scores, hinge, gradient rows.  linear.py:78: s = <u, v> + b_u + b_i; loss.py:7-9:
@@ -846,11 +742,13 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
             }
             if (bf & SAMP_USER_SINGLE) {
                 Row<4, IT> p = xu, s0, s1;
-#pragma unroll
-                for (int a = 0; a < IT; ++a) s0.c[a] = s1.c[a] = Vec<4>::zero();
+                row_zero(s0);
+                row_zero(s1);
                 if (KIND != TRS_OPT_SGD) s0 = slot_row(su_slot + 1);
                 if (KIND == TRS_OPT_SPARSE_ADAM) s1 = slot_row(su_slot + 2);
-                sh_update_store<KIND, IT>(C.user[qu], (size_t)lu * dim, nch, gl, G, opt, scale, p, s0, s1, gu);
+                OptScalars ok = opt;
+                ok.kind = KIND;  // compile-time optimizer: opt_update's branches fold
+                update_store_row<4, G, IT>(C.user[qu], (size_t)lu * dim, nch, gl, ok, scale, p, s0, s1, gu);
             } else {
                 float* du = C.stage_u[qu] + po + (size_t)b * dim;
 #pragma unroll
@@ -866,10 +764,10 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
         // samples) and the overflow rounds.
         for (int rr = 0;; ++rr) {
             if (wait_pending && (rr == NREG || !overlap)) {  // every warp of the CTA comes through here once per step
-                if (tr && threadIdx.x == 0) tr[5] = shard_now_ns();
+                if (tr && threadIdx.x == 0) tr[5] = global_ns();
                 cross_wait(C, sync_epoch + bar_no, (unsigned)cpr, timeout_ns);
                 wait_pending = false;
-                if (tr && threadIdx.x == 0) tr[6] = shard_now_ns();
+                if (tr && threadIdx.x == 0) tr[6] = global_ns();
             }
             const bool late = rr >= NREG;            // pass 1 / overflow
             const int rnd = late ? rr - NREG : rr;
@@ -930,11 +828,11 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
                             }
                         }
                     }
-                    sh_cp_async_commit();
+                    cp_async_commit();
                 }
 #pragma unroll
                 for (int i = 0; i < SBA; ++i) {
-                    sh_cp_async_wait(SBA - 1 - i);
+                    cp_async_wait(SBA - 1 - i);
                     const uint32_t bf = __shfl_sync(0xffffffffu, cur.b[i / G], i % G, G);
                     const uint32_t q = __shfl_sync(0xffffffffu, cur.q[i / G], i % G, G);
                     const uint32_t lu = __shfl_sync(0xffffffffu, cur.lu[i / G], i % G, G);
@@ -986,11 +884,11 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
                             if (lin) bias_r[i] = __ldcg(lin + lrow);
                         }
                     }
-                    sh_cp_async_commit();
+                    cp_async_commit();
                 }
 #pragma unroll
                 for (int i = 0; i < SBO; ++i) {
-                    sh_cp_async_wait(SBO - 1 - i);
+                    cp_async_wait(SBO - 1 - i);
                     const uint32_t bf = __shfl_sync(0xffffffffu, cur.b[i / G], i % G, G);
                     const uint32_t q = __shfl_sync(0xffffffffu, cur.q[i / G], i % G, G);
                     const uint32_t lu = __shfl_sync(0xffffffffu, cur.lu[i / G], i % G, G);
@@ -1036,12 +934,12 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
 #pragma unroll
             for (int w = 0; w < NT / 32; ++w) H += s_loss[w];
             C.loss_part[(size_t)si * cpr + c] = H;
-            if (tr) tr[1] = shard_now_ns();
+            if (tr) tr[1] = global_ns();
         }
         ++bar_no;
         cross_arrive(C, true);
         cross_wait(C, sync_epoch + bar_no, (unsigned)cpr, timeout_ns);
-        if (tr && threadIdx.x == 0) tr[2] = shard_now_ns();
+        if (tr && threadIdx.x == 0) tr[2] = global_ns();
 
         // ------------------------------ phase B ------------------------------------------
         // First the NEXT step's item rows: every clean one (not updated by this step, plan flag) of my group's first
@@ -1063,21 +961,21 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
                         const bool fp = !(bf & SAMP_DIRTY_POS), fn = !(bf & SAMP_DIRTY_NEG);
                         const uint32_t per = (uint32_t)dim * 4u + (TP.lin ? 16u : 0u);
                         const uint32_t bytes = (fp ? per : 0u) + (fn ? per : 0u);
-                        if (bytes) sh_mbar_expect_tx(my_bar, bytes);
+                        if (bytes) mbar_expect_tx(my_bar, bytes);
                         const int j = (round_lo(r) + i) * 2;
                         if (fp) {
-                            sh_bulk_g2s(my_pf_rows + (size_t)j * ROWB, TP.emb + (size_t)recN[r].lp[z] * dim, (uint32_t)dim * 4u, my_bar);
-                            if (TP.lin) sh_bulk_g2s(my_pf_bias + (size_t)j * 16, TP.lin + (recN[r].lp[z] & ~3u), 16u, my_bar);
+                            bulk_g2s(my_pf_rows + (size_t)j * ROWB, TP.emb + (size_t)recN[r].lp[z] * dim, (uint32_t)dim * 4u, my_bar);
+                            if (TP.lin) bulk_g2s(my_pf_bias + (size_t)j * 16, TP.lin + (recN[r].lp[z] & ~3u), 16u, my_bar);
                         }
                         if (fn) {
-                            sh_bulk_g2s(my_pf_rows + (size_t)(j + 1) * ROWB, TN.emb + (size_t)recN[r].ln[z] * dim, (uint32_t)dim * 4u, my_bar);
-                            if (TN.lin) sh_bulk_g2s(my_pf_bias + (size_t)(j + 1) * 16, TN.lin + (recN[r].ln[z] & ~3u), 16u, my_bar);
+                            bulk_g2s(my_pf_rows + (size_t)(j + 1) * ROWB, TN.emb + (size_t)recN[r].ln[z] * dim, (uint32_t)dim * 4u, my_bar);
+                            if (TN.lin) bulk_g2s(my_pf_bias + (size_t)(j + 1) * 16, TN.lin + (recN[r].ln[z] & ~3u), 16u, my_bar);
                         }
                     }
                 }
             }
             __syncwarp();  // every expect_tx of the group precedes its one arrival
-            if (gl == 0) sh_mbar_arrive(my_bar);
+            if (gl == 0) mbar_arrive(my_bar);
             pf_live = true;
         }
         // Owned rows: a row group takes PB positions of the step's sorted list per round; only the first position of
@@ -1106,13 +1004,13 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
                         else { if (KIND == TRS_OPT_SPARSE_ADAM) bsc[i] = __ldcg(t.lin_s1 + key); }
                     }
                 }
-                sh_cp_async_commit();
+                cp_async_commit();
             }
             Desc cur = dB;
             if (p0 + gstride * PB < nP) fetch_descs(dB, lo, nU, nI, pb + gstride * PB, nP);
 #pragma unroll
             for (int i = 0; i < PB; ++i) {
-                sh_cp_async_wait(PB - 1 - i);
+                cp_async_wait(PB - 1 - i);
                 const uint32_t key = __shfl_sync(0xffffffffu, cur.key[i / G], i % G, G);
                 const uint32_t sf = __shfl_sync(0xffffffffu, cur.sf[i / G], i % G, G);
                 const bool it = (sf >> 31) != 0u;
@@ -1126,8 +1024,8 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
                 if (!(sf & (1u << 29))) continue;
                 const trs_table& t = it ? tI : tU;
                 Row<4, IT> g = slot_row(i * 4 + 0), p = slot_row(i * 4 + 1), s0, s1;
-#pragma unroll
-                for (int a = 0; a < IT; ++a) s0.c[a] = s1.c[a] = Vec<4>::zero();
+                row_zero(s0);
+                row_zero(s1);
                 if (KIND != TRS_OPT_SGD) s0 = slot_row(i * 4 + 2);
                 if (KIND == TRS_OPT_SPARSE_ADAM) s1 = slot_row(i * 4 + 3);
                 if (sf & (1u << 30)) {  // duplicates (rare under uniform ids): the rest of the run, in slot order
@@ -1139,34 +1037,25 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
                     for (int q = k + 1; q < n && __ldg(K + q) == key; ++q) {
                         const uint32_t v = __ldg(P + q) & 0x1FFFFFFFu;
                         const uint32_t j = it ? v : (__ldg(C.samp + lo + v) & SAMP_POS);
-                        const Row<4, IT> r = ld_row(stage + (size_t)j * dim);
-#pragma unroll
-                        for (int a = 0; a < IT; ++a)
-#pragma unroll
-                            for (int e = 0; e < 4; ++e) g.c[a][e] = __fadd_rn(g.c[a][e], r.c[a][e]);
+                        row_acc(g, ld_row(stage + (size_t)j * dim));
                         if (it && item_lin && gl == 0) gb = __fadd_rn(gb, __ldcg(my_stage_b + j));
                     }
                 }
-                sh_update_store<KIND, IT>(t, (size_t)key * dim, nch, gl, G, opt, scale, p, s0, s1, g);
-                if (it && item_lin && gl == 0) {
-                    OptScalars ok = opt;
-                    ok.kind = KIND;
-                    opt_update(ok, scale, gb, pl, l0, l1);
-                    t.lin[key] = pl;
-                    if (KIND != TRS_OPT_SGD) t.lin_s0[key] = l0;
-                    if (KIND == TRS_OPT_SPARSE_ADAM) t.lin_s1[key] = l1;
-                }
+                OptScalars ok = opt;
+                ok.kind = KIND;
+                update_store_row<4, G, IT>(t, (size_t)key * dim, nch, gl, ok, scale, p, s0, s1, g);
+                if (it && item_lin && gl == 0) update_store_lin(t, key, ok, scale, gb, pl, l0, l1);
             }
         }
         if (tr) {
             __syncthreads();
-            if (threadIdx.x == 0) tr[3] = shard_now_ns();
+            if (threadIdx.x == 0) tr[3] = global_ns();
         }
         // the owners' updates are done: arrive, and wait inside the next step's phase A (after its pass 0)
         ++bar_no;
         cross_arrive(C, false);
         wait_pending = true;
-        if (tr && threadIdx.x == 0) tr[4] = shard_now_ns();
+        if (tr && threadIdx.x == 0) tr[4] = global_ns();
     }
     if (wait_pending) cross_wait(C, sync_epoch + bar_no, (unsigned)cpr, timeout_ns);
 
@@ -1270,21 +1159,9 @@ extern "C" size_t trs_shard_plan_bytes(const trs_epoch* ep) {
     return shard_plan_layout(ep->n_samples, ep->batch).total;
 }
 
-static size_t shard_tmp_pairs_bytes(const trs_epoch* ep) {
-    return ((size_t)4 * ep->n_samples * sizeof(uint32_t) + 511) / 256 * 256;
-}
-static int route_tiles(const trs_epoch* ep) { return (int)((2ll * ep->batch + RT_TILE - 1) / RT_TILE); }
-
-static size_t dirty_bitmap_bytes(const trs_epoch* ep) {
-    bool exact;
-    const int lb = dirty_log2_bits(ep, (int64_t)1 << 40, &exact);  // the hashed size: an exact bitmap is never larger
-    return (((size_t)n_steps_of(ep) << lb) / 8 + 255) / 256 * 256;   // one for the item rows, one for the user rows
-}
-
 extern "C" size_t trs_shard_plan_tmp_bytes(const trs_epoch* ep) {
     if (!ep || ep->batch <= 0) return 0;
-    const size_t tile_cnt = ((size_t)n_steps_of(ep) * route_tiles(ep) * sizeof(uint32_t) + 255) / 256 * 256;
-    return shard_tmp_pairs_bytes(ep) + tile_cnt + (hist_bytes(ep) + 255) / 256 * 256 + 2 * dirty_bitmap_bytes(ep);
+    return shard_plan_tmp(ep).total;
 }
 
 extern "C" int trs_shard_plan_build(const trs_shard* sh, const trs_epoch* ep, void* plan, size_t plan_bytes,
@@ -1299,18 +1176,20 @@ extern "C" int trs_shard_plan_build(const trs_shard* sh, const trs_epoch* ep, vo
     if (ep->n_samples == 0) return TRS_OK;
     TRS_REQUIRE(n_steps_of(ep) <= 65535, "shard_plan_build: %lld steps in one call (limit 65535)", (long long)n_steps_of(ep));
     const ShardPlanLayout L = shard_plan_layout(ep->n_samples, ep->batch);
-    if (plan_bytes < L.total || tmp_bytes < trs_shard_plan_tmp_bytes(ep)) {
+    const ShardPlanTmp T = shard_plan_tmp(ep);
+    if (plan_bytes < L.total || tmp_bytes < T.total) {
         set_error("shard plan workspace too small: plan %zu < %zu or tmp %zu < %zu", plan_bytes, L.total, tmp_bytes,
-                  trs_shard_plan_tmp_bytes(ep));
+                  T.total);
         return TRS_ERR_WORKSPACE;
     }
     cudaStream_t st = (cudaStream_t)stream;
     char* P = (char*)plan;
+    char* Tm = (char*)tmp;
     const int64_t n = ep->n_samples, steps = n_steps_of(ep);
-    uint32_t* tkey = (uint32_t*)tmp;
-    uint32_t* tval = tkey + 2 * n;
-    uint32_t* tile_cnt = (uint32_t*)((char*)tmp + shard_tmp_pairs_bytes(ep));
-    uint32_t* hist = (uint32_t*)((char*)tile_cnt + ((size_t)steps * route_tiles(ep) * sizeof(uint32_t) + 255) / 256 * 256);
+    uint32_t* tkey = (uint32_t*)(Tm + T.tkey);
+    uint32_t* tval = (uint32_t*)(Tm + T.tval);
+    uint32_t* tile_cnt = (uint32_t*)(Tm + T.tile_cnt);
+    uint32_t* hist = (uint32_t*)(Tm + T.hist);
     uint32_t* samp_cnt = (uint32_t*)(P + L.samp_cnt);
     uint32_t* own_cnt = (uint32_t*)(P + L.own_cnt);
     uint32_t* samp = (uint32_t*)(P + L.samp);
@@ -1339,7 +1218,7 @@ extern "C" int trs_shard_plan_build(const trs_shard* sh, const trs_epoch* ep, vo
     {   // dirty flags of the rank's samples (see dirty_bitmap_kernel)
         bool exact;
         const int lb = dirty_log2_bits(ep, sh->n_items, &exact);
-        uint32_t* bitmap = (uint32_t*)((char*)hist + (hist_bytes(ep) + 255) / 256 * 256);
+        uint32_t* bitmap = (uint32_t*)(Tm + T.bitmap);
         TRS_CUDA(cudaMemsetAsync(bitmap, 0, ((size_t)steps << lb) / 8, st));
         dim3 g2((unsigned)((2ll * ep->batch + RT_TILE - 1) / RT_TILE), (unsigned)steps);
         dirty_bitmap_kernel<<<g2, RT_THREADS, 0, st>>>(ep->pos, ep->neg, n, ep->batch, bitmap, lb, exact);
@@ -1347,7 +1226,7 @@ extern "C" int trs_shard_plan_build(const trs_shard* sh, const trs_epoch* ep, vo
         dirty_mark_kernel<<<g1, RT_THREADS, 0, st>>>(ep->pos, ep->neg, n, ep->batch, bitmap, lb, exact, samp_cnt, samp);
         bool ex_unused;
         const int lbu = dirty_log2_bits(ep, (int64_t)1 << 40, &ex_unused);  // always hashed
-        uint32_t* ubitmap = (uint32_t*)((char*)bitmap + dirty_bitmap_bytes(ep));
+        uint32_t* ubitmap = (uint32_t*)(Tm + T.ubitmap);
         TRS_CUDA(cudaMemsetAsync(ubitmap, 0, ((size_t)steps << lbu) / 8, st));
         single_mark_kernel<<<g1, RT_THREADS, 0, st>>>((const uint32_t*)(P + L.ukey), (uint32_t*)(P + L.uval), own_cnt, samp,
                                                      ep->batch, ubitmap, lbu);
@@ -1438,8 +1317,6 @@ extern "C" int trs_shard_train_steps(const trs_shard* shards, int n_local, const
         c.loss_out = loss_sum_host[i];
         c.status = status;
         c.trace = g_shard_trace ? g_shard_trace + (size_t)i * n_steps * cpr * 8 : nullptr;
-        // the rank's own grid-barrier counter restarts with every launch (peers never touch it)
-        TRS_CUDA(cudaMemsetAsync(sh.sync[sh.rank], 0, 128, st));  // words 0 and 16
     }
     const ShardCtx* ctxs_dev = nullptr;
     if (n_local > 1) {  // emulation of a whole group on one GPU (tests): contexts travel through the workspace

@@ -34,34 +34,21 @@ segment_update_kernel(const __grid_constant__ trs_table t, int dim, const uint32
         Row<V, IT> g = load_row<V, G, IT>(grad + (size_t)P[k] * dim, nch, gl);
         float gl_sum = grad_lin ? grad_lin[P[k]] : 0.f;
         for (int q = k + 1; q < n && K[q] == key; ++q) {  // duplicates, in list order
-            const Row<V, IT> r = load_row<V, G, IT>(grad + (size_t)P[q] * dim, nch, gl);
-#pragma unroll
-            for (int a = 0; a < IT; ++a)
-#pragma unroll
-                for (int b = 0; b < V; ++b) g.c[a][b] = __fadd_rn(g.c[a][b], r.c[a][b]);
+            row_acc(g, load_row<V, G, IT>(grad + (size_t)P[q] * dim, nch, gl));
             if (grad_lin) gl_sum = __fadd_rn(gl_sum, grad_lin[P[q]]);
         }
         const size_t roff = (size_t)key * dim;
         Row<V, IT> p = load_row<V, G, IT>(t.emb + roff, nch, gl), s0, s1;
-#pragma unroll
-        for (int a = 0; a < IT; ++a) s0.c[a] = s1.c[a] = Vec<V>::zero();
+        row_zero(s0);
+        row_zero(s1);
         if (opt.kind != TRS_OPT_SGD) s0 = load_row<V, G, IT>(t.emb_s0 + roff, nch, gl);
         if (opt.kind == TRS_OPT_SPARSE_ADAM) s1 = load_row<V, G, IT>(t.emb_s1 + roff, nch, gl);
-#pragma unroll
-        for (int a = 0; a < IT; ++a)
-#pragma unroll
-            for (int b = 0; b < V; ++b) opt_update(opt, scale, g.c[a][b], p.c[a][b], s0.c[a][b], s1.c[a][b]);
-        store_row<V, G, IT>(t.emb + roff, nch, gl, p);
-        if (opt.kind != TRS_OPT_SGD) store_row<V, G, IT>(t.emb_s0 + roff, nch, gl, s0);
-        if (opt.kind == TRS_OPT_SPARSE_ADAM) store_row<V, G, IT>(t.emb_s1 + roff, nch, gl, s1);
+        update_store_row<V, G, IT>(t, roff, nch, gl, opt, scale, p, s0, s1, g);
         if (grad_lin && t.lin && gl == 0) {
             float pl = t.lin[key], l0 = 0.f, l1 = 0.f;
             if (opt.kind != TRS_OPT_SGD) l0 = t.lin_s0[key];
             if (opt.kind == TRS_OPT_SPARSE_ADAM) l1 = t.lin_s1[key];
-            opt_update(opt, scale, gl_sum, pl, l0, l1);
-            t.lin[key] = pl;
-            if (opt.kind != TRS_OPT_SGD) t.lin_s0[key] = l0;
-            if (opt.kind == TRS_OPT_SPARSE_ADAM) t.lin_s1[key] = l1;
+            update_store_lin(t, key, opt, scale, gl_sum, pl, l0, l1);
         }
     }
 }

@@ -1,63 +1,19 @@
-// tc.cuh -- sm_100a tensor-core plumbing written as inline PTX: mbarrier, TMA (cp.async.bulk.tensor),
-// tcgen05 (alloc / mma / commit / ld) and the shared-memory / instruction descriptors of
-// tcgen05.mma.kind::f16.  Used by gemm.cu (MLP tower) and topk.cu (predict).
+// tc.cuh -- sm_100a tensor-core plumbing written as inline PTX: TMA tensor loads (cp.async.bulk.tensor),
+// tcgen05 (alloc / mma / commit / ld / st) and the shared-memory / instruction descriptors of
+// tcgen05.mma.kind::f16; the mbarriers they complete on are in ptx.cuh.  Used by gemm.cu (MLP tower) and
+// topk.cu (predict).
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
 
 #include "common.cuh"
+#include "ptx.cuh"
 
 namespace trs {
 namespace tc {
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-// ---- mbarrier ---------------------------------------------------------------------------------
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void fence_barrier_init() {
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes)
-                 : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    return ok != 0;
-}
-// Non-suspending poll: try_wait may park the warp for a hardware time slice when the phase is not complete at
-// the first look; on a hand-off that completes within a few hundred cycles that slice is the critical path.
-__device__ __forceinline__ void mbar_wait_spin(uint64_t* bar, uint32_t parity) {
-    uint32_t ok;
-    do {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok)
-            : "r"(smem_u32(bar)), "r"(parity)
-            : "memory");
-    } while (!ok);
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-    while (!mbar_try_wait(bar, parity)) {
-    }
-}
-
 // ---- TMA ----------------------------------------------------------------------------------------
+__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* m) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(m) : "memory");
 }

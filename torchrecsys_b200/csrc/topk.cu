@@ -63,11 +63,7 @@ struct TopkDev {
 };
 constexpr int TK_TRACE_TILES = 1024;  // traced tiles: [trace_t0, trace_t0 + TILES)
 
-__device__ __forceinline__ uint32_t float_key(float x) {  // order-preserving map float -> uint32
-    const uint32_t b = __float_as_uint(x);
-    return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-}
-__device__ __forceinline__ float key_float(uint32_t k) {
+__device__ __forceinline__ float key_float(uint32_t k) {  // inverse of float_key (common.cuh)
     return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
 }
 
@@ -173,14 +169,14 @@ topk_score_kernel(const __grid_constant__ CUtensorMap tmap_v,
     if (warp == 0 && lane == 0) {
         tc::tma_prefetch_desc(&tmap_v);
         for (int s = 0; s < g.stages; ++s) {
-            tc::mbar_init(&full[s], 1);
-            tc::mbar_init(&empty[s], 1);
+            mbar_init(&full[s], 1);
+            mbar_init(&empty[s], 1);
         }
         for (int b = 0; b < 2; ++b) {
-            tc::mbar_init(&acc_full[b], 1);
-            tc::mbar_init(&acc_empty[b], 4);  // one arrival per epilogue warp
+            mbar_init(&acc_full[b], 1);
+            mbar_init(&acc_empty[b], 4);  // one arrival per epilogue warp
         }
-        tc::fence_barrier_init();
+        fence_barrier_init();
     }
     if (warp == 1) tc::tmem_alloc(tmem_slot, TK_TMEM_COLS);
     tc::tc_fence_before();
@@ -230,10 +226,10 @@ topk_score_kernel(const __grid_constant__ CUtensorMap tmap_v,
                     __nanosleep(500);
                 }
             }
-            tc::mbar_wait(&empty[s], ph ^ 1u);
+            mbar_wait(&empty[s], ph ^ 1u);
             if (tracing && lane == 0 && t >= g.trace_t0 && t < g.trace_t0 + TK_TRACE_TILES) g.trace[(t - g.trace_t0) * 8 + 0] = clock64();
             if (tc::elect_one()) {
-                tc::mbar_arrive_expect_tx(&full[s], g.nbox * TK_BOX_BYTES);
+                mbar_arrive_expect_tx(&full[s], g.nbox * TK_BOX_BYTES);
                 for (int b = 0; b < g.nbox; ++b)
                     tc::tma_load_2d(sB + (s * g.nbox + b) * TK_BOX_BYTES, &tmap_v, &full[s], b * 64, (tile0 + t) * TK_BN);
             }
@@ -249,9 +245,9 @@ topk_score_kernel(const __grid_constant__ CUtensorMap tmap_v,
             if (s == g.stages) { s = 0; ph ^= 1u; }
             const int buf = t & 1;
             const uint32_t bph = (uint32_t)(t >> 1) & 1u;
-            tc::mbar_wait(&acc_empty[buf], bph ^ 1u);
+            mbar_wait(&acc_empty[buf], bph ^ 1u);
             if (tracing && lane == 0 && t >= g.trace_t0 && t < g.trace_t0 + TK_TRACE_TILES) g.trace[(t - g.trace_t0) * 8 + 1] = clock64();
-            tc::mbar_wait(&full[s], ph);
+            mbar_wait(&full[s], ph);
             if (tracing && lane == 0 && t >= g.trace_t0 && t < g.trace_t0 + TK_TRACE_TILES) g.trace[(t - g.trace_t0) * 8 + 2] = clock64();
             tc::tc_fence_after();
             if (tc::elect_one()) {
@@ -284,7 +280,7 @@ topk_score_kernel(const __grid_constant__ CUtensorMap tmap_v,
         for (int t = 0; t < ntiles; ++t) {
             const int buf = t & 1;
             const uint32_t bph = (uint32_t)(t >> 1) & 1u;
-            tc::mbar_wait(&acc_full[buf], bph);
+            mbar_wait(&acc_full[buf], bph);
             const bool etr = tracing && warp == 2 && lane == 0 && t >= g.trace_t0 && t < g.trace_t0 + TK_TRACE_TILES;
             if (etr) g.trace[(t - g.trace_t0) * 8 + 4] = clock64();
             tc::tc_fence_after();
@@ -304,7 +300,7 @@ topk_score_kernel(const __grid_constant__ CUtensorMap tmap_v,
                 if (half == TK_BATCHES - 1) {
                     tc::tc_fence_before();
                     __syncwarp();
-                    if (lane == 0) tc::mbar_arrive(&acc_empty[buf]);
+                    if (lane == 0) mbar_arrive(&acc_empty[buf]);
                     if (etr) g.trace[(t - g.trace_t0) * 8 + 5] = clock64();
                 }
                 if (valid && !over) {

@@ -26,6 +26,7 @@
 #include <stdlib.h>
 
 #include "plan.cuh"
+#include "ptx.cuh"
 #include "scorer.cuh"
 #include "train.cuh"
 
@@ -86,14 +87,6 @@ static StageLayout stage_layout(const trs_model* m, const trs_epoch* ep, int gri
 }
 
 // ---- small device helpers -------------------------------------------------------------------
-__device__ __forceinline__ unsigned long long global_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)::"memory");
-    return t;
-}
-__device__ __forceinline__ void prefetch_l2(const void* p) {
-    asm volatile("prefetch.global.L2 [%0];" ::"l"(p));
-}
 template <int V, int G, int IT>
 __device__ __forceinline__ void prefetch_row(const float* base, int nch, int gl) {
 #pragma unroll
@@ -101,18 +94,6 @@ __device__ __forceinline__ void prefetch_row(const float* base, int nch, int gl)
         const int c = gl + i * G;
         if (c < nch) prefetch_l2(base + (size_t)c * V);
     }
-}
-template <int V, int IT>
-__device__ __forceinline__ void row_zero(Row<V, IT>& r) {
-#pragma unroll
-    for (int i = 0; i < IT; ++i) r.c[i] = Vec<V>::zero();
-}
-template <int V, int IT>
-__device__ __forceinline__ void row_acc(Row<V, IT>& a, const Row<V, IT>& b) {  // a += b, unfused
-#pragma unroll
-    for (int i = 0; i < IT; ++i)
-#pragma unroll
-        for (int k = 0; k < V; ++k) a.c[i][k] = __fadd_rn(a.c[i][k], b.c[i][k]);
 }
 template <int V, int IT>
 __device__ __forceinline__ Row<V, IT> row_scaled_diff(float a, const Row<V, IT>& x,
@@ -143,13 +124,11 @@ __device__ __forceinline__ void grid_barrier(unsigned* counter, unsigned& target
     __syncthreads();
     target += gridDim.x;
     if (threadIdx.x == 0) {
-        asm volatile("fence.acq_rel.gpu;" ::: "memory");
-        asm volatile("red.relaxed.gpu.global.add.u32 [%0], 1;" ::"l"(counter) : "memory");
-        unsigned seen;
-        do {
-            asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(seen) : "l"(counter) : "memory");
-        } while ((int)(seen - target) < 0);
-        asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(seen) : "l"(counter) : "memory");
+        fence_acq_rel_gpu();
+        red_relaxed_gpu(counter);
+        while ((int)(ld_relaxed_gpu(counter) - target) < 0) {
+        }
+        (void)ld_acquire_gpu(counter);
     }
     __syncthreads();
 }
@@ -180,28 +159,12 @@ __device__ __forceinline__ SpaceRef resolve_space(int space, const trs_model& m,
     return r;
 }
 
-// update one row held in registers and write it (param + the optimizer's state tensors)
-template <int V, int G, int IT>
-__device__ __forceinline__ void update_store_row(const trs_table& t, size_t roff, int nch, int gl, const OptScalars& o,
-                                                 float scale, Row<V, IT>& p, Row<V, IT>& s0, Row<V, IT>& s1,
-                                                 const Row<V, IT>& g) {
-#pragma unroll
-    for (int a = 0; a < IT; ++a)
-#pragma unroll
-        for (int b = 0; b < V; ++b) opt_update(o, scale, g.c[a][b], p.c[a][b], s0.c[a][b], s1.c[a][b]);
-    store_row<V, G, IT>(t.emb + roff, nch, gl, p);
-    if (o.kind != TRS_OPT_SGD) store_row<V, G, IT>(t.emb_s0 + roff, nch, gl, s0);
-    if (o.kind == TRS_OPT_SPARSE_ADAM) store_row<V, G, IT>(t.emb_s1 + roff, nch, gl, s1);
-}
 // the width-1 companion of a row (bias / first-order weight), one thread
 __device__ __forceinline__ void update_lin(const trs_table& t, uint32_t key, const OptScalars& o, float scale, float g) {
     float pl = __ldcg(t.lin + key), l0 = 0.f, l1 = 0.f;
     if (o.kind != TRS_OPT_SGD) l0 = __ldcg(t.lin_s0 + key);
     if (o.kind == TRS_OPT_SPARSE_ADAM) l1 = __ldcg(t.lin_s1 + key);
-    opt_update(o, scale, g, pl, l0, l1);
-    t.lin[key] = pl;
-    if (o.kind != TRS_OPT_SGD) t.lin_s0[key] = l0;
-    if (o.kind == TRS_OPT_SPARSE_ADAM) t.lin_s1[key] = l1;
+    update_store_lin(t, key, o, scale, g, pl, l0, l1);
 }
 
 // ---- cp.async ring: per-thread prefetch slots in shared memory (V == 4 only) -------------------
@@ -233,14 +196,6 @@ template <int V, int IT>
 constexpr size_t train_smem_bytes() {
     return front_smem_bytes<V, IT>() + (size_t)train_threads<V, IT>() * (IT * V * 4 + 4) + MLIN_CAP * 4;
 }
-
-__device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
-    const unsigned sa = (unsigned)__cvta_generic_to_shared(smem);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa), "l"(gmem) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 template <int NT, int IT>
 struct Ring {
@@ -514,7 +469,7 @@ train_kernel(const __grid_constant__ trs_model m, const __grid_constant__ trs_ep
                 *reinterpret_cast<float4*>(s_mlin + i) = __ldcg(reinterpret_cast<const float4*>(m.meta[0].lin + i));
         }
         if (PFETCH) {
-            cp_async_wait<0>();  // my own copies of this step's rows (issued during the last phase B)
+            cp_async_wait(0);  // my own copies of this step's rows (issued during the last phase B)
             // the metadata rows of my first two samples (updated by every step: L2-hot) -> shared memory,
             // issued together so that the second sample does not wait for them again
             if (F > 0 && NET != TRS_NET_MLP) {
@@ -585,7 +540,7 @@ train_kernel(const __grid_constant__ trs_model m, const __grid_constant__ trs_ep
             for (int f = 0; f < MF; ++f) {
                 if (f < F) {
                     if (PFETCH && kk < PF && valid) {
-                        cp_async_wait<0>();
+                        cp_async_wait(0);
                         mp[f] = pf_row(kk, 9);
                         mn[f] = pf_row(kk, 10);
                     } else {
@@ -749,7 +704,7 @@ train_kernel(const __grid_constant__ trs_model m, const __grid_constant__ trs_ep
             }
             if (tracing && kk == 0) tr[10] = global_ns() + (unsigned long long)(__float_as_uint(gu.c[0][0] + gp.c[0][0]) & 1u);
             if (valid) {
-                if (slot) cp_async_wait<0>();  // my state-row copies of this sample
+                if (slot) cp_async_wait(0);  // my state-row copies of this sample
                 auto fused = [&](const trs_table& tb, size_t off, int t, Row<V, IT>& p, const Row<V, IT>& g) {
                     Row<V, IT> s0, s1;
                     row_zero(s0);
@@ -780,12 +735,9 @@ train_kernel(const __grid_constant__ trs_model m, const __grid_constant__ trs_ep
                 if ((!fn || meta_lin) && gl == 0) st.gbI[Bs + b] = gbn;
                 if (tracing && kk == 0) tr[11] = global_ns();
                 if (ldo) {  // lanes 0..2: the width-1 companions, state already in registers
-                    float pl = gl == 0 ? bu : (gl == 1 ? bip : bin);
+                    const float pl = gl == 0 ? bu : (gl == 1 ? bip : bin);
                     const float gg = gl == 0 ? gbu : (gl == 1 ? gbp : gbn);
-                    opt_update(opt, scale, gg, pl, lin_s0, lin_s1);
-                    ltab.lin[lkey] = pl;
-                    if (kind != TRS_OPT_SGD) ltab.lin_s0[lkey] = lin_s0;
-                    if (kind == TRS_OPT_SPARSE_ADAM) ltab.lin_s1[lkey] = lin_s1;
+                    update_store_lin(ltab, lkey, opt, scale, gg, pl, lin_s0, lin_s1);
                 }
             }
         }
@@ -853,7 +805,7 @@ train_kernel(const __grid_constant__ trs_model m, const __grid_constant__ trs_ep
         // gradients wait for the barrier
         if (tracing) tr[12] = global_ns();
         if (RINGED) {
-            cp_async_wait<0>();
+            cp_async_wait(0);
             if (!(dbg & 4)) {
                 for (int n = 0; n < RING; ++n) issue_state(n_items, n, lo);
             }
@@ -984,13 +936,9 @@ train_kernel(const __grid_constant__ trs_model m, const __grid_constant__ trs_ep
         }
         // finish the width-1 companion items
         if (lin_live) {
-            const trs_table& t = *lin_sp.t;
             const int c = (int)((lin_it.x >> 8) & 0xffu);
             for (int q = 1; q < c; ++q) lin_g = __fadd_rn(lin_g, __ldcg(lin_sp.stage_lin + lin_sp.P[lin_it.y + q]));
-            opt_update(opt, scale, lin_g, lin_p, lin_0, lin_1);
-            t.lin[lin_it.z] = lin_p;
-            if (kind != TRS_OPT_SGD) t.lin_s0[lin_it.z] = lin_0;
-            if (kind == TRS_OPT_SPARSE_ADAM) t.lin_s1[lin_it.z] = lin_1;
+            update_store_lin(*lin_sp.t, lin_it.z, opt, scale, lin_g, lin_p, lin_0, lin_1);
         }
         if (!(dbg & 32)) {  // more short segments than threads: the rest, one at a time
             for (int i = lin_i + NT * (int)gridDim.x; i < n_items; i += NT * (int)gridDim.x) {
@@ -1006,10 +954,10 @@ train_kernel(const __grid_constant__ trs_model m, const __grid_constant__ trs_ep
         if (tracing) tr[6] = global_ns();
         // short segments through the ring
         if (!(dbg & 4)) {
-            if (RINGED) cp_async_wait<0>();
+            if (RINGED) cp_async_wait(0);
             const int my_items = n_items > gid ? (n_items - gid + ngroups - 1) / ngroups : 0;
             for (int n = 0; n < my_items; ++n) {
-                if (RINGED && n >= RING) cp_async_wait<RING - 1>();
+                if (RINGED && n >= RING) cp_async_wait(RING - 1);
                 consume(items, n_items, n, lo, scale);
                 if (RINGED) {
                     issue_state(n_items, n + RING, lo);
@@ -1018,7 +966,7 @@ train_kernel(const __grid_constant__ trs_model m, const __grid_constant__ trs_ep
                     cp_async_commit();
                 }
             }
-            if (RINGED) cp_async_wait<0>();
+            if (RINGED) cp_async_wait(0);
         }
         if (tracing) tr[7] = global_ns();
         // descriptors of the next step's first work items
@@ -1036,7 +984,7 @@ train_kernel(const __grid_constant__ trs_model m, const __grid_constant__ trs_ep
         if (tracing) tr[3] = global_ns();
         if (!(dbg & 8)) grid_barrier(st.barrier, bar_target);
     }
-    cp_async_wait<0>();
+    cp_async_wait(0);
 
     // batch-mean hinge per step, summed over CTAs in a fixed order (deterministic)
     if (NET != TRS_NET_MLP && blockIdx.x == 0) {

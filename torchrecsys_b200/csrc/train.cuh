@@ -1,5 +1,7 @@
-// train.cuh -- what mlp.cu needs from train.cu: the reduce + update phase of the fused training kernel,
-// run on gradient rows the MLP backward staged itself.
+// train.cuh -- the row-wise optimizer step shared by the training kernels (train.cu, shard.cu, sharded.cu): the
+// update of one value, of a row held in registers and of a width-1 companion, each followed by the stores of the
+// parameter and its optimizer state; and what mlp.cu needs from train.cu: the reduce + update phase of the fused
+// training kernel, run on gradient rows the MLP backward staged itself.
 #pragma once
 #include "common.cuh"
 
@@ -38,6 +40,35 @@ __device__ __forceinline__ void opt_update(const OptScalars& o, float scale, flo
     } else {
         p = __fadd_rn(p, __fmul_rn(-scale, g));
     }
+}
+
+// update one row held in registers and write it (param + the optimizer's state tensors)
+template <int V, int G, int IT>
+__device__ __forceinline__ void update_store_row(const trs_table& t, size_t roff, int nch, int gl, const OptScalars& o,
+                                                 float scale, Row<V, IT>& p, Row<V, IT>& s0, Row<V, IT>& s1,
+                                                 const Row<V, IT>& g) {
+#pragma unroll
+    for (int a = 0; a < IT; ++a)
+#pragma unroll
+        for (int b = 0; b < V; ++b) opt_update(o, scale, g.c[a][b], p.c[a][b], s0.c[a][b], s1.c[a][b]);
+#pragma unroll
+    for (int a = 0; a < IT; ++a) {
+        const int c = gl + a * G;
+        if (c < nch) {
+            p.c[a].st(t.emb + roff + (size_t)c * V);
+            if (o.kind != TRS_OPT_SGD) s0.c[a].st(t.emb_s0 + roff + (size_t)c * V);
+            if (o.kind == TRS_OPT_SPARSE_ADAM) s1.c[a].st(t.emb_s1 + roff + (size_t)c * V);
+        }
+    }
+}
+// the same for the width-1 companion of a row (bias / first-order weight), one thread: value p and state s0 / s1
+// already loaded
+__device__ __forceinline__ void update_store_lin(const trs_table& t, uint32_t key, const OptScalars& o, float scale,
+                                                 float g, float p, float s0, float s1) {
+    opt_update(o, scale, g, p, s0, s1);
+    t.lin[key] = p;
+    if (o.kind != TRS_OPT_SGD) t.lin_s0[key] = s0;
+    if (o.kind == TRS_OPT_SPARSE_ADAM) t.lin_s1[key] = s1;
 }
 
 // fills OptScalars from the C-ABI optimizer description (beta / eps rounded to fp32 as torch's scalar ops do)
