@@ -2,6 +2,7 @@
 phase A, leaves barrier 1, finishes phase B, and how long the next phase A waits for the step's end (globaltimer stamps,
 trs_debug_shard_trace).
     python tools/shard_phases.py [--world 1] [--users 50000000] [--items 5000000] [--steps 12] [--it 2]   # one GPU
+        [--one-pass 0]   # one rank: the two-phase kernel instead of the one-pass one (trs_debug_shard_one_pass)
     torchrun --nproc-per-node N tools/shard_phases.py ...                                                 # real peers"""
 import argparse
 import ctypes as C
@@ -26,6 +27,7 @@ ap.add_argument("--batch", type=int, default=16384)
 ap.add_argument("--steps", type=int, default=12)
 ap.add_argument("--it", type=int, default=1)
 ap.add_argument("--overlap", type=int, default=-1)
+ap.add_argument("--one-pass", type=int, default=1)
 a = ap.parse_args()
 real = "RANK" in os.environ and int(os.environ.get("WORLD_SIZE", "1")) > 1
 local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -38,6 +40,7 @@ if real:
 L = _lib.lib()
 L.trs_debug_shard_chunks_per_lane(a.it)
 L.trs_debug_shard_overlap(a.overlap)
+L.trs_debug_shard_one_pass(a.one_pass)
 G, B = a.world, a.batch * a.world
 tr = ShardedLinearTrainer(a.users, a.items, a.dim, global_batch=B, device=dev, emulate_world=None if real else G)
 rng = np.random.default_rng(0)
@@ -59,7 +62,8 @@ t = buf.cpu().numpy().reshape(n_local, a.steps, cpr, 8).astype(np.float64) / 1e3
 names = ["A done", "bar1 left", "B done", "arrived at end"]
 if rank == 0:
     print(f"world {G}{' (real peers)' if real else ' (one GPU)'}, {cpr} CTAs per rank, batch/rank {a.batch}, "
-          f"{a.it} chunks per lane; microseconds from the step's earliest start")
+          f"{a.it} chunks per lane, {'one-pass' if L.trs_debug_shard_last_one_pass() == 1 else 'two-phase'} kernel; "
+          "microseconds from the step's earliest start")
 for r in range(n_local):
     if rank == 0:
         for s in range(max(2, a.steps - 4), a.steps):

@@ -54,6 +54,10 @@ struct ShardPlanLayout {
     size_t samp;      // [n]          step s at s*B: position b of each placed sample in the step, ascending
     size_t ukey, uval;  // [n]        sorted (local row, slot) pairs of the owned user lookups; step s at s*B
     size_t ikey, ival;  // [2n]       ... item lookups (slot b: positive of sample b, B_s + b: its negative); 2*s*B
+    // one rank only (item_single_*_kernel), for the one-pass kernel:
+    size_t cntB;        // [steps][2] own_cnt with the item count of ikeyB / ivalB
+    size_t iflag;       // [2n] bytes 1: the item row of lookup slot j is looked up once in the step; 2*s*B
+    size_t ikeyB, ivalB;  // [2n]     the pairs of ikey / ival whose row the step looks up more than once; 2*s*B
     size_t total;
 };
 static ShardPlanLayout shard_plan_layout(int64_t n, int B) {
@@ -72,6 +76,10 @@ static ShardPlanLayout shard_plan_layout(int64_t n, int B) {
     L.uval = take((size_t)n);
     L.ikey = take((size_t)2 * n);
     L.ival = take((size_t)2 * n);
+    L.cntB = take((size_t)2 * steps);
+    L.iflag = take(((size_t)2 * n + 3) / 4);
+    L.ikeyB = take((size_t)2 * n);
+    L.ivalB = take((size_t)2 * n);
     L.total = off;
     return L;
 }
@@ -348,6 +356,103 @@ user_dirty_mark_kernel(const int64_t* __restrict__ user, int B, uint32_t world, 
     }
 }
 
+// One rank: an item row looked up ONCE in a step has no other reader or writer in it either, so the one-pass kernel
+// updates it in phase A like a single user row.  Per step, item_single_count_kernel marks every item lookup slot single
+// or not (iflag) and counts the other pairs per tile; item_single_scatter_kernel copies those pairs, whole runs in order,
+// to ikeyB / ivalB: what phase B still does.  Grid (tiles of 2 B lookups, steps), as the route kernels.
+__device__ __forceinline__ bool item_pair_multi(const uint32_t* K, int n, int k) {
+    const uint32_t key = K[k];
+    return (k > 0 && K[k - 1] == key) || (k + 1 < n && K[k + 1] == key);
+}
+__global__ void __launch_bounds__(RT_THREADS)
+item_single_count_kernel(const uint32_t* __restrict__ ikey, const uint32_t* __restrict__ ival,
+                         const uint32_t* __restrict__ own_cnt, int B, uint8_t* __restrict__ iflag,
+                         uint32_t* __restrict__ tile_cnt, int tiles) {
+    __shared__ uint32_t s_w[RT_THREADS / 32];
+    const int64_t step = blockIdx.y;
+    const int tile = blockIdx.x;
+    const int n = (int)own_cnt[2 * step + 1];
+    const int64_t seg = 2 * step * (int64_t)B;
+    uint32_t cnt = 0;
+#pragma unroll
+    for (int r = 0; r < RT_ROWS; ++r) {
+        const int k = tile * RT_TILE + r * RT_THREADS + threadIdx.x;
+        if (k < n) {
+            const bool m = item_pair_multi(ikey + seg, n, k);
+            iflag[seg + ival[seg + k]] = m ? 0 : 1;
+            cnt += m ? 1u : 0u;
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+    if ((threadIdx.x & 31) == 0) s_w[threadIdx.x >> 5] = cnt;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        uint32_t t = 0;
+        for (int w = 0; w < RT_THREADS / 32; ++w) t += s_w[w];
+        tile_cnt[step * tiles + tile] = t;
+    }
+}
+__global__ void __launch_bounds__(RT_THREADS)
+item_single_scatter_kernel(const uint32_t* __restrict__ ikey, const uint32_t* __restrict__ ival,
+                           const uint32_t* __restrict__ own_cnt, int B, const uint32_t* __restrict__ tile_cnt, int tiles,
+                           uint32_t* __restrict__ ikeyB, uint32_t* __restrict__ ivalB, uint32_t* __restrict__ cntB) {
+    __shared__ uint32_t s_w[RT_THREADS / 32], s_b[RT_THREADS / 32], s_t[RT_THREADS / 32];
+    __shared__ uint32_t s_base;
+    const int64_t step = blockIdx.y;
+    const int tile = blockIdx.x;
+    const int n = (int)own_cnt[2 * step + 1];
+    const int64_t seg = 2 * step * (int64_t)B;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    {   // pairs kept by the tiles before mine (tile 0 also publishes the step's counts)
+        uint32_t before = 0, total = 0;
+        for (int t = threadIdx.x; t < tiles; t += RT_THREADS) {
+            const uint32_t c = tile_cnt[step * tiles + t];
+            total += c;
+            if (t < tile) before += c;
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            before += __shfl_xor_sync(0xffffffffu, before, o);
+            total += __shfl_xor_sync(0xffffffffu, total, o);
+        }
+        if (lane == 0) { s_b[warp] = before; s_t[warp] = total; }
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            uint32_t bb = 0, tt = 0;
+            for (int w = 0; w < RT_THREADS / 32; ++w) { bb += s_b[w]; tt += s_t[w]; }
+            s_base = bb;
+            if (tile == 0) {
+                cntB[2 * step] = own_cnt[2 * step];
+                cntB[2 * step + 1] = tt;
+            }
+        }
+        __syncthreads();
+    }
+    uint32_t run = s_base;
+    for (int r = 0; r < RT_ROWS; ++r) {
+        const int k = tile * RT_TILE + r * RT_THREADS + threadIdx.x;
+        const bool m = k < n && item_pair_multi(ikey + seg, n, k);
+        const uint32_t bal = __ballot_sync(0xffffffffu, m);
+        if (lane == 0) s_w[warp] = __popc(bal);
+        __syncthreads();
+        uint32_t wbase = 0, tot = 0;
+#pragma unroll
+        for (int w = 0; w < RT_THREADS / 32; ++w) {
+            const uint32_t c = s_w[w];
+            if (w < warp) wbase += c;
+            tot += c;
+        }
+        if (m) {
+            const uint32_t p = run + wbase + __popc(bal & ((1u << lane) - 1u));
+            ikeyB[seg + p] = ikey[seg + k];
+            ivalB[seg + p] = ival[seg + k];
+        }
+        run += tot;
+        __syncthreads();
+    }
+}
+
 // bits of a step's bitmap: 16x the item lookups of a step (~2 % false positives, see dirty_probe), or one bit per item if that is less
 static int dirty_log2_bits(const trs_epoch* ep, int64_t n_items, bool* exact) {
     int lb = 10;
@@ -420,6 +525,14 @@ struct ShardCtx {  // everything one (virtual) rank needs; copied to shared memo
     unsigned long long* trace;  // debug (trs_debug_shard_trace): [n_steps][cta_per_rank][8] globaltimer stamps, or NULL
 };
 
+// one-pass kernel, per sample: bit 0 / 1 of fl the positive / negative item row is looked up once in the step, its
+// local row, its slot (optimizer state in the next two) and its bias' optimizer state
+struct OneItems {
+    uint32_t fl, lp, ln;
+    int sp, sn;
+    float pl0, pl1, nl0, nl1;
+};
+
 template <int IT>
 constexpr int shard_threads() { return IT <= 2 ? 512 : 256; }
 template <int IT>
@@ -484,17 +597,24 @@ __device__ __forceinline__ void cross_wait(const ShardCtx& C, unsigned e, unsign
 // samples per row group whose item rows are fetched a step ahead (IT == 1 only: shared memory)
 template <int G, int IT>
 constexpr int shard_pf_samples() { return IT == 1 ? (G >= 8 ? 7 : 6) : 0; }  // what fits beside the 12 row slots in 227 KB
-template <int G, int IT>
+// The one-pass kernel (one rank, IT == 1) has no region: per row group ONE_S samples in flight, each with its three
+// rows and their optimizer states in ONE_SLOTS thread-private slots.  Two in flight measured 41.30 us per step at the
+// benchmark's shape against 41.54 us with three (one B200 at 1000 W, profiles/shard_r3.md)
+constexpr int ONE_S = 2, ONE_SLOTS = 9;
+template <int G, int IT, bool ONE>
 constexpr size_t shard_smem_total() {
     constexpr size_t NT = shard_threads<IT>(), GPB = NT / G, PFS = shard_pf_samples<G, IT>();
+    if (ONE) return NT * ONE_S * ONE_SLOTS * IT * 16;
     return shard_smem_bytes<IT>() + GPB * PFS * 2 * ((size_t)G * IT * 16 + 16) + GPB * 8;
 }
 
-template <int KIND, int G, int IT>
+template <int KIND, int G, int IT, bool ONE>
 __global__ void __launch_bounds__((shard_threads<IT>()), 1)
 shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __restrict__ ctxs, const int cpr,
                    const __grid_constant__ trs_epoch ep, const __grid_constant__ OptScalars opt, const int first_step,
-                   const int n_steps, const unsigned sync_epoch, const unsigned long long timeout_ns) {
+                   const int n_steps, const unsigned sync_epoch, const unsigned long long timeout_ns,
+                   const uint8_t* __restrict__ iflag) {
+    static_assert(!ONE || IT == 1, "the one-pass kernel takes one chunk per lane");
     constexpr int NT = shard_threads<IT>();
     constexpr int GPB = NT / G, GPW = 32 / G;
     constexpr int PB = shard_slots<IT>() / 4;  // owned rows in flight per row group (phase B): 4 slots each
@@ -504,13 +624,16 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
     // the 12 thread-private slots then hold the USER row with its optimizer state for SBA = 4 samples at a time:
     // regular rounds [0, SBA) and [SBA, PFS).  Samples beyond PFS (and every sample when there is no region, IT > 1)
     // go SBO = 2 per round with all five rows in the thread-private slots.
-    constexpr int PFS = shard_pf_samples<G, IT>();
+    // The loss adds a group's hinges in this layout's order whichever kernel runs: ordinals [0, HREG) one by one
+    // (then a + 0 per unused regular slot), the later ordinals in a sum of their own.
+    constexpr int HREG = shard_pf_samples<G, IT>();
+    constexpr int PFS = ONE ? 0 : HREG;
     constexpr int SBA = 4, SBO = 2;
     constexpr int NREG = PFS ? 2 : 0;          // regular rounds
     constexpr int NPR = NREG ? NREG : 1;       // rounds whose records are fetched a step ahead
     constexpr int RPL = (SBA + G - 1) / G;     // sample records a lane holds per round
     constexpr int ROWB = G * IT * 16;          // bytes of a region row slot
-    static_assert(shard_smem_total<G, IT>() + 2048 <= 227 * 1024, "shared memory budget");
+    static_assert(shard_smem_total<G, IT, ONE>() + 2048 <= 227 * 1024, "shared memory budget");
     static_assert(!PFS || (PFS > SBA && PFS <= 2 * SBA), "round layout");
     __shared__ ShardCtx C;
     __shared__ float s_loss[NT / 32];
@@ -621,6 +744,24 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
             }
         }
     };
+    // one-pass kernel: lane gl holds the record of my group's ordinal blk * G + gl; one rank, so a local row is the id.
+    // fl: bit 0 / 1 the positive / negative row is looked up once in the step (iflag at its lookup slot)
+    struct Rec1 { uint32_t b, lu, lp, ln, fl; };
+    auto fetch_one = [&](Rec1& R, int64_t lo_, int nS_, int blk) {
+        const int k = gfirst + (blk * G + gl) * gstride;
+        R.b = 0xFFFFFFFFu;
+        R.lu = R.lp = R.ln = R.fl = 0u;
+        if (k < nS_) {
+            const int Bs_ = (int)min((int64_t)ep.batch, ep.n_samples - lo_);
+            const uint32_t bf = __ldg(C.samp + lo_ + k);
+            const uint32_t b = bf & SAMP_POS;
+            R.b = bf;
+            R.lu = (uint32_t)__ldg(ep.user + lo_ + b);
+            R.lp = (uint32_t)__ldg(ep.pos + lo_ + b);
+            R.ln = (uint32_t)__ldg(ep.neg + lo_ + b);
+            R.fl = (uint32_t)__ldg(iflag + 2 * lo_ + b) | ((uint32_t)__ldg(iflag + 2 * lo_ + Bs_ + b) << 1);
+        }
+    };
     auto round_lo = [&](int r) { return r < NREG ? (r == 0 ? 0 : SBA) : PFS + SBO * (r - NREG); };
     auto round_n = [&](int r) { return r < NREG ? (r == 0 ? SBA : PFS - SBA) : SBO; };
     // ---- descriptors of a phase-B round: the owned lookups of a step are one list of positions, user space
@@ -653,12 +794,17 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
     };
 
     Rec recN[NPR];      // records of the next phase A's first NPR rounds
+    Rec1 recO;          // one-pass kernel: the current block of records (block 0 of the next phase A between steps)
     int nS_cur = 0;
     {
         const int64_t lo0 = (int64_t)first_step * ep.batch;
         nS_cur = (int)C.samp_cnt[first_step];
+        if constexpr (ONE) {
+            fetch_one(recO, lo0, nS_cur, 0);
+        } else {
 #pragma unroll
-        for (int r = 0; r < NPR; ++r) fetch_records(recN[r], lo0, nS_cur, gfirst + round_lo(r) * gstride, round_n(r));
+            for (int r = 0; r < NPR; ++r) fetch_records(recN[r], lo0, nS_cur, gfirst + round_lo(r) * gstride, round_n(r));
+        }
     }
     bool pf_live = false;     // the current step's region holds prefetched item rows (all but the dirty ones)
     uint32_t pf_parity = 0;
@@ -704,9 +850,11 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
         // One sample: scores, hinge, gradient rows.  linear.py:78: s = <u, v> + b_u + b_i; loss.py:7-9:
         // h = s- - s+ + 1, d/ds = [h >= 0] / B.  A user row that this step looks up ONCE (plan flag: no other sample of
         // the global batch reads or writes it, and its owner is this rank) is updated right here from its state rows
-        // in slots su_slot + 1 / + 2; every other gradient row goes to its owner's staging buffer.
+        // in slots su_slot + 1 / + 2; every other gradient row goes to its owner's staging buffer.  The one-pass kernel
+        // treats an item row that the step looks up once (oi.fl) the same way, from slots oi.sp / oi.sn + 1 / + 2.
         auto process = [&](bool valid, uint32_t bf, uint32_t q, uint32_t lu, const Row<4, IT>& xu, const Row<4, IT>& xp,
-                           const Row<4, IT>& xn, float bu, float bip, float bin, int su_slot, float& hinge) {
+                           const Row<4, IT>& xn, float bu, float bip, float bin, int su_slot, float& hinge,
+                           const OneItems& oi) {
             const float sp = (group_sum<G>(row_dot_partial(xu, xp)) + bu) + bip;
             const float sn = (group_sum<G>(row_dot_partial(xu, xn)) + bu) + bin;
             const float h = __fadd_rn(__fsub_rn(sn, sp), 1.0f);
@@ -718,27 +866,63 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
             float* dp = C.stage_i[qp] + po + (size_t)b * dim;
             float* dn = C.stage_i[qn] + po + (size_t)(Bs + b) * dim;
             Row<4, IT> gu;
+            if constexpr (ONE) {
+                // the gradient rows exactly as phase B would read them back from the staging buffer (no contraction)
+                Row<4, IT> gp, gn;
 #pragma unroll
-            for (int a = 0; a < IT; ++a) {
-                const int ch = gl + a * G;
-#pragma unroll
-                for (int e = 0; e < 4; ++e) gu.c[a][e] = g * (xn.c[a][e] - xp.c[a][e]);
-                if (ch < nch) {
-                    Vec<4> gp, gn;
+                for (int a = 0; a < IT; ++a)
 #pragma unroll
                     for (int e = 0; e < 4; ++e) {
-                        gp[e] = -g * xu.c[a][e];
-                        gn[e] = g * xu.c[a][e];
+                        gu.c[a][e] = g * (xn.c[a][e] - xp.c[a][e]);
+                        gp.c[a][e] = __fmul_rn(-g, xu.c[a][e]);
+                        gn.c[a][e] = __fmul_rn(g, xu.c[a][e]);
                     }
-                    if (hint_remote || (int)qp == me) st_v4_hint(dp + (size_t)ch * 4, gp.v, pol_keep);
-                    else gp.st(dp + (size_t)ch * 4);
-                    if (hint_remote || (int)qn == me) st_v4_hint(dn + (size_t)ch * 4, gn.v, pol_keep);
-                    else gn.st(dn + (size_t)ch * 4);
+                auto item_out = [&](bool single, uint32_t row, int sl, const Row<4, IT>& x, Row<4, IT>& gr, float* dst,
+                                    float gb, float pl, float l0, float l1, uint32_t bslot) {
+                    if (single) {
+                        Row<4, IT> p = x, s0, s1;
+                        row_zero(s0);
+                        row_zero(s1);
+                        if (KIND != TRS_OPT_SGD) s0 = slot_row(sl + 1);
+                        if (KIND == TRS_OPT_SPARSE_ADAM) s1 = slot_row(sl + 2);
+                        OptScalars ok = opt;
+                        ok.kind = KIND;
+                        update_store_row<4, G, IT>(tI, (size_t)row * dim, nch, gl, ok, scale, p, s0, s1, gr);
+                        if (item_lin && gl == 0) update_store_lin(tI, row, ok, scale, gb, pl, l0, l1);
+                    } else {
+#pragma unroll
+                        for (int a = 0; a < IT; ++a) {
+                            const int ch = gl + a * G;
+                            if (ch < nch) st_v4_hint(dst + (size_t)ch * 4, gr.c[a].v, pol_keep);
+                        }
+                        if (gl == 0) (C.stage_b[me] + po)[bslot] = gb;
+                    }
+                };
+                item_out(oi.fl & 1u, oi.lp, oi.sp, xp, gp, dp, -g, bip, oi.pl0, oi.pl1, b);
+                item_out(oi.fl & 2u, oi.ln, oi.sn, xn, gn, dn, g, bin, oi.nl0, oi.nl1, Bs + b);
+            } else {
+#pragma unroll
+                for (int a = 0; a < IT; ++a) {
+                    const int ch = gl + a * G;
+#pragma unroll
+                    for (int e = 0; e < 4; ++e) gu.c[a][e] = g * (xn.c[a][e] - xp.c[a][e]);
+                    if (ch < nch) {
+                        Vec<4> gp, gn;
+#pragma unroll
+                        for (int e = 0; e < 4; ++e) {
+                            gp[e] = -g * xu.c[a][e];
+                            gn[e] = g * xu.c[a][e];
+                        }
+                        if (hint_remote || (int)qp == me) st_v4_hint(dp + (size_t)ch * 4, gp.v, pol_keep);
+                        else gp.st(dp + (size_t)ch * 4);
+                        if (hint_remote || (int)qn == me) st_v4_hint(dn + (size_t)ch * 4, gn.v, pol_keep);
+                        else gn.st(dn + (size_t)ch * 4);
+                    }
                 }
-            }
-            if (gl == 0) {
-                (C.stage_b[qp] + po)[b] = -g;
-                (C.stage_b[qn] + po)[Bs + b] = g;
+                if (gl == 0) {
+                    (C.stage_b[qp] + po)[b] = -g;
+                    (C.stage_b[qn] + po)[Bs + b] = g;
+                }
             }
             if (bf & SAMP_USER_SINGLE) {
                 Row<4, IT> p = xu, s0, s1;
@@ -758,165 +942,283 @@ shard_train_kernel(const __grid_constant__ ShardCtx ctx0, const ShardCtx* __rest
                 }
             }
         };
-        // Two passes over the regular rounds.  Pass 0 takes the samples none of whose three rows the previous step's
-        // owners update (plan flags) BEFORE waiting for the barrier that ends the previous step: their rows are final,
-        // and their gradient rows go to the other copy of the staging buffers.  Then the wait, then pass 1 (the flagged
-        // samples) and the overflow rounds.
-        for (int rr = 0;; ++rr) {
-            if (wait_pending && (rr == NREG || !overlap)) {  // every warp of the CTA comes through here once per step
+        const OneItems no_items{};
+        if constexpr (ONE) {
+            // One pass over my group's samples in ordinal order (the loss order), after the wait for the previous
+            // step's end.  Sample o + ONE_S's rows start their trip (cp.async into slots ONE_SLOTS * j ..) before
+            // sample o runs: user, positive, negative row at + 0 / 3 / 6, each followed by its optimizer state when
+            // phase A updates that row.  Records come G samples at a time (Rec1); lane t & 3 holds scalar t of a
+            // sample in tv0 (t < 4) or tv1: 0 user bias, 1 / 2 positive / negative bias, 3 / 4 and 5 / 6 their states.
+            if (wait_pending) {
                 if (tr && threadIdx.x == 0) tr[5] = global_ns();
                 cross_wait(C, sync_epoch + bar_no, (unsigned)cpr, timeout_ns);
                 wait_pending = false;
                 if (tr && threadIdx.x == 0) tr[6] = global_ns();
             }
-            const bool late = rr >= NREG;            // pass 1 / overflow
-            const int rnd = late ? rr - NREG : rr;
-            const int o_lo = round_lo(rnd), n_r = round_n(rnd);
-            const int k0 = gfirst - goff + o_lo * gstride;
-            if (k0 >= nS) {  // warp-uniform
-                if (late) break;
-                continue;
-            }
-            const int kb = k0 + goff;
-            Rec cur;
-            if (rnd < NPR) {
-#pragma unroll
-                for (int r = 0; r < NPR; ++r)
-                    if (r == rnd) cur = recN[r];
-            } else {
-                fetch_records(cur, lo, nS, kb, n_r);
-            }
-            if (rnd < NREG) {
-                // ---- regular round: item rows in the region, user row + state in slots 3i .. 3i + 2 ----
-                if (late) {  // nothing flagged in the warp's groups: pass 0 did the whole round
-                    if (!overlap) continue;
-                    bool d = false;
-#pragma unroll
-                    for (int z = 0; z < RPL; ++z) d = d || (cur.b[z] != 0xFFFFFFFFu && (cur.b[z] & SAMP_DIRTY_ANY) != 0u);
-                    if (!__any_sync(0xffffffffu, d)) continue;
+            const int kw = gfirst - goff;  // the warp's first group: the trip count is warp-uniform
+            const int nord = kw < nS ? (nS - kw + gstride - 1) / gstride : 0;
+            int blk = 0;
+            uint32_t rb[ONE_S], ru[ONE_S], rp[ONE_S], rn[ONE_S], rf[ONE_S];
+            float tv0[ONE_S], tv1[ONE_S];
+            auto scalar = [&](int t, uint32_t lu, uint32_t lp, uint32_t ln, uint32_t fl) {
+                const bool p = t == 1 || t == 3 || t == 4;
+                const float* src = t == 0 ? tU.lin : (t <= 2 ? tI.lin : nullptr);
+                if (t >= 3 && item_lin && (fl & (p ? 1u : 2u))) {
+                    if ((t == 3 || t == 5) && KIND != TRS_OPT_SGD) src = tI.lin_s0;
+                    if ((t == 4 || t == 6) && KIND == TRS_OPT_SPARSE_ADAM) src = tI.lin_s1;
                 }
-                float bias_r[SBA];  // lane t < 3 holds the width-1 companion of lookup t (user, positive, negative)
+                return src ? __ldcg(src + (t == 0 ? lu : (p ? lp : ln))) : 0.f;
+            };
+            auto issue = [&](int o, int j) {
+                uint32_t bf = 0xFFFFFFFFu, lu = 0u, lp = 0u, ln = 0u, fl = 0u;
+                if (o < nord) {
+                    if (o / G != blk) {
+                        blk = o / G;
+                        fetch_one(recO, lo, nS, blk);
+                    }
+                    bf = __shfl_sync(0xffffffffu, recO.b, o % G, G);
+                    lu = __shfl_sync(0xffffffffu, recO.lu, o % G, G);
+                    lp = __shfl_sync(0xffffffffu, recO.lp, o % G, G);
+                    ln = __shfl_sync(0xffffffffu, recO.ln, o % G, G);
+                    fl = __shfl_sync(0xffffffffu, recO.fl, o % G, G);
+                }
+                rb[j] = bf;
+                ru[j] = lu;
+                rp[j] = lp;
+                rn[j] = ln;
+                rf[j] = fl;
+                tv0[j] = tv1[j] = 0.f;
+                if (bf != 0xFFFFFFFFu) {
+                    const int sl = j * ONE_SLOTS;
+                    copy_row(sl + 0, tU.emb + (size_t)lu * dim);
+                    if (bf & SAMP_USER_SINGLE) {
+                        if (KIND != TRS_OPT_SGD) copy_row(sl + 1, tU.emb_s0 + (size_t)lu * dim);
+                        if (KIND == TRS_OPT_SPARSE_ADAM) copy_row(sl + 2, tU.emb_s1 + (size_t)lu * dim);
+                    }
+                    copy_row(sl + 3, tI.emb + (size_t)lp * dim);
+                    if (fl & 1u) {
+                        if (KIND != TRS_OPT_SGD) copy_row(sl + 4, tI.emb_s0 + (size_t)lp * dim);
+                        if (KIND == TRS_OPT_SPARSE_ADAM) copy_row(sl + 5, tI.emb_s1 + (size_t)lp * dim);
+                    }
+                    copy_row(sl + 6, tI.emb + (size_t)ln * dim);
+                    if (fl & 2u) {
+                        if (KIND != TRS_OPT_SGD) copy_row(sl + 7, tI.emb_s0 + (size_t)ln * dim);
+                        if (KIND == TRS_OPT_SPARSE_ADAM) copy_row(sl + 8, tI.emb_s1 + (size_t)ln * dim);
+                    }
+                    if (gl < 4) {
+                        tv0[j] = scalar(gl, lu, lp, ln, fl);
+                        tv1[j] = scalar(gl + 4, lu, lp, ln, fl);
+                    }
+                }
+                cp_async_commit();
+            };
+            auto run = [&](int o, int j) {
+                const uint32_t bf = rb[j];
+                const bool valid = bf != 0xFFFFFFFFu;
+                const int sl = j * ONE_SLOTS;
+                Row<4, IT> xu, xp, xn;
+                if (valid) {
+                    xu = slot_row(sl + 0);
+                    xp = slot_row(sl + 3);
+                    xn = slot_row(sl + 6);
+                } else {
 #pragma unroll
-                for (int i = 0; i < SBA; ++i) {
-                    const uint32_t bf = __shfl_sync(0xffffffffu, cur.b[i / G], i % G, G);
-                    const uint32_t q = __shfl_sync(0xffffffffu, cur.q[i / G], i % G, G);
-                    const uint32_t lu = __shfl_sync(0xffffffffu, cur.lu[i / G], i % G, G);
-                    const uint32_t lp = __shfl_sync(0xffffffffu, cur.lp[i / G], i % G, G);
-                    const uint32_t ln = __shfl_sync(0xffffffffu, cur.ln[i / G], i % G, G);
-                    bias_r[i] = 0.f;
-                    if (i < n_r && bf != 0xFFFFFFFFu && (overlap ? ((bf & SAMP_DIRTY_ANY) != 0u) == late : !late)) {
-                        const int ord = o_lo + i;
-                        const bool have_p = pf_live && !(bf & SAMP_DIRTY_POS), have_n = pf_live && !(bf & SAMP_DIRTY_NEG);
-                        const trs_table& TU = C.user[q & 15u];
-                        const trs_table& TP = C.item[(q >> 4) & 15u];
-                        const trs_table& TN = C.item[(q >> 8) & 15u];
-                        copy_row(i * 3 + 0, TU.emb + (size_t)lu * dim);
-                        if (bf & SAMP_USER_SINGLE) {
-                            if (KIND != TRS_OPT_SGD) copy_row(i * 3 + 1, TU.emb_s0 + (size_t)lu * dim);
-                            if (KIND == TRS_OPT_SPARSE_ADAM) copy_row(i * 3 + 2, TU.emb_s1 + (size_t)lu * dim);
-                        }
-                        if (!have_p) copy_region(ord * 2 + 0, TP.emb + (size_t)lp * dim);
-                        if (!have_n) copy_region(ord * 2 + 1, TN.emb + (size_t)ln * dim);
-                        if (gl < 3) {
-                            const float* lin = gl == 0 ? TU.lin : (gl == 1 ? TP.lin : TN.lin);
-                            const uint32_t lrow = gl == 0 ? lu : (gl == 1 ? lp : ln);
-                            const bool have = gl == 1 ? have_p : (gl == 2 ? have_n : false);
-                            if (lin) {
-                                if (have) bias_r[i] = reinterpret_cast<const float*>(
-                                              my_pf_bias + (size_t)(ord * 2 + (gl - 1)) * 16)[lrow & 3u];
-                                else bias_r[i] = __ldcg(lin + lrow);
+                    for (int a = 0; a < IT; ++a) xu.c[a] = xp.c[a] = xn.c[a] = Vec<4>::zero();
+                }
+                const float bu = __shfl_sync(0xffffffffu, tv0[j], 0, G);
+                const float bip = __shfl_sync(0xffffffffu, tv0[j], 1, G);
+                const float bin = __shfl_sync(0xffffffffu, tv0[j], 2, G);
+                OneItems oi;
+                oi.fl = rf[j];
+                oi.lp = rp[j];
+                oi.ln = rn[j];
+                oi.sp = sl + 3;
+                oi.sn = sl + 6;
+                oi.pl0 = __shfl_sync(0xffffffffu, tv0[j], 3, G);
+                oi.pl1 = __shfl_sync(0xffffffffu, tv1[j], 0, G);
+                oi.nl0 = __shfl_sync(0xffffffffu, tv1[j], 1, G);
+                oi.nl1 = __shfl_sync(0xffffffffu, tv1[j], 2, G);
+                float hv = 0.f;
+                process(valid, bf, 0u, ru[j], xu, xp, xn, bu, bip, bin, sl, hv, oi);
+                if (valid) {
+                    if (o < HREG) hreg[0] += hv; else hover += hv;
+                }
+            };
+#pragma unroll
+            for (int j = 0; j < ONE_S; ++j) issue(j, j);
+            for (int o0 = 0; o0 < nord; o0 += ONE_S) {
+#pragma unroll
+                for (int j = 0; j < ONE_S; ++j) {
+                    cp_async_wait(ONE_S - 1);
+                    if (o0 + j < nord) run(o0 + j, j);
+                    issue(o0 + j + ONE_S, j);
+                }
+            }
+        } else {
+            // Two passes over the regular rounds.  Pass 0 takes the samples none of whose three rows the previous
+            // step's owners update (plan flags) BEFORE waiting for the barrier that ends the previous step: their rows
+            // are final, and their gradient rows go to the other copy of the staging buffers.  Then the wait, then
+            // pass 1 (the flagged samples) and the overflow rounds.
+            for (int rr = 0;; ++rr) {
+                if (wait_pending && (rr == NREG || !overlap)) {  // every warp of the CTA comes through here once per step
+                    if (tr && threadIdx.x == 0) tr[5] = global_ns();
+                    cross_wait(C, sync_epoch + bar_no, (unsigned)cpr, timeout_ns);
+                    wait_pending = false;
+                    if (tr && threadIdx.x == 0) tr[6] = global_ns();
+                }
+                const bool late = rr >= NREG;            // pass 1 / overflow
+                const int rnd = late ? rr - NREG : rr;
+                const int o_lo = round_lo(rnd), n_r = round_n(rnd);
+                const int k0 = gfirst - goff + o_lo * gstride;
+                if (k0 >= nS) {  // warp-uniform
+                    if (late) break;
+                    continue;
+                }
+                const int kb = k0 + goff;
+                Rec cur;
+                if (rnd < NPR) {
+#pragma unroll
+                    for (int r = 0; r < NPR; ++r)
+                        if (r == rnd) cur = recN[r];
+                } else {
+                    fetch_records(cur, lo, nS, kb, n_r);
+                }
+                if (rnd < NREG) {
+                    // ---- regular round: item rows in the region, user row + state in slots 3i .. 3i + 2 ----
+                    if (late) {  // nothing flagged in the warp's groups: pass 0 did the whole round
+                        if (!overlap) continue;
+                        bool d = false;
+#pragma unroll
+                        for (int z = 0; z < RPL; ++z) d = d || (cur.b[z] != 0xFFFFFFFFu && (cur.b[z] & SAMP_DIRTY_ANY) != 0u);
+                        if (!__any_sync(0xffffffffu, d)) continue;
+                    }
+                    float bias_r[SBA];  // lane t < 3 holds the width-1 companion of lookup t (user, positive, negative)
+#pragma unroll
+                    for (int i = 0; i < SBA; ++i) {
+                        const uint32_t bf = __shfl_sync(0xffffffffu, cur.b[i / G], i % G, G);
+                        const uint32_t q = __shfl_sync(0xffffffffu, cur.q[i / G], i % G, G);
+                        const uint32_t lu = __shfl_sync(0xffffffffu, cur.lu[i / G], i % G, G);
+                        const uint32_t lp = __shfl_sync(0xffffffffu, cur.lp[i / G], i % G, G);
+                        const uint32_t ln = __shfl_sync(0xffffffffu, cur.ln[i / G], i % G, G);
+                        bias_r[i] = 0.f;
+                        if (i < n_r && bf != 0xFFFFFFFFu && (overlap ? ((bf & SAMP_DIRTY_ANY) != 0u) == late : !late)) {
+                            const int ord = o_lo + i;
+                            const bool have_p = pf_live && !(bf & SAMP_DIRTY_POS), have_n = pf_live && !(bf & SAMP_DIRTY_NEG);
+                            const trs_table& TU = C.user[q & 15u];
+                            const trs_table& TP = C.item[(q >> 4) & 15u];
+                            const trs_table& TN = C.item[(q >> 8) & 15u];
+                            copy_row(i * 3 + 0, TU.emb + (size_t)lu * dim);
+                            if (bf & SAMP_USER_SINGLE) {
+                                if (KIND != TRS_OPT_SGD) copy_row(i * 3 + 1, TU.emb_s0 + (size_t)lu * dim);
+                                if (KIND == TRS_OPT_SPARSE_ADAM) copy_row(i * 3 + 2, TU.emb_s1 + (size_t)lu * dim);
+                            }
+                            if (!have_p) copy_region(ord * 2 + 0, TP.emb + (size_t)lp * dim);
+                            if (!have_n) copy_region(ord * 2 + 1, TN.emb + (size_t)ln * dim);
+                            if (gl < 3) {
+                                const float* lin = gl == 0 ? TU.lin : (gl == 1 ? TP.lin : TN.lin);
+                                const uint32_t lrow = gl == 0 ? lu : (gl == 1 ? lp : ln);
+                                const bool have = gl == 1 ? have_p : (gl == 2 ? have_n : false);
+                                if (lin) {
+                                    if (have) bias_r[i] = reinterpret_cast<const float*>(
+                                                  my_pf_bias + (size_t)(ord * 2 + (gl - 1)) * 16)[lrow & 3u];
+                                    else bias_r[i] = __ldcg(lin + lrow);
+                                }
                             }
                         }
+                        cp_async_commit();
                     }
-                    cp_async_commit();
-                }
 #pragma unroll
-                for (int i = 0; i < SBA; ++i) {
-                    cp_async_wait(SBA - 1 - i);
-                    const uint32_t bf = __shfl_sync(0xffffffffu, cur.b[i / G], i % G, G);
-                    const uint32_t q = __shfl_sync(0xffffffffu, cur.q[i / G], i % G, G);
-                    const uint32_t lu = __shfl_sync(0xffffffffu, cur.lu[i / G], i % G, G);
-                    const bool valid = i < n_r && bf != 0xFFFFFFFFu &&
-                                       (overlap ? ((bf & SAMP_DIRTY_ANY) != 0u) == late : !late);
-                    Row<4, IT> xu, xp, xn;
-                    if (valid) {
-                        xu = slot_row(i * 3 + 0);
-                        xp = region_row((o_lo + i) * 2 + 0);
-                        xn = region_row((o_lo + i) * 2 + 1);
-                    } else {
+                    for (int i = 0; i < SBA; ++i) {
+                        cp_async_wait(SBA - 1 - i);
+                        const uint32_t bf = __shfl_sync(0xffffffffu, cur.b[i / G], i % G, G);
+                        const uint32_t q = __shfl_sync(0xffffffffu, cur.q[i / G], i % G, G);
+                        const uint32_t lu = __shfl_sync(0xffffffffu, cur.lu[i / G], i % G, G);
+                        const bool valid = i < n_r && bf != 0xFFFFFFFFu &&
+                                           (overlap ? ((bf & SAMP_DIRTY_ANY) != 0u) == late : !late);
+                        Row<4, IT> xu, xp, xn;
+                        if (valid) {
+                            xu = slot_row(i * 3 + 0);
+                            xp = region_row((o_lo + i) * 2 + 0);
+                            xn = region_row((o_lo + i) * 2 + 1);
+                        } else {
 #pragma unroll
-                        for (int a = 0; a < IT; ++a) xu.c[a] = xp.c[a] = xn.c[a] = Vec<4>::zero();
-                    }
-                    const float bu = __shfl_sync(0xffffffffu, bias_r[i], 0, G);
-                    const float bip = __shfl_sync(0xffffffffu, bias_r[i], 1, G);
-                    const float bin = __shfl_sync(0xffffffffu, bias_r[i], 2, G);
-                    float hv = 0.f;
-                    process(valid, bf, q, lu, xu, xp, xn, bu, bip, bin, i * 3, hv);
-                    if (valid) {
-                        if (rnd == 0) hreg[i] = hv; else hreg[SBA + i] = hv;
-                    }
-                }
-            } else {
-                // ---- overflow round: two samples, all five rows in the thread-private slots 5i .. 5i + 4 ----
-                float bias_r[SBO];
-#pragma unroll
-                for (int i = 0; i < SBO; ++i) {
-                    const uint32_t bf = __shfl_sync(0xffffffffu, cur.b[i / G], i % G, G);
-                    const uint32_t q = __shfl_sync(0xffffffffu, cur.q[i / G], i % G, G);
-                    const uint32_t lu = __shfl_sync(0xffffffffu, cur.lu[i / G], i % G, G);
-                    const uint32_t lp = __shfl_sync(0xffffffffu, cur.lp[i / G], i % G, G);
-                    const uint32_t ln = __shfl_sync(0xffffffffu, cur.ln[i / G], i % G, G);
-                    bias_r[i] = 0.f;
-                    if (bf != 0xFFFFFFFFu) {
-                        const trs_table& TU = C.user[q & 15u];
-                        const trs_table& TP = C.item[(q >> 4) & 15u];
-                        const trs_table& TN = C.item[(q >> 8) & 15u];
-                        copy_row(i * 5 + 0, TU.emb + (size_t)lu * dim);
-                        if (bf & SAMP_USER_SINGLE) {
-                            if (KIND != TRS_OPT_SGD) copy_row(i * 5 + 1, TU.emb_s0 + (size_t)lu * dim);
-                            if (KIND == TRS_OPT_SPARSE_ADAM) copy_row(i * 5 + 2, TU.emb_s1 + (size_t)lu * dim);
+                            for (int a = 0; a < IT; ++a) xu.c[a] = xp.c[a] = xn.c[a] = Vec<4>::zero();
                         }
-                        copy_row(i * 5 + 3, TP.emb + (size_t)lp * dim);
-                        copy_row(i * 5 + 4, TN.emb + (size_t)ln * dim);
-                        if (gl < 3) {
-                            const float* lin = gl == 0 ? TU.lin : (gl == 1 ? TP.lin : TN.lin);
-                            const uint32_t lrow = gl == 0 ? lu : (gl == 1 ? lp : ln);
-                            if (lin) bias_r[i] = __ldcg(lin + lrow);
+                        const float bu = __shfl_sync(0xffffffffu, bias_r[i], 0, G);
+                        const float bip = __shfl_sync(0xffffffffu, bias_r[i], 1, G);
+                        const float bin = __shfl_sync(0xffffffffu, bias_r[i], 2, G);
+                        float hv = 0.f;
+                        process(valid, bf, q, lu, xu, xp, xn, bu, bip, bin, i * 3, hv, no_items);
+                        if (valid) {
+                            if (rnd == 0) hreg[i] = hv; else hreg[SBA + i] = hv;
                         }
                     }
-                    cp_async_commit();
-                }
+                } else {
+                    // ---- overflow round: two samples, all five rows in the thread-private slots 5i .. 5i + 4 ----
+                    float bias_r[SBO];
 #pragma unroll
-                for (int i = 0; i < SBO; ++i) {
-                    cp_async_wait(SBO - 1 - i);
-                    const uint32_t bf = __shfl_sync(0xffffffffu, cur.b[i / G], i % G, G);
-                    const uint32_t q = __shfl_sync(0xffffffffu, cur.q[i / G], i % G, G);
-                    const uint32_t lu = __shfl_sync(0xffffffffu, cur.lu[i / G], i % G, G);
-                    const bool valid = bf != 0xFFFFFFFFu;
-                    Row<4, IT> xu, xp, xn;
-                    if (valid) {
-                        xu = slot_row(i * 5 + 0);
-                        xp = slot_row(i * 5 + 3);
-                        xn = slot_row(i * 5 + 4);
-                    } else {
-#pragma unroll
-                        for (int a = 0; a < IT; ++a) xu.c[a] = xp.c[a] = xn.c[a] = Vec<4>::zero();
+                    for (int i = 0; i < SBO; ++i) {
+                        const uint32_t bf = __shfl_sync(0xffffffffu, cur.b[i / G], i % G, G);
+                        const uint32_t q = __shfl_sync(0xffffffffu, cur.q[i / G], i % G, G);
+                        const uint32_t lu = __shfl_sync(0xffffffffu, cur.lu[i / G], i % G, G);
+                        const uint32_t lp = __shfl_sync(0xffffffffu, cur.lp[i / G], i % G, G);
+                        const uint32_t ln = __shfl_sync(0xffffffffu, cur.ln[i / G], i % G, G);
+                        bias_r[i] = 0.f;
+                        if (bf != 0xFFFFFFFFu) {
+                            const trs_table& TU = C.user[q & 15u];
+                            const trs_table& TP = C.item[(q >> 4) & 15u];
+                            const trs_table& TN = C.item[(q >> 8) & 15u];
+                            copy_row(i * 5 + 0, TU.emb + (size_t)lu * dim);
+                            if (bf & SAMP_USER_SINGLE) {
+                                if (KIND != TRS_OPT_SGD) copy_row(i * 5 + 1, TU.emb_s0 + (size_t)lu * dim);
+                                if (KIND == TRS_OPT_SPARSE_ADAM) copy_row(i * 5 + 2, TU.emb_s1 + (size_t)lu * dim);
+                            }
+                            copy_row(i * 5 + 3, TP.emb + (size_t)lp * dim);
+                            copy_row(i * 5 + 4, TN.emb + (size_t)ln * dim);
+                            if (gl < 3) {
+                                const float* lin = gl == 0 ? TU.lin : (gl == 1 ? TP.lin : TN.lin);
+                                const uint32_t lrow = gl == 0 ? lu : (gl == 1 ? lp : ln);
+                                if (lin) bias_r[i] = __ldcg(lin + lrow);
+                            }
+                        }
+                        cp_async_commit();
                     }
-                    const float bu = __shfl_sync(0xffffffffu, bias_r[i], 0, G);
-                    const float bip = __shfl_sync(0xffffffffu, bias_r[i], 1, G);
-                    const float bin = __shfl_sync(0xffffffffu, bias_r[i], 2, G);
-                    float hv = 0.f;
-                    process(valid, bf, q, lu, xu, xp, xn, bu, bip, bin, i * 5, hv);
-                    hover += hv;
+#pragma unroll
+                    for (int i = 0; i < SBO; ++i) {
+                        cp_async_wait(SBO - 1 - i);
+                        const uint32_t bf = __shfl_sync(0xffffffffu, cur.b[i / G], i % G, G);
+                        const uint32_t q = __shfl_sync(0xffffffffu, cur.q[i / G], i % G, G);
+                        const uint32_t lu = __shfl_sync(0xffffffffu, cur.lu[i / G], i % G, G);
+                        const bool valid = bf != 0xFFFFFFFFu;
+                        Row<4, IT> xu, xp, xn;
+                        if (valid) {
+                            xu = slot_row(i * 5 + 0);
+                            xp = slot_row(i * 5 + 3);
+                            xn = slot_row(i * 5 + 4);
+                        } else {
+#pragma unroll
+                            for (int a = 0; a < IT; ++a) xu.c[a] = xp.c[a] = xn.c[a] = Vec<4>::zero();
+                        }
+                        const float bu = __shfl_sync(0xffffffffu, bias_r[i], 0, G);
+                        const float bip = __shfl_sync(0xffffffffu, bias_r[i], 1, G);
+                        const float bin = __shfl_sync(0xffffffffu, bias_r[i], 2, G);
+                        float hv = 0.f;
+                        process(valid, bf, q, lu, xu, xp, xn, bu, bip, bin, i * 5, hv, no_items);
+                        hover += hv;
+                    }
                 }
             }
         }
         // the next step's first rounds of records (plan + epoch data), then my first phase-B descriptors: all in
         // flight across the barrier
         if (more) {
+            if constexpr (ONE) {
+                fetch_one(recO, lo + ep.batch, nS_next, 0);
+            } else {
 #pragma unroll
-            for (int r = 0; r < NPR; ++r)
-                fetch_records(recN[r], lo + ep.batch, nS_next, gfirst + round_lo(r) * gstride, round_n(r));
+                for (int r = 0; r < NPR; ++r)
+                    fetch_records(recN[r], lo + ep.batch, nS_next, gfirst + round_lo(r) * gstride, round_n(r));
+            }
         }
         nS_cur = nS_next;
         const int nP = nU + nI;
@@ -1087,29 +1389,43 @@ static ShardStage shard_stage_layout(int dim, int64_t B) {
     return L;
 }
 
-template <int KIND, int G, int IT>
+template <int KIND, int G, int IT, bool ONE>
 static cudaError_t launch_shard_k(const ShardCtx* ctx0, const ShardCtx* ctxs, int cpr, int n_local, const trs_epoch* ep,
                                   const OptScalars* os, int first_step, int n_steps, unsigned sync_epoch,
-                                  unsigned long long timeout_ns, cudaStream_t stream) {
-    const void* fn = (const void*)shard_train_kernel<KIND, G, IT>;
-    const size_t smem = shard_smem_total<G, IT>();
+                                  unsigned long long timeout_ns, const uint8_t* iflag, cudaStream_t stream) {
+    const void* fn = (const void*)shard_train_kernel<KIND, G, IT, ONE>;
+    const size_t smem = shard_smem_total<G, IT, ONE>();
     cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     void* args[] = {(void*)ctx0, (void*)&ctxs, (void*)&cpr, (void*)ep, (void*)os, (void*)&first_step,
-                    (void*)&n_steps, (void*)&sync_epoch, (void*)&timeout_ns};
+                    (void*)&n_steps, (void*)&sync_epoch, (void*)&timeout_ns, (void*)&iflag};
     return cudaLaunchCooperativeKernel(fn, dim3(cpr * n_local), dim3(shard_threads<IT>()), args, smem, stream);
 }
+template <int KIND, int G, int IT>
+static cudaError_t launch_shard_o(bool one, const ShardCtx* ctx0, const ShardCtx* ctxs, int cpr, int n_local,
+                                  const trs_epoch* ep, const OptScalars* os, int first_step, int n_steps,
+                                  unsigned sync_epoch, unsigned long long timeout_ns, const uint8_t* iflag,
+                                  cudaStream_t stream) {
+    if constexpr (IT == 1) {
+        if (one)
+            return launch_shard_k<KIND, G, IT, true>(ctx0, ctxs, cpr, n_local, ep, os, first_step, n_steps, sync_epoch,
+                                                     timeout_ns, iflag, stream);
+    }
+    return launch_shard_k<KIND, G, IT, false>(ctx0, ctxs, cpr, n_local, ep, os, first_step, n_steps, sync_epoch,
+                                              timeout_ns, iflag, stream);
+}
 template <int G, int IT>
-static cudaError_t launch_shard(const ShardCtx* ctx0, const ShardCtx* ctxs, int cpr, int n_local, const trs_epoch* ep,
-                                const OptScalars* os, int first_step, int n_steps, unsigned sync_epoch,
-                                unsigned long long timeout_ns, cudaStream_t stream) {
+static cudaError_t launch_shard(bool one, const ShardCtx* ctx0, const ShardCtx* ctxs, int cpr, int n_local,
+                                const trs_epoch* ep, const OptScalars* os, int first_step, int n_steps,
+                                unsigned sync_epoch, unsigned long long timeout_ns, const uint8_t* iflag,
+                                cudaStream_t stream) {
     switch (os->kind) {
         case TRS_OPT_SGD:
-            return launch_shard_k<TRS_OPT_SGD, G, IT>(ctx0, ctxs, cpr, n_local, ep, os, first_step, n_steps, sync_epoch, timeout_ns, stream);
+            return launch_shard_o<TRS_OPT_SGD, G, IT>(one, ctx0, ctxs, cpr, n_local, ep, os, first_step, n_steps, sync_epoch, timeout_ns, iflag, stream);
         case TRS_OPT_ADAGRAD:
-            return launch_shard_k<TRS_OPT_ADAGRAD, G, IT>(ctx0, ctxs, cpr, n_local, ep, os, first_step, n_steps, sync_epoch, timeout_ns, stream);
+            return launch_shard_o<TRS_OPT_ADAGRAD, G, IT>(one, ctx0, ctxs, cpr, n_local, ep, os, first_step, n_steps, sync_epoch, timeout_ns, iflag, stream);
         default:
-            return launch_shard_k<TRS_OPT_SPARSE_ADAM, G, IT>(ctx0, ctxs, cpr, n_local, ep, os, first_step, n_steps, sync_epoch, timeout_ns, stream);
+            return launch_shard_o<TRS_OPT_SPARSE_ADAM, G, IT>(one, ctx0, ctxs, cpr, n_local, ep, os, first_step, n_steps, sync_epoch, timeout_ns, iflag, stream);
     }
 }
 
@@ -1120,6 +1436,8 @@ static int g_shard_prefer_it = 1;
 static unsigned long long* g_shard_trace = nullptr;
 static int g_shard_overlap = -1;
 static int g_shard_remote_hint = 1;
+static int g_shard_one_pass = 1;
+static int g_shard_last_one_pass = -1;
 
 static bool pick_shard_shape(int dim, int* G, int* IT) {
     if (dim <= 0 || dim % 4 || dim > 512) return false;
@@ -1234,6 +1552,17 @@ extern "C" int trs_shard_plan_build(const trs_shard* sh, const trs_epoch* ep, vo
         user_compact_kernel<<<(unsigned)steps, 1024, 0, st>>>((uint32_t*)(P + L.ukey), (uint32_t*)(P + L.uval), own_cnt,
                                                              ep->batch);
     }
+    if (W == 1) {  // after user_compact_kernel: cntB copies the final user counts
+        const int tiles = (int)((2ll * ep->batch + RT_TILE - 1) / RT_TILE);
+        const dim3 grid((unsigned)tiles, (unsigned)steps);
+        const uint32_t* ikey = (const uint32_t*)(P + L.ikey);
+        const uint32_t* ival = (const uint32_t*)(P + L.ival);
+        item_single_count_kernel<<<grid, RT_THREADS, 0, st>>>(ikey, ival, own_cnt, ep->batch, (uint8_t*)(P + L.iflag),
+                                                              tile_cnt, tiles);
+        item_single_scatter_kernel<<<grid, RT_THREADS, 0, st>>>(ikey, ival, own_cnt, ep->batch, tile_cnt, tiles,
+                                                                (uint32_t*)(P + L.ikeyB), (uint32_t*)(P + L.ivalB),
+                                                                (uint32_t*)(P + L.cntB));
+    }
     TRS_CUDA(cudaGetLastError());
     return TRS_OK;
 }
@@ -1270,6 +1599,11 @@ extern "C" int trs_shard_train_steps(const trs_shard* shards, int n_local, const
     const int cpr = shard_cpr(n_local);
     TRS_REQUIRE(cpr >= 1, "more local ranks than SMs");
     const ShardPlanLayout PL = shard_plan_layout(ep->n_samples, ep->batch);
+    int sg = 0, sit = 0;
+    const bool shape_ok = pick_shard_shape(shards[0].dim, &sg, &sit);
+    // one rank in one launch: every item row's owner is the rank that reads it, so phase A updates the single ones
+    const bool one = shape_ok && g_shard_one_pass && n_local == 1 && shards[0].world == 1 && sit == 1;
+    const uint8_t* iflag = one ? (const uint8_t*)plans_host[0] + PL.iflag : nullptr;
     cudaStream_t st = (cudaStream_t)stream;
     ShardCtx ctx[TRS_MAX_RANKS];
     const size_t ctx_bytes = ((size_t)n_local * sizeof(ShardCtx) + 255) / 256 * 256;
@@ -1311,8 +1645,9 @@ extern "C" int trs_shard_train_steps(const trs_shard* shards, int n_local, const
         c.samp = (const uint32_t*)(P + PL.samp);
         c.ukey = (const uint32_t*)(P + PL.ukey);
         c.uval = (const uint32_t*)(P + PL.uval);
-        c.ikey = (const uint32_t*)(P + PL.ikey);
-        c.ival = (const uint32_t*)(P + PL.ival);
+        c.ikey = (const uint32_t*)(P + (one ? PL.ikeyB : PL.ikey));
+        c.ival = (const uint32_t*)(P + (one ? PL.ivalB : PL.ival));
+        if (one) c.own_cnt = (const uint32_t*)(P + PL.cntB);
         c.loss_part = loss_part + (size_t)i * steps * cpr;
         c.loss_out = loss_sum_host[i];
         c.status = status;
@@ -1326,12 +1661,11 @@ extern "C" int trs_shard_train_steps(const trs_shard* shards, int n_local, const
     const OptScalars os = make_opt_scalars(optim);
     const unsigned long long timeout_ns = (unsigned long long)(timeout_ms > 0 ? timeout_ms : 20000) * 1000000ull;
     cudaError_t err = cudaErrorInvalidValue;
-    int sg = 0, sit = 0;
-    TRS_REQUIRE(pick_shard_shape(shards[0].dim, &sg, &sit), "unsupported n_factors %d", shards[0].dim);
+    TRS_REQUIRE(shape_ok, "unsupported n_factors %d", shards[0].dim);
 #define TRS_SHARD_CASE(G_, IT_)                                                                                     \
     case G_ * 100 + IT_:                                                                                            \
-        err = launch_shard<G_, IT_>(&ctx[0], ctxs_dev, cpr, n_local, ep, &os, first_step, n_steps, (unsigned)sync_epoch, \
-                                    timeout_ns, st);                                                                \
+        err = launch_shard<G_, IT_>(one, &ctx[0], ctxs_dev, cpr, n_local, ep, &os, first_step, n_steps,              \
+                                    (unsigned)sync_epoch, timeout_ns, iflag, st);                                   \
         break;
     switch (sg * 100 + sit) {
         TRS_SHARD_CASE(4, 1)
@@ -1347,6 +1681,7 @@ extern "C" int trs_shard_train_steps(const trs_shard* shards, int n_local, const
     }
 #undef TRS_SHARD_CASE
     TRS_CUDA(err);
+    g_shard_last_one_pass = one ? 1 : 0;
     return TRS_OK;
 }
 
@@ -1361,6 +1696,11 @@ extern "C" void trs_debug_shard_trace(void* buf) { g_shard_trace = (unsigned lon
 extern "C" void trs_debug_shard_overlap(int mode) { g_shard_overlap = mode < 0 ? -1 : (mode ? 1 : 0); }
 // tuning hook: the evict_last policy on gradient rows stored into PEER memory (1, default) or only on local ones (0)
 extern "C" void trs_debug_shard_remote_hint(int on) { g_shard_remote_hint = on ? 1 : 0; }
+// tuning hook (results do not depend on it): 1 (default) lets a one-rank launch with one chunk per lane run the one-pass
+// kernel, whose phase A also updates the item rows a step looks up once; 0 forces the two-phase kernel there
+extern "C" void trs_debug_shard_one_pass(int on) { g_shard_one_pass = on ? 1 : 0; }
+// debug hook: 1 if the last trs_shard_train_steps launch ran the one-pass kernel, 0 if the two-phase one, -1 before any
+extern "C" int trs_debug_shard_last_one_pass(void) { return g_shard_last_one_pass; }
 
 
 // ---- CUDA IPC plumbing ---------------------------------------------------------------------------------------

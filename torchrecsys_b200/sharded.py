@@ -242,8 +242,10 @@ class ShardedLinearTrainer:
     def plan_launches(self) -> int:
         """CUDA kernels one trs_shard_plan_build launches for one rank (bench.py's gpu_launches)."""
         passes = lambda rows: max(1, -(-max(1, (max(rows, 2) - 1).bit_length()) // 8))
-        # per id space: count + scatter + 2 per radix pass; then the item filter, the three flag kernels, the compaction
-        return 2 * (2 + passes(-(-self.n_users // self.world)) + passes(-(-self.n_items // self.world))) + 5
+        # per id space: count + scatter + 2 per radix pass; then the item filter, the three flag kernels, the compaction;
+        # one rank: the single item rows' flags and phase B's item pairs (count + scatter)
+        return 2 * (2 + passes(-(-self.n_users // self.world)) + passes(-(-self.n_items // self.world))) + 5 + \
+            2 * (self.world == 1)
 
     def check_status(self) -> None:
         if int(self.status.item()) != 0:
