@@ -365,6 +365,19 @@ int trs_shard_train_steps(const trs_shard* shards, int n_local, const trs_epoch*
                           int n_steps, uint64_t sync_epoch, float* const* loss_sum_host, int32_t* status,
                           int timeout_ms, trs_stream_t stream);
 
+/* Serving on the shards where they live: every row is read from its owner through the pointers of `shard` (peer
+ * mappings), nothing is gathered.  Ids must lie in [0, n_users) / [0, n_items).  The caller orders these reads
+ * against the owners' next training launch (sharded.py ends each serving call with a group collective). */
+/* a10 (model.py:292-338) for batches [first_batch, first_batch + n_batches) of the global epoch: loss[b - first_batch]
+ * and auc[b - first_batch] as trs_eval_pairwise computes them on the gathered model, bit for bit; pos_out / neg_out
+ * (nullable) receive the raw scores from the range's first sample on. */
+int trs_shard_eval_pairwise(const trs_shard* shard, const trs_epoch* epoch, int64_t first_batch, int64_t n_batches,
+                            float* loss, float* auc, float* pos_out, float* neg_out, trs_stream_t stream);
+/* emb_out[j, :] = row ids[j] of the user (table 0) or item (table 1) table, lin_out[j] (nullable) = its bias, both
+ * copied bit for bit from the owner. */
+int trs_shard_gather_rows(const trs_shard* shard, int table, const int64_t* ids, int64_t n, float* emb_out,
+                          float* lin_out, trs_stream_t stream);
+
 /* CUDA IPC plumbing for the peer mapping (the only entry points that touch address spaces; they never allocate
  * device memory).  export: 64-byte handle of the allocation that contains `ptr` + the offset of ptr inside it;
  * open: maps that allocation into this process (peer access enabled lazily) and returns its base; close unmaps. */

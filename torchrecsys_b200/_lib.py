@@ -28,7 +28,8 @@ SYMBOLS = [
     "trs_topk_merge", "trs_shard_stage_bytes", "trs_shard_plan_bytes", "trs_shard_plan_tmp_bytes",
     "trs_shard_plan_build", "trs_shard_workspace_bytes", "trs_shard_train_steps", "trs_ipc_export",
     "trs_ipc_open", "trs_ipc_close", "trs_scores_backward", "trs_sort_workspace_bytes", "trs_sorted_auc",
-    "trs_epoch_shuffle", "trs_gather_rows_i64", "trs_predict_topk_reuse",
+    "trs_epoch_shuffle", "trs_gather_rows_i64", "trs_predict_topk_reuse", "trs_shard_eval_pairwise",
+    "trs_shard_gather_rows",
 ]
 
 
@@ -432,6 +433,26 @@ def shard_train_steps(shards: Sequence[Shard], epoch: Epoch, optim: Optim, plans
                                    C.c_size_t(workspace.numel()), first_step, n_steps, C.c_uint64(sync_epoch), loss_ptrs,
                                    C.c_void_p(_ptr(status, torch.int32)), timeout_ms, _stream()))
     return workspace
+
+
+def shard_eval_pairwise(shard: Shard, epoch: Epoch, first_batch: int, n_batches: int, loss, auc, pos=None,
+                        neg=None) -> None:
+    """Batches [first_batch, first_batch + n_batches) of the global epoch, every row read from its owner: loss / auc
+    [>= n_batches] and the optional scores pos / neg [>= the range's samples] are written from index 0."""
+    f32 = torch.float32
+    _check(lib().trs_shard_eval_pairwise(C.byref(shard), C.byref(epoch), C.c_int64(first_batch), C.c_int64(n_batches),
+                                         C.c_void_p(_ptr(loss, f32)), C.c_void_p(_ptr(auc, f32)),
+                                         C.c_void_p(_ptr(pos, f32)), C.c_void_p(_ptr(neg, f32)), _stream()))
+
+
+def shard_gather_rows(shard: Shard, table: int, ids, device):
+    """(rows [n, dim], biases [n, 1]) of global ids of the user (0) or item (1) table, copied from their owners."""
+    n = ids.shape[0]
+    emb = torch.empty((n, shard.dim), dtype=torch.float32, device=device)
+    lin = torch.empty((n, 1), dtype=torch.float32, device=device)
+    _check(lib().trs_shard_gather_rows(C.byref(shard), table, C.c_void_p(_ptr(ids, torch.int64)), C.c_int64(n),
+                                       C.c_void_p(emb.data_ptr()), C.c_void_p(lin.data_ptr()), _stream()))
+    return emb, lin
 
 
 def ipc_export(t: torch.Tensor):

@@ -215,6 +215,8 @@ inline bool pick_row_shape(int dim, RowShape* s) {
     } while (0)
 
 int check_model(const trs_model* m, RowShape* shape);
+// rank / world / dim / row counts of a row-sharded group (csrc/shard.cu)
+int check_shard(const trs_shard* sh, RowShape* shape);
 
 static inline int64_t n_steps_of(const trs_epoch* e) {
     return (e->n_samples + e->batch - 1) / e->batch;

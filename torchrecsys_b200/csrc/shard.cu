@@ -1452,7 +1452,7 @@ static bool pick_shard_shape(int dim, int* G, int* IT) {
     return it <= 4;
 }
 
-static int check_shard(const trs_shard* sh, RowShape* shape) {
+int check_shard(const trs_shard* sh, RowShape* shape) {
     TRS_REQUIRE(sh != nullptr, "shard is NULL");
     TRS_REQUIRE(sh->world >= 1 && sh->world <= TRS_MAX_RANKS, "world %d outside 1..%d", sh->world, TRS_MAX_RANKS);
     TRS_REQUIRE(sh->rank >= 0 && sh->rank < sh->world, "rank %d outside the group of %d", sh->rank, sh->world);

@@ -13,6 +13,8 @@ Row-sharded training (BASELINE configs[3], Linear 50M x 5M, dim 128)  -- ``Shard
     owner's staging buffer, and every owner coalesces + updates its own rows -- two flag barriers per step.
     ``state_dict()`` / ``load_state_dict()`` gather / scatter the shards (parameters AND optimizer state) in the
     reference's single-process layout and key names, so checkpoints interchange with ``TorchRecSys``.
+    ``evaluate`` / ``eval_pairwise`` / ``predict_topk`` / ``lookup`` serve the model where it lives: their kernels
+    (csrc/shard_serve.cu) read every row from its owner through the same peer mappings, nothing is gathered.
     One GPU can host the whole group (``emulate_world=G``): the parity tests run that way on a 1-GPU box.
 
 Item-sharded predict (BASELINE configs[4])
@@ -133,6 +135,9 @@ class ShardedLinearTrainer:
         self._h2d = None          # train_epoch_host: two device id buffers + the copy stream
         self.status = torch.zeros(1, dtype=torch.int32, device=self.device)
         self.launches = 0
+        self._state_version = 0   # bumped by load_state_dict: with sync_epoch, says whether the tables changed
+        self._topk_caches: Dict[int, object] = {}   # per local rank: predict's prepared bf16 item-shard operand
+        self.last_predict_overflow = 0   # users predict_topk ranked exactly on this process's shards (last call)
 
     # ---- peer mapping -----------------------------------------------------------------------------
     def _map_peers(self) -> None:
@@ -399,10 +404,150 @@ class ShardedLinearTrainer:
                         self.state[r][name][i][1].copy_(optimizer_state[bkey][sname][r::G].to(self.device).view(-1, 1))
         if optimizer_state is not None:
             self.binding.step0 = int(optimizer_state["user.weight"].get("step", 0))
+        self._state_version += 1
         if len(self.local_ranks) < G:
             if self.device.type == "cuda":
                 torch.cuda.synchronize(self.device)
             dist.barrier(group=self.group)  # peers read these rows: nobody trains before everyone has loaded
+
+    # ---- serving on the shards: lookup / eval_pairwise / evaluate / predict_topk, nothing gathered ------------------
+    # Ordering rule.  In a real group a rank must not train while another rank still reads its rows.
+    #  * Reads after training are safe: every training launch ends waiting for every rank's last arrival (csrc/shard.cu,
+    #    the cross_wait after the step loop), and load_state_dict ends with a barrier.
+    #  * Reads before the next training: each method below that launches a peer-reading kernel ends with a group
+    #    collective on this rank's stream before it returns -- eval_pairwise the all-gather, predict_topk the
+    #    all_to_all, lookup a one-element all-reduce.  This rank's next training kernel is queued behind that
+    #    collective, and the collective cannot complete before every rank's reads have finished: no host
+    #    synchronisation is needed.
+    # In a real group these methods are collective: every rank calls them with the same arguments.
+    TOPK_MAX_FACTORS = 239   # predict_batch's kernel path (csrc/topk.cu: check_topk); k in 1..128 likewise
+
+    def _require_cuda(self) -> None:
+        if self.bases is None:
+            raise RuntimeError("torchrecsys_b200 has no CPU fallback: the row-sharded tables need CUDA devices")
+
+    def _device_ids(self, ids, n: int, what: str) -> torch.Tensor:
+        """int64 ids on this device; IndexError outside [0, n), as TorchRecSys raises."""
+        ids = torch.as_tensor(ids, dtype=torch.int64).reshape(-1)
+        if ids.numel() and (int(ids.min()) < 0 or int(ids.max()) >= n):
+            raise IndexError(f"{what} ids must lie in [0, {n})")
+        return ids.to(self.device).contiguous()
+
+    def lookup(self, name: str, ids) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Rows of global ``ids`` of the ``"user"`` or ``"item"`` table and their biases, (emb [n, D], bias [n, 1]),
+        copied from their owners bit for bit."""
+        self._require_cuda()
+        if name not in ("user", "item"):
+            raise ValueError(f"table must be 'user' or 'item', got {name!r}")
+        ids = self._device_ids(ids, self.n_users if name == "user" else self.n_items, name)
+        out = self._lib.shard_gather_rows(self._shard_struct(self.local_ranks[0]), int(name == "item"), ids, self.device)
+        if len(self.local_ranks) < self.world:
+            dist.all_reduce(torch.zeros(1, device=self.device), group=self.group)   # the ordering rule above
+        return out
+
+    def eval_pairwise(self, user: torch.Tensor, pos: torch.Tensor, neg: torch.Tensor, batch_size: int = 512,
+                      want_scores: bool = False):
+        """``_lib.eval_pairwise`` on the shards -> (loss [nb], auc [nb], pos scores, neg scores; None unless
+        ``want_scores``), bit-identical to it on the gathered model.  user / pos / neg: the GLOBAL test epoch (int64
+        device tensors, identical on every rank).  Rank q evaluates the whole batches [q P, (q + 1) P), P = ceil(nb / W):
+        a batch is never divided between ranks, so its mean hinge keeps its association."""
+        self._require_cuda()
+        _lib, W, B = self._lib, self.world, int(batch_size)
+        n = user.shape[0]
+        nb = -(-n // B)
+        P = -(-nb // W)
+        L = len(self.local_ranks)
+        # [rank, (loss, auc), batch] and [rank, (pos, neg), sample], each rank's block at its batch range
+        stats = torch.empty((L, 2, P), dtype=torch.float32, device=self.device)
+        scores = torch.empty((L, 2, P * B), dtype=torch.float32, device=self.device) if want_scores else None
+        if nb:
+            epoch = _lib.make_epoch(user, pos, neg, None, None, B)
+            for i, r in enumerate(self.local_ranks):
+                lo = min(r * P, nb)
+                _lib.shard_eval_pairwise(self._shard_struct(r), epoch, lo, min(nb, lo + P) - lo, stats[i, 0], stats[i, 1],
+                                         *((scores[i, 0], scores[i, 1]) if want_scores else ()))
+            if L < W:   # every rank takes part, also one whose range is empty (the ordering rule above)
+                parts = [stats] + ([scores] if want_scores else [])
+                full = [torch.empty((W,) + tuple(t.shape[1:]), dtype=t.dtype, device=t.device) for t in parts]
+                for f, t in zip(full, parts):
+                    dist.all_gather_into_tensor(f, t, group=self.group)
+                stats, scores = full[0], (full[1] if want_scores else None)
+        # fresh tensors, as _lib.eval_pairwise returns: a torch reduction's association follows its input's alignment
+        loss, auc = (stats[:, j].reshape(-1)[:nb].clone() for j in (0, 1))
+        if not want_scores:
+            return loss, auc, None, None
+        return loss, auc, scores[:, 0].reshape(-1)[:n].clone(), scores[:, 1].reshape(-1)[:n].clone()
+
+    def evaluate(self, user: torch.Tensor, pos: torch.Tensor, neg: torch.Tensor, batch_size: int = 512,
+                 eval_metrics=("loss", "auc")) -> Dict[str, float]:
+        """``TorchRecSys.evaluate``'s metrics on the shards, returned rather than printed: ``loss`` / ``auc`` the mean
+        over batches of ``eval_pairwise``, ``roc_auc`` the sort-based ROC-AUC of the whole split, 0 for an unknown name.
+        ``neg`` is the caller's negatives (e.g. those ``TorchRecSys._with_negatives`` draws)."""
+        from .model import TorchRecSys
+        loss, auc, ps, ns = self.eval_pairwise(user, pos, neg, batch_size, want_scores="roc_auc" in eval_metrics)
+        results, out = {"loss": loss, "auc": auc}, {}
+        for metric in eval_metrics:
+            if metric in results:
+                out[metric] = float(results[metric].mean().item())
+            elif metric == "roc_auc":
+                out[metric] = TorchRecSys._roc_auc(ps, ns)
+            else:
+                out[metric] = 0
+        return out
+
+    def predict_topk(self, users, k: int) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Top-k items of each user against the whole catalogue -> (idx int64 [Q, min(k, n_items)], score fp32), on the
+        device and the same on every rank; equal to ``_lib.predict_topk`` / ``TorchRecSys.predict_batch`` on the gathered
+        model (best first, ties towards the lower item id).  Each rank ranks its own item shard against the query users'
+        rows; the per-shard lists are merged."""
+        self._require_cuda()
+        if not 1 <= int(k) <= 128:
+            raise ValueError(f"top_k must be in 1..128 on the row-sharded tables (got {k})")
+        if self.dim > self.TOPK_MAX_FACTORS:
+            raise ValueError(f"predict_topk on the row-sharded tables needs n_factors <= {self.TOPK_MAX_FACTORS}")
+        _lib, W, k = self._lib, self.world, int(k)
+        users = self._device_ids(users, self.n_users, "user")
+        Q, kk = users.numel(), min(k, self.n_items)
+        self.last_predict_overflow = 0
+        if Q == 0:
+            return (torch.empty((0, kk), dtype=torch.int64, device=self.device),
+                    torch.empty((0, kk), dtype=torch.float32, device=self.device))
+        u_emb, u_lin = _lib.shard_gather_rows(self._shard_struct(self.local_ranks[0]), 0, users, self.device)
+        queries = torch.arange(Q, device=self.device)
+        key = (self.sync_epoch, self._state_version)   # unchanged tables: the prepared item operand is reused
+
+        def local_topk(r: int):
+            """(global idx, score) [Q, k] of rank r's item shard, -1 / -inf padded."""
+            emb, lin = self.tables[r]["item"]
+            rows = emb.shape[0]
+            if rows == 0:
+                return (torch.full((Q, k), -1, dtype=torch.int64, device=self.device),
+                        torch.full((Q, k), float("-inf"), device=self.device))
+            model = _lib.make_model(_lib.NET_LINEAR, self.dim, _lib.make_table(u_emb, lin=u_lin),
+                                    _lib.make_table(emb, lin=lin), [])
+            idx, score, over = _lib.predict_topk(model, queries, k, cache=self._topk_caches.setdefault(r, _lib.TopkCache()),
+                                                 cache_key=key)
+            for q in torch.nonzero(over).flatten().tolist():   # candidate set did not fit: score the shard and sort
+                s = _lib.scores(model, torch.full((rows,), q, dtype=torch.int64, device=self.device),
+                                torch.arange(rows, device=self.device))
+                s, order = torch.sort(s, descending=True, stable=True)
+                m = min(k, rows)
+                idx[q, :m], score[q, :m] = order[:m], s[:m]
+                idx[q, m:], score[q, m:] = -1, float("-inf")
+                self.last_predict_overflow += 1
+            # local order is global order within a shard: (score desc, local id asc) merges as (score desc, global id asc)
+            return torch.where(idx >= 0, idx * W + r, idx), score
+
+        if len(self.local_ranks) == W:
+            lists = [local_topk(r) for r in self.local_ranks]
+            if W == 1:
+                idx, score = lists[0]
+            else:
+                idx, score = _lib.topk_merge(torch.stack([s for _, s in lists]), torch.stack([i for i, _ in lists]), k)
+        else:   # the item-sharded predict's all_to_all merger (the ordering rule above); no block offset here
+            idx, score = sharded_predict_topk(lambda u, kq, offset: local_topk(self.rank), users, k, self.n_items,
+                                              self.group)
+        return idx[:, :kk].contiguous(), score[:, :kk].contiguous()
 
     # ---- the bridge to TorchRecSys(net_type='linear'): shard a model + its torch optimizer, and hand them back ------
     @classmethod
