@@ -377,6 +377,24 @@ int trs_shard_eval_pairwise(const trs_shard* shard, const trs_epoch* epoch, int6
  * copied bit for bit from the owner. */
 int trs_shard_gather_rows(const trs_shard* shard, int table, const int64_t* ids, int64_t n, float* emb_out,
                           float* lin_out, trs_stream_t stream);
+/* Exact top-k of rank shard->rank's OWN item shard for n_query dense query rows user_emb [n_query, dim] / user_lin
+ * [n_query] (nullable; e.g. from trs_shard_gather_rows): out_idx[q, 0..k) = GLOBAL item ids (local * world + rank) of
+ * the k best scores, out_score[q, :] those fp32 scores, equal bit for bit to trs_scores on the gathered model, ordered
+ * by (score desc, id asc) with equal values as ties (torch.sort(stable=True, descending=True)); slots with no item are
+ * -1 / -inf.  1 <= k <= 1024.  excl_ptr [n_query + 1] / excl_ids (both nullable): per query position, the sorted LOCAL
+ * item ids of this shard to leave out.  Reads only the rank's own shard.  workspace: the _workspace_bytes size (0 =
+ * bad arguments, see trs_last_error). */
+size_t trs_shard_topk_exact_workspace_bytes(const trs_shard* shard, int64_t n_query, int k);
+int trs_shard_topk_exact(const trs_shard* shard, const float* user_emb, const float* user_lin, int64_t n_query, int k,
+                         const int64_t* excl_ptr, const int64_t* excl_ids, int64_t* out_idx, float* out_score,
+                         void* workspace, size_t workspace_bytes, trs_stream_t stream);
+/* Merge n_lists sorted lists (score / idx [n_lists, n_query, k_in], each row ordered by (score desc, id asc), idx < 0 =
+ * padding at the end) into out [n_query, k_out] in the same order, -1 / -inf padded.  excl_ptr [n_query + 1] /
+ * excl_ids (both nullable): per query, sorted ids (in the lists' id space) to drop.  O(n_lists^2 k_in log k_in) per
+ * query; n_lists * (k_in + 1) <= 40960. */
+int trs_shard_topk_merge_sorted(const float* score, const int64_t* idx, int n_lists, int64_t n_query, int k_in,
+                                int k_out, const int64_t* excl_ptr, const int64_t* excl_ids, int64_t* out_idx,
+                                float* out_score, trs_stream_t stream);
 
 /* CUDA IPC plumbing for the peer mapping (the only entry points that touch address spaces; they never allocate
  * device memory).  export: 64-byte handle of the allocation that contains `ptr` + the offset of ptr inside it;

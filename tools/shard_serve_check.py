@@ -1,5 +1,5 @@
 """torchrun worker: evaluation, prediction and row lookups on the row-sharded tables over REAL peers (CUDA-IPC mapped
-shards read over NVLink; torchrecsys_b200/sharded.py + csrc/shard_serve.cu), each against the single-GPU kernels on
+shards read over NVLink; torchrecsys_b200/sharded.py + csrc/shard_serve.cu, recommend with exclusions), each against the single-GPU kernels on
 the gathered model, bit for bit.  Training runs between the serving calls, so the ordering of peer reads against the
 owners' next updates is exercised too.  Prints SHARD SERVE CHECK OK on rank 0."""
 import os
@@ -62,6 +62,20 @@ def main():
             idx, score = tr.predict_topk(users, k)
             w_idx, w_score = want_topk(model, users, k)
             assert torch.equal(idx, w_idx) and torch.equal(score, w_score), (rnd, k)
+        ex_user = rng.integers(0, U, 20000)               # ~7 excluded items per user, duplicates included
+        ex_item = rng.integers(0, I, ex_user.size)
+        codes = torch.from_numpy(np.unique(ex_user * I + ex_item)).to(dev)
+        items = torch.arange(I, device=dev)
+        for k in (10, 100, 1000):                          # tensor-core path, then the exact kernel
+            for exact in (False, True):
+                idx, score = tr.recommend(users, k, exclude=(ex_user, ex_item), _force_exact=exact)
+                for q, u in enumerate(users[:64].tolist()):
+                    s, o = torch.sort(_lib.scores(model, torch.full_like(items, u), items), descending=True, stable=True)
+                    keep_ = ~torch.isin(u * I + o, codes)
+                    o, s = o[keep_][:k], s[keep_][:k]
+                    m = o.numel()
+                    assert torch.equal(idx[q, :m], o) and torch.equal(score[q, :m], s), (rnd, k, exact, u)
+                    assert bool((idx[q, m:] == -1).all()), (rnd, k, exact, u)
         ids = torch.from_numpy(rng.integers(0, U, 1000)).to(dev)
         emb, bias = tr.lookup("user", ids)
         assert torch.equal(emb, keep["user.weight"][ids]) and torch.equal(bias, keep["user_bias.weight"][ids])

@@ -9,10 +9,19 @@ allocated), with CUDA events; prints one JSON line per measurement (rank 0).
   * predict_topk of 18944 users at top-100, users/s, first call (prepares the bf16 item operand) and a cached call;
   * for comparison, what to_model + predict_batch cost: the gather of the tables (state_dict, the part of to_model that
     moves data) followed by trs_predict_topk on the gathered model, with the peak device memory above the trainer's.
-The tables are read from HBM (several GB; far beyond the 126 MB L2)."""
+The tables are read from HBM (several GB; far beyond the 126 MB L2).
+
+    python tools/shard_serve_time.py --recommend           # recommend cases only (one GPU)
+
+  * recommend of 18944 users at D = 128: k = 100 with about 20 excluded items per user (tensor-core path) and k = 1000
+    (exact kernel), with the exact path's share of its FP32-FMA bound; at D = 256 (SGD state, so that it fits) k = 100
+    (exact kernel); what a user does today for k = 1000 -- gather the tables, then TorchRecSys._predict_exact's trs_scores
+    over every item + a stable sort per user -- for a sample of users, per user.
+  The card's name, power limit and clocks are read with nvidia-smi in the same run."""
 import argparse
 import json
 import os
+import subprocess
 import sys
 
 import torch
@@ -38,6 +47,81 @@ def timed(fn, reps):
     return sorted(out)[len(out) // 2], out
 
 
+# FP32 FMA on CUDA cores: 148 SMs x 128 lanes x 2 FLOP x 1.965 GHz (max SM clock); derived, the card may clock lower
+FMA_BOUND_FLOPS = 148 * 128 * 2 * 1.965e9
+
+
+def card():
+    """name, power limit and clocks as nvidia-smi reports them now."""
+    q = "name,power.limit,clocks.max.sm,clocks.sm"
+    try:
+        line = subprocess.run(["nvidia-smi", f"--query-gpu={q}", "--format=csv,noheader", "-i",
+                               str(torch.cuda.current_device())], capture_output=True, text=True, timeout=60).stdout
+    except (OSError, subprocess.SubprocessError) as e:
+        return {"nvidia_smi": f"unavailable: {e}"}
+    return dict(zip(q.split(","), (v.strip() for v in line.strip().split(","))))
+
+
+def recommend_cases(a, dev):
+    out = []
+    g = torch.Generator(device=dev).manual_seed(11)
+    head = {"gpu": torch.cuda.get_device_properties(dev).name, "world": 1, "users": a.users, "items": a.items}
+    for D, opt in ((128, "sparse_adam"), (256, "sgd")):
+        tr = ShardedLinearTrainer(a.users, a.items, D, global_batch=16384, optimizer=opt, lr=1e-3, device=dev,
+                                  emulate_world=1)
+        for name in ("user", "item"):
+            tr.tables[0][name][1].normal_(0, .1)
+        # distinct users: a user drawn twice would have 40 excluded items and push k + 40 past the tensor-core limit
+        q = torch.randperm(a.users, device=dev, generator=g)[:a.queries]
+        ex_user = q.repeat_interleave(20)
+        ex_item = torch.randint(0, a.items, (ex_user.numel(),), device=dev, generator=g)
+        h = dict(head, dim=D, optimizer=opt, queries=a.queries)
+        cases = [(100, (ex_user, ex_item), "exclude ~20 per user")] if D == 128 else []
+        cases += [(1000, None, "no exclusion")] if D == 128 else [(100, None, "no exclusion")]
+        for k, ex, label in cases:
+            ms, runs = timed(lambda: tr.recommend(q, k, exclude=ex), a.reps)
+            row = dict(h, what=f"recommend k={k}, {label}", k=k, ms=ms, runs_ms=runs, users_per_s=a.queries / ms * 1e3)
+            row.update(path=tr.last_recommend_paths[0])   # the path recommend took
+            if row["path"] == "exact":   # 2 D FLOP per (user, item)
+                flop = 2.0 * D * a.items * a.queries
+                row.update(tflops=flop / ms / 1e9, fma_bound_ms=flop / FMA_BOUND_FLOPS * 1e3,
+                           share_of_fma_bound=flop / FMA_BOUND_FLOPS * 1e3 / ms)
+            out.append(row)
+        if D == 128:   # today's k = 1000: gather the tables, then trs_scores over every item + stable sort per user
+            torch.cuda.synchronize()
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            sd = tr.state_dict()
+            model = _lib.make_model(_lib.NET_LINEAR, D, _lib.make_table(sd["user.weight"], lin=sd["user_bias.weight"]),
+                                    _lib.make_table(sd["item.weight"], lin=sd["item_bias.weight"]), [])
+            e1.record()
+            torch.cuda.synchronize()
+            gather_ms = e0.elapsed_time(e1)
+            items = torch.arange(a.items, device=dev)
+
+            def exact_one(u):
+                s = _lib.scores(model, torch.full_like(items, u), items)
+                return torch.sort(s, descending=True, stable=True)[1][:1000].cpu()
+
+            sample = q[:a.sample_users].tolist()
+            exact_one(sample[0])
+            torch.cuda.synchronize()
+            e0.record()
+            for u in sample:
+                exact_one(u)
+            e1.record()
+            torch.cuda.synchronize()
+            per = e0.elapsed_time(e1) / len(sample)
+            out.append(dict(h, what="gather + _predict_exact per user, k=1000", k=1000, gather_ms=gather_ms,
+                            sampled_users=len(sample), ms_per_user=per,
+                            ms_for_all_queries_estimated=per * a.queries + gather_ms))
+            del sd, model
+        tr.close()
+        del tr
+        torch.cuda.empty_cache()
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--users", type=int, default=50_000_000)
@@ -47,7 +131,15 @@ def main():
     ap.add_argument("--queries", type=int, default=18944)
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--no-gather", action="store_true", help="skip the to_model + predict_batch comparison")
+    ap.add_argument("--recommend", action="store_true", help="only the recommend cases (one GPU)")
+    ap.add_argument("--sample-users", type=int, default=16)
     a = ap.parse_args()
+    if a.recommend:
+        dev = torch.device("cuda", 0)
+        c = card()
+        for o in recommend_cases(a, dev):
+            print(json.dumps(dict(o, card=c)))
+        return
     real = "WORLD_SIZE" in os.environ and int(os.environ["WORLD_SIZE"]) > 1
     local = int(os.environ.get("LOCAL_RANK", 0))
     torch.cuda.set_device(local)

@@ -29,7 +29,8 @@ SYMBOLS = [
     "trs_shard_plan_build", "trs_shard_workspace_bytes", "trs_shard_train_steps", "trs_ipc_export",
     "trs_ipc_open", "trs_ipc_close", "trs_scores_backward", "trs_sort_workspace_bytes", "trs_sorted_auc",
     "trs_epoch_shuffle", "trs_gather_rows_i64", "trs_predict_topk_reuse", "trs_shard_eval_pairwise",
-    "trs_shard_gather_rows",
+    "trs_shard_gather_rows", "trs_shard_topk_exact_workspace_bytes", "trs_shard_topk_exact",
+    "trs_shard_topk_merge_sorted",
 ]
 
 
@@ -77,7 +78,7 @@ def lib() -> C.CDLL:
         L.trs_last_error.restype = C.c_char_p
         for name in ("trs_plan_bytes", "trs_plan_tmp_bytes", "trs_train_workspace_bytes", "trs_shard_stage_bytes",
                      "trs_shard_plan_bytes", "trs_shard_plan_tmp_bytes", "trs_shard_workspace_bytes",
-                     "trs_sort_workspace_bytes"):
+                     "trs_sort_workspace_bytes", "trs_shard_topk_exact_workspace_bytes"):
             getattr(L, name).restype = C.c_size_t
         if L.trs_abi_version() != 1:
             raise RuntimeError("libtrs_b200.so ABI version mismatch")
@@ -453,6 +454,42 @@ def shard_gather_rows(shard: Shard, table: int, ids, device):
     _check(lib().trs_shard_gather_rows(C.byref(shard), table, C.c_void_p(_ptr(ids, torch.int64)), C.c_int64(n),
                                        C.c_void_p(emb.data_ptr()), C.c_void_p(lin.data_ptr()), _stream()))
     return emb, lin
+
+
+def shard_topk_exact(shard: Shard, user_emb, user_lin, k: int, excl_ptr=None, excl_ids=None, workspace=None):
+    """Exact top-k of rank ``shard.rank``'s own item shard for the query rows user_emb [Q, dim] / user_lin [Q] ->
+    (global idx int64 [Q, k], score fp32 [Q, k], workspace to keep), -1 / -inf padded.  excl_ptr [Q + 1] / excl_ids:
+    per query position, the sorted local item ids of this shard to leave out."""
+    L = lib()
+    n = user_emb.shape[0]
+    dev = user_emb.device
+    idx = torch.empty((n, k), dtype=torch.int64, device=dev)
+    score = torch.empty((n, k), dtype=torch.float32, device=dev)
+    nbytes = L.trs_shard_topk_exact_workspace_bytes(C.byref(shard), C.c_int64(n), k)
+    if nbytes == 0:
+        raise RuntimeError(f"libtrs_b200: {L.trs_last_error().decode()}")
+    workspace = _grown(workspace, nbytes, dev)
+    i64 = torch.int64
+    _check(L.trs_shard_topk_exact(C.byref(shard), C.c_void_p(_ptr(user_emb, torch.float32)),
+                                  C.c_void_p(_ptr(user_lin, torch.float32)), C.c_int64(n), k,
+                                  C.c_void_p(_ptr(excl_ptr, i64)), C.c_void_p(_ptr(excl_ids, i64)),
+                                  C.c_void_p(idx.data_ptr()), C.c_void_p(score.data_ptr()),
+                                  C.c_void_p(workspace.data_ptr()), C.c_size_t(workspace.numel()), _stream()))
+    return idx, score, workspace
+
+
+def topk_merge_sorted(score, idx, k: int, excl_ptr=None, excl_ids=None):
+    """Sorted lists score / idx [n_lists, n_query, k_in] -> merged (idx [n_query, k], score [n_query, k]) by (score
+    desc, id asc), -1 / -inf padded; excl_ptr [n_query + 1] / excl_ids drop the given ids of each query."""
+    n_lists, nq, k_in = score.shape
+    out_idx = torch.empty((nq, k), dtype=torch.int64, device=score.device)
+    out_score = torch.empty((nq, k), dtype=torch.float32, device=score.device)
+    i64 = torch.int64
+    _check(lib().trs_shard_topk_merge_sorted(C.c_void_p(_ptr(score, torch.float32)), C.c_void_p(_ptr(idx, i64)),
+                                             n_lists, C.c_int64(nq), k_in, k, C.c_void_p(_ptr(excl_ptr, i64)),
+                                             C.c_void_p(_ptr(excl_ids, i64)), C.c_void_p(out_idx.data_ptr()),
+                                             C.c_void_p(out_score.data_ptr()), _stream()))
+    return out_idx, out_score
 
 
 def ipc_export(t: torch.Tensor):

@@ -27,6 +27,7 @@ from __future__ import annotations
 
 from typing import Callable, Dict, List, Optional, Tuple
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -138,6 +139,7 @@ class ShardedLinearTrainer:
         self._state_version = 0   # bumped by load_state_dict: with sync_epoch, says whether the tables changed
         self._topk_caches: Dict[int, object] = {}   # per local rank: predict's prepared bf16 item-shard operand
         self.last_predict_overflow = 0   # users predict_topk ranked exactly on this process's shards (last call)
+        self.last_recommend_paths: Dict[int, str] = {}   # local rank -> "tensor core" / "exact" of the last recommend
 
     # ---- peer mapping -----------------------------------------------------------------------------
     def _map_peers(self) -> None:
@@ -527,16 +529,13 @@ class ShardedLinearTrainer:
                                     _lib.make_table(emb, lin=lin), [])
             idx, score, over = _lib.predict_topk(model, queries, k, cache=self._topk_caches.setdefault(r, _lib.TopkCache()),
                                                  cache_key=key)
-            for q in torch.nonzero(over).flatten().tolist():   # candidate set did not fit: score the shard and sort
-                s = _lib.scores(model, torch.full((rows,), q, dtype=torch.int64, device=self.device),
-                                torch.arange(rows, device=self.device))
-                s, order = torch.sort(s, descending=True, stable=True)
-                m = min(k, rows)
-                idx[q, :m], score[q, :m] = order[:m], s[:m]
-                idx[q, m:], score[q, m:] = -1, float("-inf")
-                self.last_predict_overflow += 1
             # local order is global order within a shard: (score desc, local id asc) merges as (score desc, global id asc)
-            return torch.where(idx >= 0, idx * W + r, idx), score
+            idx = torch.where(idx >= 0, idx * W + r, idx)
+            over = torch.nonzero(over).flatten()
+            if over.numel():   # candidate set did not fit: rank those users exactly
+                idx[over], score[over] = self._exact_topk(r, u_emb[over], u_lin[over], k)
+                self.last_predict_overflow += over.numel()
+            return idx, score
 
         if len(self.local_ranks) == W:
             lists = [local_topk(r) for r in self.local_ranks]
@@ -547,6 +546,108 @@ class ShardedLinearTrainer:
         else:   # the item-sharded predict's all_to_all merger (the ordering rule above); no block offset here
             idx, score = sharded_predict_topk(lambda u, kq, offset: local_topk(self.rank), users, k, self.n_items,
                                               self.group)
+        return idx[:, :kk].contiguous(), score[:, :kk].contiguous()
+
+    RECOMMEND_MAX_K = 1024   # trs_shard_topk_exact
+
+    EXACT_CHUNK = 32768   # query users per trs_shard_topk_exact call: its workspace stays <= ~0.5 GB at k = 1024
+
+    def _exact_topk(self, r: int, u_emb, u_lin, k: int, excl_ptr=None, excl_ids=None):
+        """trs_shard_topk_exact on local rank r's item shard -> (global idx [Q, k], score [Q, k]), in chunks of
+        EXACT_CHUNK query users; the workspace lives for this call only."""
+        sh, u_lin, Q = self._shard_struct(r), u_lin.reshape(-1), u_emb.shape[0]
+        if Q <= self.EXACT_CHUNK:
+            return self._lib.shard_topk_exact(sh, u_emb, u_lin, k, excl_ptr, excl_ids)[:2]
+        idx = torch.empty((Q, k), dtype=torch.int64, device=self.device)
+        score = torch.empty((Q, k), dtype=torch.float32, device=self.device)
+        ws = None
+        for lo in range(0, Q, self.EXACT_CHUNK):
+            hi = min(Q, lo + self.EXACT_CHUNK)
+            ptr = ids = None
+            if excl_ptr is not None:   # the chunk's rows of the CSR, re-based
+                ptr = (excl_ptr[lo:hi + 1] - excl_ptr[lo]).contiguous()
+                ids = excl_ids[int(excl_ptr[lo]):int(excl_ptr[hi])].contiguous()
+            i, s, ws = self._lib.shard_topk_exact(sh, u_emb[lo:hi], u_lin[lo:hi], k, ptr, ids, ws)
+            idx[lo:hi], score[lo:hi] = i, s
+        return idx, score
+
+    def _exclusion_csr(self, r: int, users: torch.Tensor, ex_user: torch.Tensor, ex_item: torch.Tensor):
+        """(row pointers [Q + 1], sorted unique local item ids) of rank r's excluded items per query position, and the
+        most any query position has."""
+        W = self.world
+        on = ex_item % W == r
+        rows = max(shard_rows(self.n_items, r, W), 1)
+        key = torch.unique(ex_user[on] * rows + ex_item[on] // W)   # sorted: by user, then local id
+        pair_user, pair_local = key // rows, key % rows
+        start = torch.searchsorted(pair_user, users, right=False)
+        count = torch.searchsorted(pair_user, users, right=True) - start
+        ptr = torch.zeros(users.numel() + 1, dtype=torch.int64, device=self.device)
+        torch.cumsum(count, 0, out=ptr[1:])
+        total = int(ptr[-1])
+        most = int(count.max()) if count.numel() else 0
+        within = torch.arange(total, device=self.device) - torch.repeat_interleave(ptr[:-1], count, output_size=total)
+        ids = pair_local[torch.repeat_interleave(start, count, output_size=total) + within]
+        return ptr, ids.contiguous(), most
+
+    def recommend(self, users, k: int, exclude=None, _force_exact: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Top-k items of each user against the whole catalogue, leaving out ``exclude = (user_ids, item_ids)`` pairs
+        (any order, duplicates allowed, pairs of users not queried ignored) -> (idx int64 [Q, min(k, n_items)], score
+        fp32), on the device and the same on every rank, best first, ties towards the lower item id; rows with fewer
+        than k remaining items end in -1 / -inf.  Scores equal ``trs_scores`` on the gathered model bit for bit.
+        1 <= k <= 1024, any n_factors.  Each rank ranks its own item shard: with the tensor-core top-k
+        (``predict_topk``'s) when n_factors <= 239 and k plus the most items one query user has excluded on the shard
+        is <= 128 -- it over-requests that many and drops the excluded ones -- else with the exact fp32 kernel."""
+        self._require_cuda()
+        if not 1 <= int(k) <= self.RECOMMEND_MAX_K:
+            raise ValueError(f"k must be in 1..{self.RECOMMEND_MAX_K} for recommend on the row-sharded tables (got {k})")
+        _lib, W, k = self._lib, self.world, int(k)
+        users = self._device_ids(users, self.n_users, "user")
+        if exclude is not None:
+            ex_user, ex_item = exclude
+            ex_user, ex_item = (t.reshape(-1) if torch.is_tensor(t) else torch.as_tensor(np.asarray(t)).reshape(-1)
+                                for t in (ex_user, ex_item))
+            if ex_user.numel() != ex_item.numel():
+                raise ValueError(f"exclude needs as many user ids as item ids (got {ex_user.numel()} and "
+                                 f"{ex_item.numel()})")
+            ex_user = self._device_ids(ex_user, self.n_users, "exclude user")
+            ex_item = self._device_ids(ex_item, self.n_items, "exclude item")
+        Q, kk = users.numel(), min(k, self.n_items)
+        if Q == 0:
+            return (torch.empty((0, kk), dtype=torch.int64, device=self.device),
+                    torch.empty((0, kk), dtype=torch.float32, device=self.device))
+        u_emb, u_lin = _lib.shard_gather_rows(self._shard_struct(self.local_ranks[0]), 0, users, self.device)
+        key = (self.sync_epoch, self._state_version)
+
+        def local_topk(r: int):
+            """(global idx, score) [Q, k] of rank r's item shard with its excluded items left out, -1 / -inf padded."""
+            ptr, ids, most = (self._exclusion_csr(r, users, ex_user, ex_item) if exclude is not None
+                              else (None, None, 0))
+            rows = shard_rows(self.n_items, r, W)
+            exact = _force_exact or rows == 0 or self.dim > self.TOPK_MAX_FACTORS or k + most > 128
+            self.last_recommend_paths[r] = "exact" if exact else "tensor core"
+            if exact:
+                return self._exact_topk(r, u_emb, u_lin, k, ptr, ids)
+            emb, lin = self.tables[r]["item"]
+            model = _lib.make_model(_lib.NET_LINEAR, self.dim, _lib.make_table(u_emb, lin=u_lin),
+                                    _lib.make_table(emb, lin=lin), [])
+            kq = k + most
+            idx, score, over = _lib.predict_topk(model, torch.arange(Q, device=self.device), kq,
+                                                 cache=self._topk_caches.setdefault(r, _lib.TopkCache()), cache_key=key)
+            over = torch.nonzero(over).flatten()
+            if over.numel():   # candidate set did not fit: rank those users exactly
+                idx[over], score[over] = self._exact_topk(r, u_emb[over], u_lin[over], kq)
+                idx[over] = torch.where(idx[over] >= 0, idx[over] // W, idx[over])   # back to local ids
+            idx, score = _lib.topk_merge_sorted(score[None], idx[None], k, ptr, ids)   # drops the excluded
+            return torch.where(idx >= 0, idx * W + r, idx), score
+
+        merge = lambda s, i, kq: _lib.topk_merge_sorted(s.contiguous(), i.contiguous(), kq)
+        if len(self.local_ranks) == W:
+            lists = [local_topk(r) for r in self.local_ranks]
+            idx, score = lists[0] if W == 1 else merge(torch.stack([s for _, s in lists]),
+                                                       torch.stack([i for i, _ in lists]), k)
+        else:   # the all_to_all merger; its all_gather is the closing collective (the ordering rule above)
+            idx, score = sharded_predict_topk(lambda u, kq, offset: local_topk(self.rank), users, k, self.n_items,
+                                              self.group, merge=merge)
         return idx[:, :kk].contiguous(), score[:, :kk].contiguous()
 
     # ---- the bridge to TorchRecSys(net_type='linear'): shard a model + its torch optimizer, and hand them back ------
