@@ -256,32 +256,6 @@ int trs_predict_topk_reuse(const trs_model* model, const int64_t* users, int64_t
                            int k, int64_t item_offset, int64_t* out_idx, float* out_score, int32_t* overflow,
                            void* workspace, size_t workspace_bytes, int items_prepared, trs_stream_t stream);
 
-/* ---- multi-GPU building blocks (SURVEY.md §8e; the reference is single-device, model.py:74) ----------- */
-/* a7 for the OWNER of a table shard: grad.coalesce() + the row-wise optimizer step (torch:
- * optim/_functional.py:44-84, optim/adagrad.py:363-373) on an explicit list of n (row id, gradient row)
- * pairs, e.g. the gradient rows other ranks sent.  Duplicate rows are summed in list order after a stable
- * sort by id (deterministic); grad_lin (nullable) is the gradient of the width-1 companion table.
- * optim->step_scale[step] scales the update as in trs_train_steps. */
-size_t trs_sparse_update_workspace_bytes(int64_t n);
-int trs_sparse_row_update(const trs_table* table, int dim, const int64_t* ids, int64_t n, const float* grad_rows,
-                          const float* grad_lin, const trs_optim* optim, int step, void* workspace,
-                          size_t workspace_bytes, trs_stream_t stream);
-
-/* Linear scorer forward x2 + hinge + backward (linear.py:54-80, loss.py:5-9) on rows gathered elsewhere:
- * u/pos/neg rows [batch, dim] and their biases [batch] in, one gradient row per lookup out
- * (g = [hinge >= 0] * inv_batch; d user_bias = 0, SURVEY D12); *loss_sum = sum of the batch's hinges.
- * workspace: at least 8 * SM-count floats. */
-int trs_linear_rows_step(int dim, int64_t batch, float inv_batch, const float* u_rows, const float* pos_rows,
-                         const float* neg_rows, const float* u_bias, const float* pos_bias, const float* neg_bias,
-                         float* g_u, float* g_pos, float* g_neg, float* g_pos_bias, float* g_neg_bias,
-                         float* loss_sum, float* workspace, size_t workspace_floats, trs_stream_t stream);
-
-/* Merge n_lists per-shard top-k lists (score / idx laid out [n_lists, n_query, k], idx < 0 = padding) into
- * the global top-k per user, ordered by (score descending, item id ascending) -- the allgather half of the
- * item-sharded predict. n_lists * k <= 4000. */
-int trs_topk_merge(const float* score, const int64_t* idx, int n_lists, int k, int64_t n_query,
-                   int64_t* out_idx, float* out_score, trs_stream_t stream);
-
 /* ---- a7 for callers that drive autograd themselves: TorchRecSys.forward -> hinge_loss -> backward (model.py:171-200) */
 /* Backward of trs_scores (Linear / FM): grad_out[b] = d loss / d score[b]; writes ONE gradient row per lookup --
  * g_user / g_item [n, dim], g_meta[f] [n, dim], and (nullable) the width-1 companions' gradients g_lin_* [n] -- exactly
@@ -391,7 +365,9 @@ int trs_shard_topk_exact(const trs_shard* shard, const float* user_emb, const fl
 /* Merge n_lists sorted lists (score / idx [n_lists, n_query, k_in], each row ordered by (score desc, id asc), idx < 0 =
  * padding at the end) into out [n_query, k_out] in the same order, -1 / -inf padded.  excl_ptr [n_query + 1] /
  * excl_ids (both nullable): per query, sorted ids (in the lists' id space) to drop.  O(n_lists^2 k_in log k_in) per
- * query; n_lists * (k_in + 1) <= 40960. */
+ * query; n_lists * (k_in + 1) <= 40960.  The one list merge of the library: item ranges of trs_shard_topk_exact, the
+ * ranks' lists of the row-sharded tables, and the item blocks' trs_predict_topk lists of the item-sharded predict,
+ * which trs_predict_topk already orders this way (a row it flags as overflowing is all padding). */
 int trs_shard_topk_merge_sorted(const float* score, const int64_t* idx, int n_lists, int64_t n_query, int k_in,
                                 int k_out, const int64_t* excl_ptr, const int64_t* excl_ids, int64_t* out_idx,
                                 float* out_score, trs_stream_t stream);

@@ -1,7 +1,6 @@
-"""Host logic of the multi-GPU paths (torchrecsys_b200/sharded.py) on the CPU: world size 2, gloo, with torch
-stand-ins for the three CUDA hooks.  Checks: the routing round trip, that a row-sharded training step over two
-ranks equals one single-process step of the numpy oracle on the concatenated (global) batch, and that the
-item-sharded predict merge returns the global stable top-k."""
+"""Host logic of the item-sharded predict (torchrecsys_b200/sharded.py: sharded_predict_topk) on the CPU: world size
+2, gloo, with torch stand-ins for the local top-k and the list merge.  Checks that the all_to_all merger returns the
+global stable top-k."""
 import os
 import socket
 
@@ -11,9 +10,7 @@ import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
 
-from oracle import cf_oracle as O
-
-U, I, D, B, WORLD = 41, 29, 8, 24, 2
+U, I, D, WORLD = 41, 29, 8, 2
 
 
 def _free_port():
@@ -24,71 +21,19 @@ def _free_port():
     return p
 
 
-def _torch_hooks(trainer):
-    """CPU stand-ins with the kernels' semantics (test-only)."""
-    def gather(name, rows):
-        emb, bias = trainer.tables[name]
-        return torch.cat([emb[rows], bias[rows]], 1)
-
-    def compute(u, vp, vn, inv_batch):
-        Dm = trainer.dim
-        sp = (u[:, :Dm] * vp[:, :Dm]).sum(1) + u[:, Dm] + vp[:, Dm]
-        sn = (u[:, :Dm] * vn[:, :Dm]).sum(1) + u[:, Dm] + vn[:, Dm]
-        h = sn - sp + 1.0
-        g = ((h >= 0).float() * inv_batch)[:, None]
-        z = torch.zeros_like(g)
-        return (torch.cat([g * (vn[:, :Dm] - vp[:, :Dm]), z], 1), torch.cat([-g * u[:, :Dm], -g], 1),
-                torch.cat([g * u[:, :Dm], g], 1), torch.clamp(h, min=0).sum().view(1))
-
-    def update(name, rows, grads):   # SGD on coalesced rows
-        emb, bias = trainer.tables[name]
-        acc = torch.zeros((emb.shape[0], trainer.dim + 1))
-        acc.index_add_(0, rows, grads)
-        emb -= trainer.lr * acc[:, :trainer.dim]
-        if name != "user":
-            bias -= trainer.lr * acc[:, trainer.dim:]
-    return {"gather": gather, "compute": compute, "update": update}
-
-
 def _worker(rank, port, q):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
     dist.init_process_group("gloo", rank=rank, world_size=WORLD)
     try:
-        from torchrecsys_b200 import routed as R, sharded as S
+        from torchrecsys_b200 import sharded as S
         torch.set_num_threads(1)
         rng = np.random.default_rng(7)
-        full = {"user.weight": rng.normal(0, .5, (U, D)).astype(np.float32),
-                "item.weight": rng.normal(0, .5, (I, D)).astype(np.float32),
-                "user_bias.weight": np.zeros((U, 1), np.float32),
-                "item_bias.weight": rng.normal(0, .1, (I, 1)).astype(np.float32)}
-        batch = {k: rng.integers(0, n, WORLD * B) for k, n in (("user", U), ("pos", I), ("neg", I))}
-        tr = R.RoutedLinearTrainer(U, I, D, optimizer="sgd", lr=0.3, device=torch.device("cpu"))
-        tr._gather, tr._compute, tr._update = (_torch_hooks(tr)[k] for k in ("gather", "compute", "update"))
-        for name, key, bkey in (("user", "user.weight", "user_bias.weight"), ("item", "item.weight", "item_bias.weight")):
-            emb, bias = tr.tables[name]
-            emb.copy_(torch.from_numpy(full[key][rank::WORLD]))
-            bias.copy_(torch.from_numpy(full[bkey][rank::WORLD]))
-        # routing round trip: what comes back for lookup j is the row of id j
-        ids = torch.from_numpy(batch["user"][rank * B:(rank + 1) * B])
-        route = R.make_route(ids, torch.zeros_like(ids), 2, WORLD)
-        back = R.exchange_back(route, tr._gather("user", route.recv_rows))
-        assert torch.equal(back[:, :D], torch.from_numpy(full["user.weight"])[ids])
-        # one sharded step == one oracle step on the global batch
-        sl = slice(rank * B, (rank + 1) * B)
-        hsum = tr.train_step(*(torch.from_numpy(batch[k][sl]) for k in ("user", "pos", "neg")))
-        dist.all_reduce(hsum)
-        spec = O.OptSpec("sgd", lr=0.3)
-        params = {k: v.copy() for k, v in full.items()}
-        want_loss = O.train_step("linear", params, O.init_opt_state(params, spec), batch, spec, 1)
-        assert abs(float(hsum) / (WORLD * B) - float(want_loss)) < 1e-5
-        got_u, _ = tr.gather_full("user")
-        got_i, got_ib = tr.gather_full("item")
-        np.testing.assert_allclose(got_u.numpy(), params["user.weight"], rtol=1e-5, atol=1e-6)
-        np.testing.assert_allclose(got_i.numpy(), params["item.weight"], rtol=1e-5, atol=1e-6)
-        np.testing.assert_allclose(got_ib.numpy(), params["item_bias.weight"], rtol=1e-5, atol=1e-6)
-        # item-sharded predict: local top-k on a contiguous block, all-gather, merge
+        user_w = rng.normal(0, .5, (U, D)).astype(np.float32)
+        item_w = rng.normal(0, .5, (I, D)).astype(np.float32)
+        item_b = rng.normal(0, .1, (I, 1)).astype(np.float32)
+        # item-sharded predict: local top-k on a contiguous block, each user's lists to one merger rank, merge, all-gather
         k = 7
-        scores_full = torch.from_numpy(params["user.weight"][:5] @ params["item.weight"].T + params["item_bias.weight"].T)
+        scores_full = torch.from_numpy(user_w[:5] @ item_w.T + item_b.T)
         scores_full = (scores_full * 4).round() / 4  # force ties
 
         def local_topk(users, kk, offset):
@@ -96,7 +41,7 @@ def _worker(rank, port, q):
             v, o = torch.sort(scores_full[users, lo:hi], dim=1, descending=True, stable=True)
             return (o[:, :kk] + offset).contiguous(), v[:, :kk].contiguous()
 
-        def merge(sc, ix, kk):  # torch stand-in of trs_topk_merge: (score desc, id asc)
+        def merge(sc, ix, kk):  # torch stand-in of trs_shard_topk_merge_sorted: (score desc, id asc)
             Q = sc.shape[1]
             s2, i2 = sc.permute(1, 0, 2).reshape(Q, -1), ix.permute(1, 0, 2).reshape(Q, -1)
             o = torch.argsort(i2, dim=1, stable=True)
@@ -115,7 +60,7 @@ def _worker(rank, port, q):
         dist.destroy_process_group()
 
 
-def test_sharded_paths_world_size_2_gloo():
+def test_item_sharded_predict_merge_world_size_2_gloo():
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = _free_port()

@@ -1,6 +1,6 @@
 """torchrun worker: the row-sharded Linear trainer over REAL peers (CUDA-IPC mapped shards, NVLink loads / stores,
-flag barriers; torchrecsys_b200/sharded.py + csrc/shard.cu), the host-driven all_to_all baseline (routed.py) and the
-item-sharded predict over NCCL -- each against the numpy oracle's single-process results on the global batch.
+flag barriers; torchrecsys_b200/sharded.py + csrc/shard.cu) and the item-sharded predict over NCCL -- each against
+the numpy oracle's single-process results on the global batch.
 Prints SHARDED CHECK OK on rank 0."""
 import os
 import sys
@@ -12,7 +12,7 @@ import torch.distributed as dist
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from oracle import cf_oracle as O  # noqa: E402
-from torchrecsys_b200 import _lib, routed as R, sharded as S  # noqa: E402
+from torchrecsys_b200 import _lib, sharded as S  # noqa: E402
 from torchrecsys_b200.collaborative.linear import Linear  # noqa: E402
 
 
@@ -51,23 +51,6 @@ def main():
         w1 = O.train_step("linear", params, state, b, spec, steps + 1)
         assert abs(float(l1) - float(w1)) < 1e-4, (kind, float(l1), float(w1))
         tr.close()
-        # ---- the round-1 baseline: host-driven all_to_all ----
-        rt = R.RoutedLinearTrainer(U, I, D, optimizer=kind, lr=0.05, device=dev)
-        for name, key, bkey in (("user", "user.weight", "user_bias.weight"), ("item", "item.weight", "item_bias.weight")):
-            emb, bias = rt.tables[name]
-            emb.copy_(torch.from_numpy(full[key][rank::world]))
-            bias.copy_(torch.from_numpy(full[bkey][rank::world]))
-        params = {k: v.copy() for k, v in full.items()}
-        state = O.init_opt_state(params, spec)
-        for s, batch in enumerate(batches):
-            hsum = rt.train_step(*(torch.from_numpy(batch[k][sl]).to(dev) for k in ("user", "pos", "neg")))
-            dist.all_reduce(hsum)
-            want = O.train_step("linear", params, state, batch, spec, s + 1)
-            assert abs(float(hsum) / (world * B) - float(want)) < 1e-4, (kind, s, float(hsum) / (world * B), float(want))
-        for name, key in (("user", "user.weight"), ("item", "item.weight")):
-            got, got_b = rt.gather_full(name)
-            np.testing.assert_allclose(got.cpu().numpy(), params[key], rtol=1e-4, atol=tol, err_msg=f"routed {kind} {key}")
-        np.testing.assert_allclose(got_b.cpu().numpy(), params["item_bias.weight"], rtol=1e-4, atol=tol)
     # item-sharded predict: each rank holds a contiguous item block of the (replicated-user) Linear model
     k, Q = 50, 200
     lo, hi = S.item_block(I, rank, world)

@@ -24,8 +24,7 @@ SYMBOLS = [
     "trs_plan_build", "trs_train_workspace_bytes", "trs_train_steps", "trs_eval_pairwise",
     "trs_gemm_bf16_tn", "trs_mlp_forward_workspace_bytes", "trs_mlp_forward",
     "trs_mlp_train_workspace_bytes", "trs_mlp_train_steps", "trs_predict_topk_workspace_bytes",
-    "trs_predict_topk", "trs_sparse_update_workspace_bytes", "trs_sparse_row_update", "trs_linear_rows_step",
-    "trs_topk_merge", "trs_shard_stage_bytes", "trs_shard_plan_bytes", "trs_shard_plan_tmp_bytes",
+    "trs_predict_topk", "trs_shard_stage_bytes", "trs_shard_plan_bytes", "trs_shard_plan_tmp_bytes",
     "trs_shard_plan_build", "trs_shard_workspace_bytes", "trs_shard_train_steps", "trs_ipc_export",
     "trs_ipc_open", "trs_ipc_close", "trs_scores_backward", "trs_sort_workspace_bytes", "trs_sorted_auc",
     "trs_epoch_shuffle", "trs_gather_rows_i64", "trs_predict_topk_reuse", "trs_shard_eval_pairwise",
@@ -343,47 +342,6 @@ def predict_topk(model: Model, users, k: int, item_meta=None, item_offset: int =
                                     C.c_void_p(over.data_ptr()), C.c_void_p(ws.data_ptr()),
                                     C.c_size_t(nbytes), int(reuse), _stream()))
     return idx, score, over
-
-
-# ---- multi-GPU building blocks ------------------------------------------------------------------------
-def sparse_row_update(table: Table, dim: int, ids, grad_rows, grad_lin, optim: Optim, step: int) -> None:
-    """coalesce + row-wise optimizer step of one (local shard of a) table on (id, gradient row) pairs."""
-    L = lib()
-    L.trs_sparse_update_workspace_bytes.restype = C.c_size_t
-    n = ids.shape[0]
-    if n == 0:
-        return
-    nbytes = L.trs_sparse_update_workspace_bytes(C.c_int64(n))
-    ws = torch.empty(nbytes, dtype=torch.uint8, device=ids.device)
-    _check(L.trs_sparse_row_update(C.byref(table), dim, C.c_void_p(_ptr(ids, torch.int64)), C.c_int64(n),
-                                   C.c_void_p(_ptr(grad_rows, torch.float32)),
-                                   C.c_void_p(_ptr(grad_lin, torch.float32)), C.byref(optim), step,
-                                   C.c_void_p(ws.data_ptr()), C.c_size_t(nbytes), _stream()))
-
-
-def linear_rows_step(u, vp, vn, bu, bip, bin_, inv_batch: float):
-    """Linear forward x2 + hinge + backward on gathered rows -> (g_u, g_vp, g_vn, g_bip, g_bin, hinge_sum)."""
-    B, D = u.shape
-    f32 = torch.float32
-    outs = [torch.empty_like(u), torch.empty_like(u), torch.empty_like(u),
-            torch.empty(B, dtype=f32, device=u.device), torch.empty(B, dtype=f32, device=u.device),
-            torch.empty(1, dtype=f32, device=u.device)]
-    ws = torch.empty(8 * device_info()[0], dtype=f32, device=u.device)
-    args = [C.c_void_p(_ptr(t, f32)) for t in (u, vp, vn, bu, bip, bin_)] + [C.c_void_p(t.data_ptr()) for t in outs]
-    _check(lib().trs_linear_rows_step(D, C.c_int64(B), C.c_float(inv_batch), *args, C.c_void_p(ws.data_ptr()),
-                                      C.c_size_t(ws.numel()), _stream()))
-    return outs
-
-
-def topk_merge(score, idx, k: int):
-    """score / idx [n_lists, n_query, k] -> merged (idx [n_query, k], score [n_query, k])."""
-    n_lists, nq = score.shape[0], score.shape[1]
-    out_idx = torch.empty((nq, k), dtype=torch.int64, device=score.device)
-    out_score = torch.full((nq, k), float("-inf"), dtype=torch.float32, device=score.device)
-    _check(lib().trs_topk_merge(C.c_void_p(_ptr(score, torch.float32)), C.c_void_p(_ptr(idx, torch.int64)),
-                                n_lists, k, C.c_int64(nq), C.c_void_p(out_idx.data_ptr()),
-                                C.c_void_p(out_score.data_ptr()), _stream()))
-    return out_idx, out_score
 
 
 # ---- row-sharded training over peer-mapped shards (include/trs.h: trs_shard) ---------------------------

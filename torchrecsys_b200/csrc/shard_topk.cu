@@ -1,7 +1,8 @@
 // shard_topk.cu -- exact top-k over a rank's own item shard of the row-sharded tables (trs_shard, csrc/shard.cu).
 //   * trs_shard_topk_exact: exact fp32 top-k of the shard for dense query rows, bit-identical to trs_scores + a stable
 //     descending sort, optionally leaving out given items (ShardedLinearTrainer.recommend; predict_topk's overflow).
-//   * trs_shard_topk_merge_sorted: merge of such sorted lists -- item ranges of one rank, or ranks.
+//   * trs_shard_topk_merge_sorted: merge of such sorted lists -- item ranges of one rank, or ranks -- and of the
+//     item blocks' trs_predict_topk lists of the item-sharded predict (sharded_predict_topk), ordered the same way.
 // Kept out of shard_serve.cu: a kernel with dynamic shared memory in that module changes the shared-memory reservation,
 // and so the SASS, of its existing kernels.
 #include "scorer.cuh"

@@ -1,4 +1,4 @@
-// train.cuh -- the row-wise optimizer step shared by the training kernels (train.cu, shard.cu, sharded.cu): the
+// train.cuh -- the row-wise optimizer step shared by the training kernels (train.cu, shard.cu): the
 // update of one value, of a row held in registers and of a width-1 companion, each followed by the stores of the
 // parameter and its optimizer state; and what mlp.cu needs from train.cu: the reduce + update phase of the fused
 // training kernel, run on gradient rows the MLP backward staged itself.

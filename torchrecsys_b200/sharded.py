@@ -13,16 +13,17 @@ Row-sharded training (BASELINE configs[3], Linear 50M x 5M, dim 128)  -- ``Shard
     owner's staging buffer, and every owner coalesces + updates its own rows -- two flag barriers per step.
     ``state_dict()`` / ``load_state_dict()`` gather / scatter the shards (parameters AND optimizer state) in the
     reference's single-process layout and key names, so checkpoints interchange with ``TorchRecSys``.
-    ``evaluate`` / ``eval_pairwise`` / ``predict_topk`` / ``lookup`` serve the model where it lives: their kernels
+    ``evaluate`` / ``eval_pairwise`` / ``lookup`` serve the model where it lives: their kernels
     (csrc/shard_serve.cu) read every row from its owner through the same peer mappings, nothing is gathered.
+    ``recommend`` (and ``predict_topk``, its narrower form) ranks each rank's own item shard (csrc/shard_topk.cu)
+    and merges the ranks' sorted lists with trs_shard_topk_merge_sorted.
     One GPU can host the whole group (``emulate_world=G``): the parity tests run that way on a 1-GPU box.
 
 Item-sharded predict (BASELINE configs[4])
     contiguous item blocks per rank (global id = offset + local id, so the single-GPU tie-break "lower item id
-    first" carries over), user rows replicated; each rank runs trs_predict_topk on its block, the
-    (score, id)[Q, k] lists are all-gathered and merged by trs_topk_merge.
-
-The host-driven all_to_all baseline of round 1 lives in ``routed.py``."""
+    first" carries over), user rows replicated; each rank runs trs_predict_topk on its block, each user's
+    sorted (score, id)[k] lists go to one merger rank by all_to_all, are merged there by
+    trs_shard_topk_merge_sorted, and the results are all-gathered."""
 from __future__ import annotations
 
 from typing import Callable, Dict, List, Optional, Tuple
@@ -138,7 +139,9 @@ class ShardedLinearTrainer:
         self.launches = 0
         self._state_version = 0   # bumped by load_state_dict: with sync_epoch, says whether the tables changed
         self._topk_caches: Dict[int, object] = {}   # per local rank: predict's prepared bf16 item-shard operand
-        self.last_predict_overflow = 0   # users predict_topk ranked exactly on this process's shards (last call)
+        # users the last predict_topk / recommend re-ranked exactly on this process's shards because the tensor-core
+        # top-k flagged their candidate set as overflowing
+        self.last_predict_overflow = 0
         self.last_recommend_paths: Dict[int, str] = {}   # local rank -> "tensor core" / "exact" of the last recommend
 
     # ---- peer mapping -----------------------------------------------------------------------------
@@ -417,10 +420,10 @@ class ShardedLinearTrainer:
     #  * Reads after training are safe: every training launch ends waiting for every rank's last arrival (csrc/shard.cu,
     #    the cross_wait after the step loop), and load_state_dict ends with a barrier.
     #  * Reads before the next training: each method below that launches a peer-reading kernel ends with a group
-    #    collective on this rank's stream before it returns -- eval_pairwise the all-gather, predict_topk the
-    #    all_to_all, lookup a one-element all-reduce.  This rank's next training kernel is queued behind that
-    #    collective, and the collective cannot complete before every rank's reads have finished: no host
-    #    synchronisation is needed.
+    #    collective on this rank's stream before it returns -- eval_pairwise the all-gather, recommend / predict_topk
+    #    the all_to_all merger's all-gather, lookup a one-element all-reduce.  This rank's next training kernel is
+    #    queued behind that collective, and the collective cannot complete before every rank's reads have finished: no
+    #    host synchronisation is needed.
     # In a real group these methods are collective: every rank calls them with the same arguments.
     TOPK_MAX_FACTORS = 239   # predict_batch's kernel path (csrc/topk.cu: check_topk); k in 1..128 likewise
 
@@ -500,53 +503,14 @@ class ShardedLinearTrainer:
     def predict_topk(self, users, k: int) -> Tuple[torch.Tensor, torch.Tensor]:
         """Top-k items of each user against the whole catalogue -> (idx int64 [Q, min(k, n_items)], score fp32), on the
         device and the same on every rank; equal to ``_lib.predict_topk`` / ``TorchRecSys.predict_batch`` on the gathered
-        model (best first, ties towards the lower item id).  Each rank ranks its own item shard against the query users'
-        rows; the per-shard lists are merged."""
+        model (best first, ties towards the lower item id).  ``recommend(users, k)`` under predict_batch's limits:
+        1 <= k <= 128 and n_factors <= 239, which keep every shard on the tensor-core top-k."""
         self._require_cuda()
         if not 1 <= int(k) <= 128:
             raise ValueError(f"top_k must be in 1..128 on the row-sharded tables (got {k})")
         if self.dim > self.TOPK_MAX_FACTORS:
             raise ValueError(f"predict_topk on the row-sharded tables needs n_factors <= {self.TOPK_MAX_FACTORS}")
-        _lib, W, k = self._lib, self.world, int(k)
-        users = self._device_ids(users, self.n_users, "user")
-        Q, kk = users.numel(), min(k, self.n_items)
-        self.last_predict_overflow = 0
-        if Q == 0:
-            return (torch.empty((0, kk), dtype=torch.int64, device=self.device),
-                    torch.empty((0, kk), dtype=torch.float32, device=self.device))
-        u_emb, u_lin = _lib.shard_gather_rows(self._shard_struct(self.local_ranks[0]), 0, users, self.device)
-        queries = torch.arange(Q, device=self.device)
-        key = (self.sync_epoch, self._state_version)   # unchanged tables: the prepared item operand is reused
-
-        def local_topk(r: int):
-            """(global idx, score) [Q, k] of rank r's item shard, -1 / -inf padded."""
-            emb, lin = self.tables[r]["item"]
-            rows = emb.shape[0]
-            if rows == 0:
-                return (torch.full((Q, k), -1, dtype=torch.int64, device=self.device),
-                        torch.full((Q, k), float("-inf"), device=self.device))
-            model = _lib.make_model(_lib.NET_LINEAR, self.dim, _lib.make_table(u_emb, lin=u_lin),
-                                    _lib.make_table(emb, lin=lin), [])
-            idx, score, over = _lib.predict_topk(model, queries, k, cache=self._topk_caches.setdefault(r, _lib.TopkCache()),
-                                                 cache_key=key)
-            # local order is global order within a shard: (score desc, local id asc) merges as (score desc, global id asc)
-            idx = torch.where(idx >= 0, idx * W + r, idx)
-            over = torch.nonzero(over).flatten()
-            if over.numel():   # candidate set did not fit: rank those users exactly
-                idx[over], score[over] = self._exact_topk(r, u_emb[over], u_lin[over], k)
-                self.last_predict_overflow += over.numel()
-            return idx, score
-
-        if len(self.local_ranks) == W:
-            lists = [local_topk(r) for r in self.local_ranks]
-            if W == 1:
-                idx, score = lists[0]
-            else:
-                idx, score = _lib.topk_merge(torch.stack([s for _, s in lists]), torch.stack([i for i, _ in lists]), k)
-        else:   # the item-sharded predict's all_to_all merger (the ordering rule above); no block offset here
-            idx, score = sharded_predict_topk(lambda u, kq, offset: local_topk(self.rank), users, k, self.n_items,
-                                              self.group)
-        return idx[:, :kk].contiguous(), score[:, :kk].contiguous()
+        return self.recommend(users, k)   # raises IndexError for bad ids
 
     RECOMMEND_MAX_K = 1024   # trs_shard_topk_exact
 
@@ -612,11 +576,13 @@ class ShardedLinearTrainer:
             ex_user = self._device_ids(ex_user, self.n_users, "exclude user")
             ex_item = self._device_ids(ex_item, self.n_items, "exclude item")
         Q, kk = users.numel(), min(k, self.n_items)
+        self.last_predict_overflow = 0
         if Q == 0:
             return (torch.empty((0, kk), dtype=torch.int64, device=self.device),
                     torch.empty((0, kk), dtype=torch.float32, device=self.device))
         u_emb, u_lin = _lib.shard_gather_rows(self._shard_struct(self.local_ranks[0]), 0, users, self.device)
-        key = (self.sync_epoch, self._state_version)
+        queries = torch.arange(Q, device=self.device)
+        key = (self.sync_epoch, self._state_version)   # unchanged tables: the prepared item operand is reused
 
         def local_topk(r: int):
             """(global idx, score) [Q, k] of rank r's item shard with its excluded items left out, -1 / -inf padded."""
@@ -631,23 +597,25 @@ class ShardedLinearTrainer:
             model = _lib.make_model(_lib.NET_LINEAR, self.dim, _lib.make_table(u_emb, lin=u_lin),
                                     _lib.make_table(emb, lin=lin), [])
             kq = k + most
-            idx, score, over = _lib.predict_topk(model, torch.arange(Q, device=self.device), kq,
+            idx, score, over = _lib.predict_topk(model, queries, kq,
                                                  cache=self._topk_caches.setdefault(r, _lib.TopkCache()), cache_key=key)
             over = torch.nonzero(over).flatten()
             if over.numel():   # candidate set did not fit: rank those users exactly
                 idx[over], score[over] = self._exact_topk(r, u_emb[over], u_lin[over], kq)
                 idx[over] = torch.where(idx[over] >= 0, idx[over] // W, idx[over])   # back to local ids
-            idx, score = _lib.topk_merge_sorted(score[None], idx[None], k, ptr, ids)   # drops the excluded
+                self.last_predict_overflow += over.numel()
+            if ptr is not None:   # drops the excluded
+                idx, score = _lib.topk_merge_sorted(score[None], idx[None], k, ptr, ids)
+            # local order is global order within a shard: (score desc, local id asc) merges as (score desc, global id asc)
             return torch.where(idx >= 0, idx * W + r, idx), score
 
-        merge = lambda s, i, kq: _lib.topk_merge_sorted(s.contiguous(), i.contiguous(), kq)
         if len(self.local_ranks) == W:
             lists = [local_topk(r) for r in self.local_ranks]
-            idx, score = lists[0] if W == 1 else merge(torch.stack([s for _, s in lists]),
-                                                       torch.stack([i for i, _ in lists]), k)
+            idx, score = lists[0] if W == 1 else merge_topk_lists(torch.stack([s for _, s in lists]),
+                                                                  torch.stack([i for i, _ in lists]), k)
         else:   # the all_to_all merger; its all_gather is the closing collective (the ordering rule above)
             idx, score = sharded_predict_topk(lambda u, kq, offset: local_topk(self.rank), users, k, self.n_items,
-                                              self.group, merge=merge)
+                                              self.group)
         return idx[:, :kk].contiguous(), score[:, :kk].contiguous()
 
     # ---- the bridge to TorchRecSys(net_type='linear'): shard a model + its torch optimizer, and hand them back ------
@@ -731,17 +699,19 @@ def item_block(n_items: int, rank: int, world: int) -> Tuple[int, int]:
 
 
 def merge_topk_lists(scores: torch.Tensor, idx: torch.Tensor, k: int, merge: Optional[Callable] = None):
-    """scores / idx [G, Q, k] -> (idx [Q, k], score [Q, k]) by (score desc, id asc); idx < 0 is padding."""
+    """scores / idx [G, Q, k_in], each row sorted by (score desc, id asc) with idx < 0 padding at the end -> (idx [Q, k],
+    score [Q, k]) in the same order, -1 / -inf padded.  ``merge`` replaces trs_shard_topk_merge_sorted (CPU tests)."""
     if merge is not None:
         return merge(scores, idx, k)
     from . import _lib
-    return _lib.topk_merge(scores.contiguous(), idx.contiguous(), k)
+    return _lib.topk_merge_sorted(scores.contiguous(), idx.contiguous(), k)
 
 
 def sharded_predict_topk(local_topk: Callable, users: torch.Tensor, k: int, n_items: int, group=None,
                          merge: Optional[Callable] = None):
-    """``local_topk(users, k, item_offset) -> (idx [Q, k] global ids, score [Q, k])`` on this rank's item block;
-    returns the merged global top-k on every rank.
+    """``local_topk(users, k, item_offset) -> (idx [Q, k] global ids, score [Q, k])`` on this rank's item block, each
+    row sorted by (score desc, id asc) and -1 / -inf padded, as trs_predict_topk writes it; returns the merged global
+    top-k on every rank.
 
     The per-rank candidate lists are exchanged with an all_to_all that sends each user's candidates to ONE merger rank
     (users split evenly over the ranks): every rank merges Q / G users x G lists instead of all Q users -- G times less
@@ -750,8 +720,8 @@ def sharded_predict_topk(local_topk: Callable, users: torch.Tensor, k: int, n_it
     lo, _ = item_block(n_items, rank, world)
     idx, score = local_topk(users, k, lo)
     Q = idx.shape[0]
-    if world == 1:
-        return merge_topk_lists(score[None], idx[None], k, merge)
+    if world == 1:   # one sorted list is its own merge
+        return idx, score
     Qc = -(-Q // world)                                   # users per merger rank
     pad = Qc * world - Q
     if pad:
