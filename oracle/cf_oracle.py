@@ -276,7 +276,9 @@ def apply_rows(p, state, rows, g, spec: OptSpec, step: int) -> None:
     """In-place update of ``p[rows]`` with coalesced gradient rows ``g``.
 
     sparse_adam: torch: optim/_functional.py:65-84; adagrad: torch: optim/adagrad.py:363-373;
-    sgd: torch: optim/sgd.py (_single_tensor_sgd: ``param.add_(grad, alpha=-lr)``)."""
+    sgd: torch: optim/sgd.py (_single_tensor_sgd: ``param.add_(grad, alpha=-lr)``).
+    Every product is rounded before its sum, as torch on CUDA does; tests/test_train_exact.py states this contract and
+    checks the kernels and torch's CUDA optimizers against this function bit for bit."""
     g = g.astype(F32)
     if spec.kind == "sgd":
         p[rows] = (p[rows] + F32(-spec.lr) * g).astype(F32)

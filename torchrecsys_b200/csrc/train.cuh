@@ -23,7 +23,9 @@ struct OptScalars {
 };
 
 // ---- row-wise optimizers (torch: optim/_functional.py:65-84, optim/adagrad.py:363-373, sgd) ----
-// Explicit _rn intrinsics keep nvcc from contracting mul+add into FMA where torch runs two ops.
+// Explicit _rn intrinsics keep nvcc from contracting mul+add into FMA where torch runs two ops.  torch on CUDA rounds
+// Adagrad's product before the sum too; torch on the CPU fuses it.  The op stream is the contract stated in
+// tests/test_train_exact.py, which checks it bit for bit, and oracle/cf_oracle.py: apply_rows restates it.
 __device__ __forceinline__ void opt_update(const OptScalars& o, float scale, float g, float& p,
                                            float& s0, float& s1) {
     if (o.kind == TRS_OPT_SPARSE_ADAM) {
